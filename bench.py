@@ -18,6 +18,8 @@ cosine schedule, known-region injection on) for `--batch` 256x256 images per GPU
 `--impl reference`: the same CPU implementation, all host threads, one JSON line.
 `--preset cfg3|cfg4|cfg5`: BASELINE.json configs[2] / [3] / [4] as one reproducible command each (see PRESETS).
 `--global-batch G`: strong scaling -- G images split over the ranks (per-GPU batch G / N).
+`--dump-outputs DIR`: after the timed steps, the images the last timed step returned go to DIR/samples.npy (float32), so
+           that two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -57,6 +59,23 @@ PRESETS = {
                  note="BASELINE configs[4]: ADM256 with LoRA-merged qkv / proj_out weights, DDIM-100 quadratic, batch 64 "
                       "batch-sharded over the ranks"),
 }
+
+
+DUMP_MAX_BYTES = 64_000_000 - 4096          # 64 MB (decimal) in all, with room for the .npy header
+
+
+def dump_samples(path, samples):
+    """Write `samples` [N, ...] as float32 to path/samples.npy.  Beyond DUMP_MAX_BYTES a fixed, seeded subset of whole
+    images is kept, in batch order, so that runs with the same arguments write the same file."""
+    import numpy as np
+    samples = samples.detach().float().cpu()
+    n = samples.shape[0]
+    keep = max(1, DUMP_MAX_BYTES // max(1, samples[:1].numel() * 4))
+    if n > keep:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        samples = samples[idx]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "samples.npy"), samples.numpy())
 
 
 def peaks():
@@ -191,8 +210,8 @@ def run_reference(args, wl):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=None, help="timed sampling loops (default 2)")
+    ap.add_argument("--warmup", type=int, default=None, help="untimed sampling loops before them (default 3)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="adm256", choices=sorted(WORKLOADS))
     ap.add_argument("--batch", type=int, default=8, help="images per GPU")
@@ -209,8 +228,20 @@ def main():
     ap.add_argument("--global-batch", type=int, default=None,
                     help="strong scaling: this many images split over the ranks (per-GPU batch = G / N)")
     ap.add_argument("--lora", action="store_true", help="LoRA-merged qkv / proj_out weights (same keys and shapes)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the images the last timed step returned to DIR/samples.npy (float32, at most 64 MB: a "
+                         "fixed, seeded subset of whole images beyond that)")
     args = ap.parse_args()
     preset = PRESETS.get(args.preset)
+    fixed_count = args.eval_only or (preset and "sweep" in preset)       # these modes time a fixed number of runs
+    if fixed_count and (args.steps is not None or args.warmup is not None):
+        ap.error("--steps / --warmup do not apply to --eval-only (40 timed evaluations) or a sweep (one loop per size)")
+    args.steps = 2 if args.steps is None else args.steps
+    args.warmup = 3 if args.warmup is None else args.warmup
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (fixed_count or args.impl == "reference"):
+        ap.error("--dump-outputs applies to the sampling benchmark only (not --eval-only, --impl reference or a sweep)")
     if preset:
         args.workload, args.sampler, args.ddim_steps, args.schedule = (preset["workload"], preset["sampler"],
                                                                         preset["ddim_steps"], preset["schedule"])
@@ -287,15 +318,21 @@ def main():
     torch.cuda.manual_seed(1234 + rank)
 
     def loop(g, k):
+        # every loop starts from the same generator state: the noise of the last timed step depends on the seed alone,
+        # not on --warmup / --steps
+        torch.cuda.manual_seed(1234 + rank)
         if args.sampler == "ddpm":
             return diffusion.p_sample_loop(fn, (B, 3, S, S), model_kwargs={"gt": g, "gt_keep_mask": k}, device=dev,
                                            use_inpainting_injection=True)
         return diffusion.ddim_sample_loop(fn, (B, 3, S, S), model_kwargs={"gt": g, "gt_keep_mask": k}, device=dev,
                                           eta=0.0, use_inpainting_injection=True)
 
+    last = {}
+
     def step_device():
         out = loop(gt, keep)
-        return gather_batch(out, B * world) if world > 1 else out
+        last["samples"] = gather_batch(out, B * world) if world > 1 else out
+        return last["samples"]
 
     def step_e2e():
         g = host_gt.to(dev, non_blocking=True)
@@ -337,6 +374,8 @@ def main():
         step_device()
     with ClockSampler(local) as clk:
         ms = timed(step_device, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_samples(args.dump_outputs, last["samples"])
     ms_e2e = timed(step_e2e, args.steps)
     images = B * world * args.steps
     value = images / (ms / 1e3)

@@ -18,6 +18,7 @@ What is pinned here (VERDICT r1 "next round" item 1):
           adm256_ddpm25.pt         p_sample_loop over a 25-step linear schedule (full loop)
           adm256_ddim100.pt        DDIM-100 cosine, B=1, injection on: final + index 50
 
+Large outputs are stored as a seeded element subset (oracle/golden_subset.py) so that every file stays under 1 MB.
 While generating, the oracle restatement is checked against the reference wherever it has the mode
 (the script aborts on disagreement).  Inputs are regenerated from integer seeds by the tests.
 """
@@ -39,6 +40,7 @@ import fidm_b200  # noqa: E402,F401
 from fidm_b200.arch import CONFIGS  # noqa: E402
 from fidm_b200.utils.synth import merge_lora, synth_batch, synth_state_dict  # noqa: E402
 from oracle import diffusion_oracle as dor  # noqa: E402
+from oracle.golden_subset import shrink  # noqa: E402
 from oracle import unet_oracle as uor  # noqa: E402
 
 import gaussian_diffusion as ref_gd  # noqa: E402  (reference)
@@ -149,6 +151,7 @@ def golden_step_modes():
                                       eta=eta, clip=clip, seed=seed, sample=got["sample"].clone(),
                                       pred_xstart=got["pred_xstart"].clone(), mean=pmv["mean"].clone(),
                                       log_variance=pmv["log_variance"].clone(), variance=pmv["variance"].clone()))
+    cases = [shrink(c, ["sample", "pred_xstart", "mean", "log_variance", "variance"], 192) for c in cases]
     torch.save(cases, os.path.join(OUT, "sampler_steps_modes.pt"))
     print("sampler step mode cases:", len(cases))
 
@@ -243,6 +246,7 @@ def golden_t64_loop_variants():
     with SeqRandn(draw_order(T, schedule="low"), 63), torch.no_grad():
         fin = helper(wrap, d, data["masked_image"], data["mask"], "cpu", use_ddim=True, injection_schedule="low")
     out["helper_ddim_low"] = {"T": T, "seed_noise": 63, "final": fin.clone()}
+    out = {k: shrink(v, [a for a in ("final", "pred_xstart_mid") if a in v], 4096) for k, v in out.items()}
     out["_meta"] = {"seed_weights": 1, "seed_data": 14, "batch": 2}
     torch.save(out, os.path.join(OUT, "t64_loop_variants.pt"))
 
@@ -266,10 +270,11 @@ def loop_256(name, T, sched, *, ddim, seed_w, seed_d, seed_n, fname, check_oracl
                 trace[i] = {k: v.clone() for k, v in o.items()}
             if i % 10 == 0:
                 print(f"  {name} {fname}: step {i}/{T}  {time.time() - t0:.0f}s", flush=True)
-    torch.save({"config": name, "T": T, "sched": sched, "ddim": ddim, "seed_weights": seed_w, "seed_data": seed_d,
-                "seed_noise": seed_n, "final": trace[T - 1]["sample"], "mid_index": T // 2,
-                "pred_xstart_mid": trace[T // 2]["pred_xstart"], "sample_mid": trace[T // 2]["sample"],
-                "seconds_reference_cpu": time.time() - t0, "cpu_threads": torch.get_num_threads()},
+    torch.save(shrink({"config": name, "T": T, "sched": sched, "ddim": ddim, "seed_weights": seed_w, "seed_data": seed_d,
+                       "seed_noise": seed_n, "final": trace[T - 1]["sample"], "mid_index": T // 2,
+                       "pred_xstart_mid": trace[T // 2]["pred_xstart"], "sample_mid": trace[T // 2]["sample"],
+                       "seconds_reference_cpu": time.time() - t0, "cpu_threads": torch.get_num_threads()},
+                      ["final", "pred_xstart_mid", "sample_mid"], 24576),
                os.path.join(OUT, fname))
     print(name, fname, "written,", f"{time.time() - t0:.0f}s")
 
@@ -291,8 +296,9 @@ def golden_adm256_eval_b8():
     rel = ((out[:1] - mine).norm() / out[:1].norm()).item()
     print("ADM256 eval: oracle rel-L2 vs reference", rel)
     assert rel < 2e-6, rel
-    torch.save({"seed_weights": 7, "seed_data": 2, "seed_x": 3, "t": t, "stride": 2, "out_sub": out[:, :, ::2, ::2].clone(),
-                "norm_per_image": out.flatten(1).norm(dim=1)}, os.path.join(OUT, "adm256_eval_b8.pt"))
+    torch.save(shrink({"seed_weights": 7, "seed_data": 2, "seed_x": 3, "t": t, "stride": 2,
+                       "out_sub": out[:, :, ::2, ::2].clone(), "norm_per_image": out.flatten(1).norm(dim=1)},
+                      ["out_sub"], 12288, per_image=True), os.path.join(OUT, "adm256_eval_b8.pt"))
 
 
 def golden_adm256_lora_quad():
@@ -309,9 +315,10 @@ def golden_adm256_lora_quad():
             steps.append({k: v.clone() for k, v in o.items()})
             if i == 2:
                 break
-    torch.save({"seed_weights": 13, "lora": dict(rank=8, alpha=64.0, seed=13), "seed_data": 15, "seed_noise": seed, "T": T,
-                "sched": "quadratic", "n_steps": 3, "sample": steps[-1]["sample"], "pred_xstart": steps[-1]["pred_xstart"],
-                "pred_xstart_first": steps[0]["pred_xstart"]}, os.path.join(OUT, "adm256_lora_quad.pt"))
+    torch.save(shrink({"seed_weights": 13, "lora": dict(rank=8, alpha=64.0, seed=13), "seed_data": 15, "seed_noise": seed,
+                       "T": T, "sched": "quadratic", "n_steps": 3, "sample": steps[-1]["sample"],
+                       "pred_xstart": steps[-1]["pred_xstart"], "pred_xstart_first": steps[0]["pred_xstart"]},
+                      ["sample", "pred_xstart", "pred_xstart_first"], 24576), os.path.join(OUT, "adm256_lora_quad.pt"))
     print("adm256 lora quadratic written")
 
 
