@@ -14,6 +14,8 @@ LIB_PATH = os.environ.get("FIDM_LIB_PATH") or os.path.join(_HERE, "libfidm_b200.
 
 F32, BF16, F16, E4M3 = 0, 1, 2, 3
 COEF_COLS = 20
+MS_COLS = 7
+MS_X0_C1, MS_X0_C2, MS_A, MS_B0, MS_B1, MS_INJ_A, MS_INJ_S = range(7)
 STEP_INJECT_ONLY, STEP_UPDATE_ONLY, STEP_UPDATE_INJECT = 0, 1, 2
 SAMPLER_DDPM, SAMPLER_DDIM, SAMPLER_DDIM_SCRIPT = 0, 1, 2
 MEAN_PREVIOUS_X, MEAN_START_X, MEAN_EPSILON = 0, 1, 2
@@ -31,6 +33,14 @@ class StepArgs(C.Structure):
                 ("t_dev", vp), ("coef", fp), ("x", fp), ("model_out", fp), ("z", fp), ("gt", fp),
                 ("keep_mask", fp), ("inject_noise", fp), ("sample", fp), ("pred_xstart", fp),
                 ("x_next", fp), ("mean_out", fp), ("logvar_out", fp),
+                ("stem_out", vp), ("stem_dtype", i32), ("stem_ld", i32), ("t_out", fp), ("t_out_value", C.c_float)]
+
+
+class MultistepArgs(C.Structure):
+    _fields_ = [("batch", i32), ("channels", i32), ("hw", i32), ("mean_type", i32), ("out_channels", i32),
+                ("clip_denoised", i32), ("mask_channels", i32), ("steps", i32), ("step", i32),
+                ("coef", fp), ("x", fp), ("model_out", fp), ("m_prev", fp), ("m_out", fp), ("x_next", fp),
+                ("inject", i32), ("gt", fp), ("keep_mask", fp), ("inject_noise", fp),
                 ("stem_out", vp), ("stem_dtype", i32), ("stem_ld", i32), ("t_out", fp), ("t_out_value", C.c_float)]
 
 
@@ -74,6 +84,7 @@ SYMBOLS = {
     "fidm_last_error_string": (C.c_char_p, []),
     "fidm_device_supported": (C.c_int, [C.c_int]),
     "fidm_sampler_step": (C.c_int, [_P(StepArgs), vp]),
+    "fidm_multistep_step": (C.c_int, [_P(MultistepArgs), vp]),
     "fidm_pack_nchw_to_nhwc": (C.c_int, [_P(PackArgs), vp]),
     "fidm_unpack_nhwc_to_nchw": (C.c_int, [vp, i32, i32, fp, i32, i32, i32, vp]),
     "fidm_prepare_inputs_u8": (C.c_int, [vp, vp, fp, fp, fp, fp, i32, i32, vp]),

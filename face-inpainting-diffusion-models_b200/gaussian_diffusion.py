@@ -22,6 +22,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
+from . import dpm_solver
 from .losses import LossType, ModelMeanType, ModelVarType  # noqa: F401
 
 try:  # tqdm is only used when progress=True, as in the reference
@@ -267,6 +268,12 @@ class GaussianDiffusion:
             return t.float() * (1000.0 / self.num_timesteps)
         return t
 
+    def _t_value(self, ts):
+        """What the model sees for the integer timestep ts: _scale_timesteps (:321-324) in fp32 arithmetic."""
+        if self.rescale_timesteps:
+            return float(np.float32(ts) * np.float32(1000.0 / self.num_timesteps))
+        return float(ts)
+
     def _call_model(self, model, x, t, model_kwargs):
         out = model(x, self._scale_timesteps(t), **(model_kwargs or {}))
         return out
@@ -438,11 +445,7 @@ class GaussianDiffusion:
         def inj_noise(ts):
             return self._cached_noise(gt, ts) if use_cumulative_noise else torch.randn_like(gt)
 
-        def t_value(ts):      # what the model sees for timestep ts: _scale_timesteps (:321-324), fp32 arithmetic
-            if self.rescale_timesteps:
-                return float(np.float32(ts) * np.float32(1000.0 / self.num_timesteps))
-            return float(ts)
-
+        t_value = self._t_value
         B = shape[0]
         T = self.num_timesteps
         first = T - 1
@@ -525,6 +528,131 @@ class GaussianDiffusion:
         for final in self._loop(True, model, shape, noise, clip_denoised, denoised_fn, cond_fn, model_kwargs,
                                 device, progress, eta, use_inpainting_injection, injection_schedule,
                                 use_cumulative_noise, False):
+            pass
+        return final["sample"]
+
+    # ------------------------------------------------------------------ DPM-Solver++ multistep (K6)
+    def _dpm_table(self, device, steps, order, cumulative):
+        key = ("dpm", str(device), int(steps), int(order), bool(cumulative))
+        if key not in self._coef_cache:
+            self._coef_cache[key] = dpm_solver.coefficient_table(self, steps, order, cumulative).to(device)
+        return self._coef_cache[key]
+
+    def _multistep(self, tab, step, x, model_out, *, m_prev=None, want_next=True, clip=True, gt=None, keep=None,
+                   inject_noise=None, stem=None, t_next=None):
+        """One K6 launch with row `step` of the table `tab`: returns (m_k, state at t_{k+1} or None).  m_prev selects
+        the second-order update; gt / keep / inject_noise the injection; stem = (NHWC network input, timestep tensor)
+        of an engine plan receives the new state and `t_next` (step-boundary fusion, as in _step)."""
+        L.require_cuda(x, model_out, m_prev, gt, keep, inject_noise)
+        B, Cn = x.shape[0], x.shape[1]
+        model_out = model_out.detach()
+        if model_out.dtype != torch.float32 or not model_out.is_contiguous():
+            model_out = model_out.to(torch.float32).contiguous()
+        assert model_out.shape[0] == B and model_out.shape[2:] == x.shape[2:], tuple(model_out.shape)
+        a = L.MultistepArgs()
+        a.batch, a.channels, a.hw = B, Cn, x.numel() // (B * Cn)
+        a.mean_type, a.out_channels, a.clip_denoised = _MEAN_CODE[self.model_mean_type], model_out.shape[1], int(bool(clip))
+        a.steps, a.step = tab.shape[0], int(step)
+        m = torch.empty_like(x)
+        nxt = torch.empty_like(x) if want_next else None
+        a.coef, a.x, a.model_out, a.m_prev, a.m_out, a.x_next = (L.ptr(v) for v in (tab, x, model_out, m_prev, m, nxt))
+        a.mask_channels = 1
+        if gt is not None:
+            a.inject, a.mask_channels = 1, keep.shape[1]
+            a.gt, a.keep_mask, a.inject_noise = L.ptr(gt), L.ptr(keep), L.ptr(inject_noise)
+        if stem is not None:
+            x_in, t_in = stem
+            a.stem_out, a.stem_dtype, a.stem_ld = L.ptr(x_in), L.dtype_code(x_in.dtype), x_in.shape[-1]
+            if t_next is not None:
+                a.t_out, a.t_out_value = L.ptr(t_in), float(t_next)
+        try:
+            L.check(L.lib().fidm_multistep_step(C.byref(a), L.stream()), "multistep_step")
+        except ValueError as e:      # an argument the library refuses: the caller passed something this path cannot run
+            raise L.FidmError(str(e)) from None
+        return m, nxt
+
+    def _dpm_solver_loop(self, model, shape, steps, order, noise, clip_denoised, model_kwargs, device, progress,
+                         use_inpainting_injection, injection_schedule, use_cumulative_noise):
+        """Per evaluation one model call and ONE K6 launch (x0 prediction, update, injection, next stem input)."""
+        if self.model_mean_type == ModelMeanType.PREVIOUS_X:
+            raise NotImplementedError("DPM-Solver++ needs an eps or x0 prediction; PREVIOUS_X models are not supported")
+        grid = dpm_solver.timestep_grid(self.num_timesteps, steps)
+        orders = dpm_solver.step_orders(steps, order)
+        if device is None:
+            device = next(model.parameters()).device
+        assert isinstance(shape, (tuple, list))
+        img = noise if noise is not None else torch.randn(*shape, device=device)
+        L.require_cuda(img)
+        tab = self._dpm_table(img.device, steps, order, use_cumulative_noise)
+        mk = model_kwargs
+        gt = keep = None
+        if use_inpainting_injection and mk:
+            gt, keep = mk.get("gt"), mk.get("gt_keep_mask")
+        inject = gt is not None and keep is not None
+        if inject:
+            gt, keep = (v.detach().to(torch.float32).contiguous() for v in (gt, keep))
+
+        def inj_noise(ts):
+            return self._cached_noise(gt, ts) if use_cumulative_noise else torch.randn_like(gt)
+
+        B = shape[0]
+        plan = None
+        fused_plan = getattr(model, "fused_plan", None)
+        if fused_plan is not None and os.environ.get("FIDM_FUSED_STEP", "1") != "0":
+            plan = fused_plan(tuple(shape), img, self._t_value(int(grid[0])), mk)
+        stem = (plan.x_in, plan.t_in) if plan is not None else None
+        ks = range(steps)
+        if progress and tqdm is not None:
+            ks = tqdm(ks)
+        with torch.no_grad():
+            t0 = int(grid[0])
+            if inject and not self._injection_gated(t0, injection_schedule):      # injection on x_T itself
+                x = self._step(L.STEP_INJECT_ONLY, img, t_inject=t0, gt=gt, keep=keep, inject_noise=inj_noise(t0),
+                               cumulative=use_cumulative_noise, want_next=True, stem=stem)["x_next"]
+            else:
+                x = img.detach().to(torch.float32).contiguous()
+            m_prev = None
+            for k in ks:
+                if plan is not None:
+                    model_output = plan.run()                    # stem input and timestep are already in place
+                else:
+                    t = torch.full((B,), int(grid[k]), device=device, dtype=torch.long)
+                    model_output = self._call_model(model, x, t, mk)
+                if k == steps - 1:                               # t = 0: the sample is the x0 prediction
+                    m, _ = self._multistep(tab, k, x, model_output, want_next=False, clip=clip_denoised)
+                    yield {"sample": m, "pred_xstart": m}
+                    break
+                nxt = int(grid[k + 1])
+                do_inj = inject and not self._injection_gated(nxt, injection_schedule)
+                m, x = self._multistep(tab, k, x, model_output, m_prev=m_prev if orders[k] == 2 else None,
+                                       clip=clip_denoised, gt=gt if do_inj else None, keep=keep if do_inj else None,
+                                       inject_noise=inj_noise(nxt) if do_inj else None, stem=stem,
+                                       t_next=self._t_value(nxt))
+                m_prev = m
+                yield {"sample": x, "pred_xstart": m}
+
+    def dpm_solver_sample_loop_progressive(self, model, shape, steps=20, order=2, noise=None, clip_denoised=True,
+                                           model_kwargs=None, device=None, progress=False,
+                                           use_inpainting_injection=False, injection_schedule="all",
+                                           use_cumulative_noise=True):
+        """Generator over one dict {"sample", "pred_xstart"} per model evaluation of dpm_solver_sample_loop:
+        "sample" is the state the next evaluation sees (after the injection), and the x0 prediction at t = 0 for the
+        last one; "pred_xstart" is the x0 prediction of that evaluation.  Every yielded tensor is a fresh buffer."""
+        yield from self._dpm_solver_loop(model, shape, steps, order, noise, clip_denoised, model_kwargs, device,
+                                         progress, use_inpainting_injection, injection_schedule, use_cumulative_noise)
+
+    def dpm_solver_sample_loop(self, model, shape, steps=20, order=2, noise=None, clip_denoised=True,
+                               model_kwargs=None, device=None, progress=False, use_inpainting_injection=False,
+                               injection_schedule="all", use_cumulative_noise=True):
+        """DPM-Solver++ (multistep, `order` 1 or 2) in `steps` model evaluations on the timesteps
+        round(linspace(T - 1, 0, steps)) of this diffusion's own table, with the class path's known-region injection
+        (on x_T, then after every update) and RNG draw order (randn(shape), then one injection noise per injection;
+        the solver itself draws nothing).  Returns the x0 prediction at t = 0."""
+        self.clear_gt_noise_cache()
+        final = None
+        for final in self._dpm_solver_loop(model, shape, steps, order, noise, clip_denoised, model_kwargs, device,
+                                           progress, use_inpainting_injection, injection_schedule,
+                                           use_cumulative_noise):
             pass
         return final["sample"]
 

@@ -119,6 +119,50 @@ typedef struct fidm_step_args {
 int fidm_sampler_step(const fidm_step_args* a, fidm_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * K6  DPM-Solver++ multistep step (Lu et al. 2022, "DPM-Solver++", multistep 2M, data prediction):
+ *   m_k    = x0 prediction at t_k:  clamp(c1*x - c2*eps) (EPSILON) | clamp(model_out) (START_X)
+ *   x_next = A*x + B0*m_k [+ B1*m_{k-1}]                                    (update t_k -> t_{k+1})
+ *   x_next = keep*(ia*gt + is*n) + (1-keep)*x_next                          (optional injection at t_{k+1})
+ * The per-step rows are computed on the host in float64 and rounded to fp32 once (dpm_solver.py).  Every product and
+ * sum is one IEEE fp32 rounding, in the order written above; the injection and the stem write are K4's expressions.
+ * All tensors fp32 NCHW contiguous.
+ * ---------------------------------------------------------------------------------------------- */
+#define FIDM_MS_COLS 7
+/* columns of the per-step table [steps][FIDM_MS_COLS]; row k belongs to the evaluation at t_k */
+enum {
+  FIDM_MS_X0_C1 = 0,   /* sqrt_recip_alphas_cumprod[t_k]   (as FIDM_C_RECIP) */
+  FIDM_MS_X0_C2 = 1,   /* sqrt_recipm1_alphas_cumprod[t_k] (as FIDM_C_RECIPM1) */
+  FIDM_MS_A = 2,       /* sigma_{t_{k+1}} / sigma_{t_k} */
+  FIDM_MS_B0 = 3,      /* weight of m_k */
+  FIDM_MS_B1 = 4,      /* weight of m_{k-1} (second-order rows) */
+  FIDM_MS_INJ_A = 5,   /* injection coefficient of gt at t_{k+1} (cumulative: FIDM_C_SQRT_AB, else FIDM_C_SQRT_AB_F32) */
+  FIDM_MS_INJ_S = 6    /* injection coefficient of the noise at t_{k+1} */
+};
+typedef struct fidm_multistep_args {
+  int32_t batch, channels, hw;          /* x is [batch][channels][hw] */
+  int32_t mean_type;                    /* FIDM_MEAN_EPSILON | FIDM_MEAN_START_X */
+  int32_t out_channels;                 /* channels of model_out: channels or 2*channels (learned variance, ignored) */
+  int32_t clip_denoised;                /* clamp m_k to [-1,1] */
+  int32_t mask_channels;                /* 1 (broadcast) or `channels` */
+  int32_t steps, step;                  /* rows of coef, and the row of this call (0 <= step < steps) */
+  const float* coef;                    /* device [steps][FIDM_MS_COLS] */
+  const float* x;                       /* state at t_k, the model's input */
+  const float* model_out;               /* [batch][out_channels][hw] */
+  const float* m_prev;                  /* m_{k-1}; NULL selects the first-order update (B1 is not used) */
+  float* m_out;                         /* m_k (the next step's history; pred_xstart) */
+  float* x_next;                        /* state at t_{k+1}; NULL: no update (the last evaluation, at t = 0) */
+  int32_t inject;                       /* 1: injection at t_{k+1} (needs gt, keep_mask, inject_noise, x_next) */
+  const float* gt;                      /* [batch][channels][hw] */
+  const float* keep_mask;               /* 1 = keep, [batch][mask_channels][hw] */
+  const float* inject_noise;            /* n_{t_{k+1}} */
+  /* step-boundary fusion, as fidm_step_args: x_next is also stored as channels [0, channels) of the NHWC network
+   * input `stem_out` (needs x_next), and t_out[0 .. batch) = t_out_value */
+  void* stem_out; int32_t stem_dtype, stem_ld;
+  float* t_out; float t_out_value;
+} fidm_multistep_args;
+int fidm_multistep_step(const fidm_multistep_args* a, fidm_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Layout converters.  Replace torch.cat([x, masked_image, mask.repeat(1,3,1,1)], 1) of
  * unet.py:199 and the NCHW activations of the reference with one NHWC (bf16|fp32) tensor padded to
  * `c_pad` channels (zeros).  Up to 3 fp32 NCHW sources; a source with repeat>1 is broadcast.
