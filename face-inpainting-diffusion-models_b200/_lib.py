@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("FIDM_LIB_PATH") or os.path.join(_HERE, "libfidm_b200.
 
 F32, BF16, F16, E4M3 = 0, 1, 2, 3
 COEF_COLS = 20
+C_SQRT_AB, C_SQRT_1MAB, C_SQRT_AB_F32, C_SQRT_1MAB_F32 = range(4)
 MS_COLS = 7
 MS_X0_C1, MS_X0_C2, MS_A, MS_B0, MS_B1, MS_INJ_A, MS_INJ_S = range(7)
 STEP_INJECT_ONLY, STEP_UPDATE_ONLY, STEP_UPDATE_INJECT = 0, 1, 2
@@ -41,6 +42,14 @@ class MultistepArgs(C.Structure):
                 ("clip_denoised", i32), ("mask_channels", i32), ("steps", i32), ("step", i32),
                 ("coef", fp), ("x", fp), ("model_out", fp), ("m_prev", fp), ("m_out", fp), ("x_next", fp),
                 ("inject", i32), ("gt", fp), ("keep_mask", fp), ("inject_noise", fp),
+                ("stem_out", vp), ("stem_dtype", i32), ("stem_ld", i32), ("t_out", fp), ("t_out_value", C.c_float)]
+
+
+class ResampleArgs(C.Structure):
+    _fields_ = [("batch", i32), ("channels", i32), ("hw", i32), ("mask_channels", i32),
+                ("undo_a", C.c_float), ("undo_s", C.c_float), ("x", fp), ("noise", fp), ("x_next", fp),
+                ("inject", i32), ("inject_a", C.c_float), ("inject_s", C.c_float),
+                ("gt", fp), ("keep_mask", fp), ("inject_noise", fp),
                 ("stem_out", vp), ("stem_dtype", i32), ("stem_ld", i32), ("t_out", fp), ("t_out_value", C.c_float)]
 
 
@@ -85,6 +94,7 @@ SYMBOLS = {
     "fidm_device_supported": (C.c_int, [C.c_int]),
     "fidm_sampler_step": (C.c_int, [_P(StepArgs), vp]),
     "fidm_multistep_step": (C.c_int, [_P(MultistepArgs), vp]),
+    "fidm_resample_undo": (C.c_int, [_P(ResampleArgs), vp]),
     "fidm_pack_nchw_to_nhwc": (C.c_int, [_P(PackArgs), vp]),
     "fidm_unpack_nhwc_to_nchw": (C.c_int, [vp, i32, i32, fp, i32, i32, i32, vp]),
     "fidm_prepare_inputs_u8": (C.c_int, [vp, vp, fp, fp, fp, fp, i32, i32, vp]),

@@ -22,7 +22,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from . import dpm_solver
+from . import dpm_solver, repaint
 from .losses import LossType, ModelMeanType, ModelVarType  # noqa: F401
 
 try:  # tqdm is only used when progress=True, as in the reference
@@ -653,6 +653,158 @@ class GaussianDiffusion:
         for final in self._dpm_solver_loop(model, shape, steps, order, noise, clip_denoised, model_kwargs, device,
                                            progress, use_inpainting_injection, injection_schedule,
                                            use_cumulative_noise):
+            pass
+        return final["sample"]
+
+    # ------------------------------------------------------------------ RePaint resampling (K4 + K7)
+    def _resample(self, x, u, undo_a, undo_s, *, t_inject=None, gt=None, keep=None, inject_noise=None, cumulative=True,
+                  stem=None, t_next=None, next_buf=None):
+        """One K7 launch: x' = undo_a*x + undo_s*u, then (t_inject not None) the injection at t_inject with the class
+        table's coefficients; stem = (NHWC network input, timestep tensor) of an engine plan receives the new state and
+        `t_next` (step-boundary fusion, as in _step).  Returns the new state (next_buf when given)."""
+        L.require_cuda(x, u, gt, keep, inject_noise)
+        keepalive = []
+
+        def c(tn):
+            tn = tn.detach()
+            if tn.dtype != torch.float32 or not tn.is_contiguous():
+                tn = tn.to(torch.float32).contiguous()
+            keepalive.append(tn)
+            return tn
+
+        x, u = c(x), c(u)
+        assert u.shape == x.shape, (tuple(u.shape), tuple(x.shape))
+        B, Cn = x.shape[0], x.shape[1]
+        a = L.ResampleArgs()
+        a.batch, a.channels, a.hw = B, Cn, x.numel() // (B * Cn)
+        a.undo_a, a.undo_s = float(undo_a), float(undo_s)
+        out = next_buf if next_buf is not None else torch.empty_like(x)
+        a.x, a.noise, a.x_next = L.ptr(x), L.ptr(u), L.ptr(out)
+        a.mask_channels = 1
+        if t_inject is not None:
+            gt, keep, inject_noise = c(gt), c(keep), c(inject_noise)
+            assert gt.shape == x.shape and inject_noise.shape == x.shape
+            assert keep.shape[0] == B and keep.shape[2:] == x.shape[2:], tuple(keep.shape)
+            if "host" not in self._coef_cache:
+                self._coef_cache["host"] = self.coefficient_table(0.0)
+            cls = self._coef_cache["host"]
+            ia, is_ = (L.C_SQRT_AB, L.C_SQRT_1MAB) if cumulative else (L.C_SQRT_AB_F32, L.C_SQRT_1MAB_F32)
+            a.inject, a.mask_channels = 1, keep.shape[1]
+            a.inject_a, a.inject_s = float(cls[t_inject, ia]), float(cls[t_inject, is_])
+            a.gt, a.keep_mask, a.inject_noise = L.ptr(gt), L.ptr(keep), L.ptr(inject_noise)
+        if stem is not None:
+            x_in, t_in = stem
+            a.stem_out, a.stem_dtype, a.stem_ld = L.ptr(x_in), L.dtype_code(x_in.dtype), x_in.shape[-1]
+            if t_next is not None:
+                a.t_out, a.t_out_value = L.ptr(t_in), float(t_next)
+        try:
+            L.check(L.lib().fidm_resample_undo(C.byref(a), L.stream()), "resample_undo")
+        except ValueError as e:      # an argument the library refuses: the caller passed something this path cannot run
+            raise L.FidmError(str(e)) from None
+        return out
+
+    def _repaint_plan(self, jump_length, jump_n_sample, model_kwargs, use_inpainting_injection):
+        """The evaluation plan, after every argument check (raises ValueError before any RNG draw or GPU work)."""
+        plan = repaint.evaluation_plan(self.alphas_cumprod, jump_length, jump_n_sample)
+        if not use_inpainting_injection:
+            raise ValueError("RePaint resampling needs the known-region injection (use_inpainting_injection=True)")
+        if not model_kwargs or model_kwargs.get("gt") is None or model_kwargs.get("gt_keep_mask") is None:
+            raise ValueError("RePaint resampling needs model_kwargs with 'gt' and 'gt_keep_mask'")
+        return plan
+
+    def _repaint_loop(self, evals, model, shape, noise, clip_denoised, model_kwargs, device, progress,
+                      injection_schedule, use_cumulative_noise, progressive):
+        """Per evaluation one model call and one K4 launch; when a jump follows the evaluation, K4 only updates and
+        one K7 launch re-noises to t_up, injects at t_up and writes the next stem input."""
+        if device is None:
+            device = next(model.parameters()).device
+        assert isinstance(shape, (tuple, list))
+        img = noise if noise is not None else torch.randn(*shape, device=device)
+        L.require_cuda(img)
+        mk = model_kwargs
+        gt, keep = mk["gt"], mk["gt_keep_mask"]
+
+        def inj_noise(ts):
+            return self._cached_noise(gt, ts) if use_cumulative_noise else torch.randn_like(gt)
+
+        t_value = self._t_value
+        B = shape[0]
+        first = evals[0].t
+        plan = None
+        fused_plan = getattr(model, "fused_plan", None)
+        if fused_plan is not None and os.environ.get("FIDM_FUSED_STEP", "1") != "0":
+            plan = fused_plan(tuple(shape), img, t_value(first), mk)
+        stem = (plan.x_in, plan.t_in) if plan is not None else None
+        bufs = [torch.empty_like(img), torch.empty_like(img)] if plan is not None else None
+        if progress and tqdm is not None:
+            evals = tqdm(evals)
+        with torch.no_grad():
+            # injection for the first evaluation happens on x_T itself
+            if not self._injection_gated(first, injection_schedule):
+                x = self._step(L.STEP_INJECT_ONLY, img, t_inject=first, gt=gt, keep=keep,
+                               inject_noise=inj_noise(first), cumulative=use_cumulative_noise,
+                               want_next=True, stem=stem, next_buf=bufs[0] if bufs else None)["x_next"]
+            else:
+                x = img
+            for k, (i, t_up, undo_a, undo_s) in enumerate(evals):
+                if plan is not None:
+                    model_output = plan.run()                        # stem input and timestep are already in place
+                else:
+                    t = torch.full((B,), i, device=device, dtype=torch.long)
+                    model_output = self._call_model(model, x, t, mk)
+                z = torch.randn_like(x)                              # RNG order: z_t, [u], then n of the next t
+                want_out = progressive or i == 0
+                nbuf = bufs[(k + 1) & 1] if bufs else None
+                if t_up is None:                                     # as _loop's DDPM step
+                    nxt = i - 1
+                    do_inj = nxt >= 0 and not self._injection_gated(nxt, injection_schedule)
+                    r = self._step(L.STEP_UPDATE_INJECT if do_inj else L.STEP_UPDATE_ONLY, x, t=i, t_inject=nxt,
+                                   model_out=model_output, z=z, gt=gt if do_inj else None,
+                                   keep=keep if do_inj else None, inject_noise=inj_noise(nxt) if do_inj else None,
+                                   ddim=False, clip=clip_denoised, cumulative=use_cumulative_noise,
+                                   want_sample=want_out or (not do_inj and plan is None), want_x0=want_out,
+                                   want_next=do_inj or plan is not None,
+                                   stem=stem if nxt >= 0 else None, t_next=t_value(nxt) if nxt >= 0 else None,
+                                   next_buf=nbuf)
+                    x = r["x_next"] if (do_inj or plan is not None) else r["sample"]
+                else:
+                    r = self._step(L.STEP_UPDATE_ONLY, x, t=i, model_out=model_output, z=z, ddim=False,
+                                   clip=clip_denoised, want_sample=True, want_x0=want_out)
+                    u = torch.randn_like(x)
+                    do_inj = not self._injection_gated(t_up, injection_schedule)
+                    x = self._resample(r["sample"], u, undo_a, undo_s, t_inject=t_up if do_inj else None,
+                                       gt=gt, keep=keep, inject_noise=inj_noise(t_up) if do_inj else None,
+                                       cumulative=use_cumulative_noise, stem=stem, t_next=t_value(t_up),
+                                       next_buf=nbuf)
+                if want_out:
+                    yield {"sample": r["sample"], "pred_xstart": r["pred_xstart"], "t": i}
+
+    def repaint_sample_loop_progressive(self, model, shape, jump_length=10, jump_n_sample=10, noise=None,
+                                        clip_denoised=True, model_kwargs=None, device=None, progress=False,
+                                        use_inpainting_injection=True, injection_schedule="all",
+                                        use_cumulative_noise=True):
+        """Generator over one dict {"sample", "pred_xstart", "t"} per model evaluation of repaint_sample_loop:
+        "sample" is the DDPM output of the evaluation at timestep "t", before any undo or injection.  The arguments
+        are checked when this is called, before the first draw."""
+        evals = self._repaint_plan(jump_length, jump_n_sample, model_kwargs, use_inpainting_injection)
+        return self._repaint_loop(evals, model, shape, noise, clip_denoised, model_kwargs, device, progress,
+                                  injection_schedule, use_cumulative_noise, True)
+
+    def repaint_sample_loop(self, model, shape, jump_length=10, jump_n_sample=10, noise=None, clip_denoised=True,
+                            model_kwargs=None, device=None, progress=False, use_inpainting_injection=True,
+                            injection_schedule="all", use_cumulative_noise=True):
+        """DDPM sampling with RePaint resampling (Lugmayr et al. 2022): the class path's DDPM step and known-region
+        injection, on RePaint's jump schedule (repaint.py) -- every `jump_length` timesteps the state is re-noised
+        back up `jump_length` levels and denoised again, `jump_n_sample - 1` times, so that the hole can agree with
+        the known region.  T + (jump_n_sample - 1) * jump_length * len(range(0, T - jump_length, jump_length)) model
+        evaluations.  RNG draw order: randn(shape), the injection noise at T - 1, then per evaluation the step noise,
+        the undo noise if a jump follows, and the injection noise of the next evaluation (with use_cumulative_noise
+        a revisited timestep reuses its cached noise).  Returns the sample at t = 0, not re-blended."""
+        evals = self._repaint_plan(jump_length, jump_n_sample, model_kwargs, use_inpainting_injection)
+        self.clear_gt_noise_cache()
+        final = None
+        for final in self._repaint_loop(evals, model, shape, noise, clip_denoised, model_kwargs, device, progress,
+                                        injection_schedule, use_cumulative_noise, False):
             pass
         return final["sample"]
 

@@ -38,9 +38,17 @@ def gather_batch(local, batch):
     return torch.cat([bufs[r][: b - a] for r, (a, b) in enumerate(sizes)], dim=0)
 
 
-def sample_sharded(diffusion, model_fn, gt, gt_keep_mask, *, ddim=True, eta=0.0, seed=0, **loop_kwargs):
+def sample_sharded(diffusion, model_fn, gt, gt_keep_mask, *, ddim=True, eta=0.0, seed=0, sampler=None, **loop_kwargs):
     """Run the inpainting loop on this rank's slice of (gt, gt_keep_mask) and gather the results.
-    Per-rank generator seed = seed + rank (parity is checked shard by shard against the oracle)."""
+    Per-rank generator seed = seed + rank (parity is checked shard by shard against the oracle).
+    sampler: "ddim" | "ddpm" | "dpm_solver" | "repaint" (None: "ddim" if `ddim` else "ddpm"); `eta` is used by
+    "ddim" only, and loop_kwargs go to the chosen loop (steps / order, jump_length / jump_n_sample, ...)."""
+    if sampler is None:
+        sampler = "ddim" if ddim else "ddpm"
+    loops = {"ddim": diffusion.ddim_sample_loop, "ddpm": diffusion.p_sample_loop,
+             "dpm_solver": diffusion.dpm_solver_sample_loop, "repaint": diffusion.repaint_sample_loop}
+    if sampler not in loops:
+        raise ValueError(f"sampler must be one of {sorted(loops)}, got {sampler!r}")
     rank = dist.get_rank() if dist.is_initialized() else 0
     world = dist.get_world_size() if dist.is_initialized() else 1
     if gt.shape[0] < world:
@@ -50,8 +58,7 @@ def sample_sharded(diffusion, model_fn, gt, gt_keep_mask, *, ddim=True, eta=0.0,
     torch.manual_seed(seed + rank)
     if g.is_cuda:
         torch.cuda.manual_seed(seed + rank)
-    loop = diffusion.ddim_sample_loop if ddim else diffusion.p_sample_loop
-    extra = {"eta": eta} if ddim else {}
-    out = loop(model_fn, tuple(g.shape), model_kwargs={"gt": g, "gt_keep_mask": k}, device=g.device,
-               use_inpainting_injection=True, **extra, **loop_kwargs)
+    extra = {"eta": eta} if sampler == "ddim" else {}
+    out = loops[sampler](model_fn, tuple(g.shape), model_kwargs={"gt": g, "gt_keep_mask": k}, device=g.device,
+                         use_inpainting_injection=True, **extra, **loop_kwargs)
     return gather_batch(out, gt.shape[0])

@@ -163,6 +163,35 @@ typedef struct fidm_multistep_args {
 int fidm_multistep_step(const fidm_multistep_args* a, fidm_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * K7  RePaint undo-and-inject (Lugmayr et al. 2022, "RePaint", Algorithm 1): after the DDPM update of the evaluation
+ * at t (K4, STEP_UPDATE_ONLY) the state x at level t-1 is re-noised to level t_up in one draw and the known region is
+ * injected for the next evaluation, at t_up:
+ *   x'  = undo_a*x + undo_s*u                                undo_a = sqrt(ab[t_up]/ab[t-1]), undo_s = sqrt(1 - ab[t_up]/ab[t-1])
+ *   x'' = keep*(inject_a*gt + inject_s*n) + (1-keep)*x'      (optional: injection at t_up, K4's expression)
+ * The coefficients are fp32 values the host computes (repaint.py: float64 rounded once; the injection pair is the
+ * class table's FIDM_C_SQRT_AB/FIDM_C_SQRT_1MAB columns for cumulative noise, the _F32 columns otherwise).  Every
+ * product and sum is one IEEE fp32 rounding, in the order written above.  All tensors fp32 NCHW contiguous.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct fidm_resample_args {
+  int32_t batch, channels, hw;          /* x is [batch][channels][hw] */
+  int32_t mask_channels;                /* 1 (broadcast) or `channels` */
+  float undo_a, undo_s;
+  const float* x;                       /* state at level t-1 (K4's "sample") */
+  const float* noise;                   /* u, the undo noise */
+  float* x_next;                        /* state the evaluation at t_up sees */
+  int32_t inject;                       /* 1: injection at t_up (needs gt, keep_mask, inject_noise) */
+  float inject_a, inject_s;
+  const float* gt;                      /* [batch][channels][hw] */
+  const float* keep_mask;               /* 1 = keep, [batch][mask_channels][hw] */
+  const float* inject_noise;            /* n_{t_up} */
+  /* step-boundary fusion, as fidm_step_args: x_next is also stored as channels [0, channels) of the NHWC network
+   * input `stem_out`, and t_out[0 .. batch) = t_out_value */
+  void* stem_out; int32_t stem_dtype, stem_ld;
+  float* t_out; float t_out_value;
+} fidm_resample_args;
+int fidm_resample_undo(const fidm_resample_args* a, fidm_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Layout converters.  Replace torch.cat([x, masked_image, mask.repeat(1,3,1,1)], 1) of
  * unet.py:199 and the NCHW activations of the reference with one NHWC (bf16|fp32) tensor padded to
  * `c_pad` channels (zeros).  Up to 3 fp32 NCHW sources; a source with repeat>1 is broadcast.
