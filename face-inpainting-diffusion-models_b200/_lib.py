@@ -124,6 +124,10 @@ class FidmError(RuntimeError):
     pass
 
 
+class ArgumentError(FidmError, ValueError):
+    """An argument the library refuses (negative status): a FidmError, and a ValueError like any bad argument."""
+
+
 def lib():
     """The loaded shared library; raises if it has not been built (no fallback path exists)."""
     global _lib
@@ -149,7 +153,7 @@ def check(rc, what=""):
         return
     msg = lib().fidm_last_error_string().decode(errors="replace")
     if rc < 0:
-        raise ValueError(f"fidm {what}: {msg} (code {rc})")
+        raise ArgumentError(f"fidm {what}: {msg} (code {rc})")
     raise FidmError(f"fidm {what}: CUDA error {rc}: {msg}")
 
 

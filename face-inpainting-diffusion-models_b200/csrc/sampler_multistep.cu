@@ -6,7 +6,7 @@
 //
 // Rounding contract (as sampler_step.cu): every product and sum is an explicit __fmul_rn / __fadd_rn / __fsub_rn, so
 // the compiler may not contract them into FMAs and oracle/dpm_solver_oracle.py can mirror the kernel bit for bit.
-#include "common.cuh"
+#include "sampler_common.cuh"
 
 namespace fidm {
 
@@ -30,14 +30,9 @@ __global__ void __launch_bounds__(256) multistep_step_kernel(const MultistepPara
   const long long total = (long long)a.batch * a.channels * hw_v;
   for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
-    const int pv = (int)(idx % hw_v);
-    const int bc = (int)(idx / hw_v);
-    const int c = bc % a.channels;
-    const int b = bc / a.channels;
-    const long long off = ((long long)b * a.channels + c) * a.hw + (long long)pv * VEC;
-    const long long ooff = ((long long)b * a.out_channels + c) * a.hw + (long long)pv * VEC;
-    const int mc = (a.mask_channels == 1) ? 0 : c;
-    const long long moff = ((long long)b * a.mask_channels + mc) * a.hw + (long long)pv * VEC;
+    const SamplerElem e = sampler_elem<VEC>(idx, a.channels, a.hw, a.mask_channels);
+    const long long off = e.off;
+    const long long ooff = ((long long)e.b * a.out_channels + e.c) * a.hw + (long long)e.pv * VEC;
 
     // every load of this element is issued before any arithmetic (one memory round trip)
     float xs[VEC], mo[VEC], mp[VEC], g[VEC], n[VEC], m[VEC];
@@ -47,7 +42,7 @@ __global__ void __launch_bounds__(256) multistep_step_kernel(const MultistepPara
     if (inj) {
       load_vec<float, VEC>(a.gt + off, g);
       load_vec<float, VEC>(a.inject_noise + off, n);
-      load_vec<float, VEC>(a.keep_mask + moff, m);
+      load_vec<float, VEC>(a.keep_mask + e.moff, m);
     }
 
     float x0[VEC];
@@ -64,25 +59,10 @@ __global__ void __launch_bounds__(256) multistep_step_kernel(const MultistepPara
     for (int i = 0; i < VEC; ++i) {
       float v = __fadd_rn(__fmul_rn(kA, xs[i]), __fmul_rn(kB0, x0[i]));
       if (second) v = __fadd_rn(v, __fmul_rn(kB1, mp[i]));
-      if (inj) {  // K4's injection: x = m*wg + (1-m)*x, wg = a*gt + s*n
-        const float wg = __fadd_rn(__fmul_rn(ca, g[i]), __fmul_rn(cs, n[i]));
-        v = __fadd_rn(__fmul_rn(m[i], wg), __fmul_rn(__fsub_rn(1.0f, m[i]), v));
-      }
-      xn[i] = v;
+      xn[i] = inj ? inject(v, m[i], g[i], n[i], ca, cs) : v;
     }
     store_vec<float, VEC>(a.x_next + off, xn);
-    // step-boundary fusion: the next evaluation's stem channels, with the pack kernel's roundings (as K4)
-    if (a.stem_out) {
-      const long long px = (long long)b * a.hw + (long long)pv * VEC;
-#pragma unroll
-      for (int i = 0; i < VEC; ++i) {
-        const long long e = (px + i) * a.stem_ld + c;
-        if (a.stem_dtype == FIDM_F16) reinterpret_cast<__half*>(a.stem_out)[e] = from_f32<__half>(xn[i]);
-        else if (a.stem_dtype == FIDM_BF16) reinterpret_cast<__nv_bfloat16*>(a.stem_out)[e] = from_f32<__nv_bfloat16>(xn[i]);
-        else reinterpret_cast<float*>(a.stem_out)[e] = xn[i];
-      }
-    }
-    if (a.t_out && idx < a.batch) a.t_out[idx] = a.t_out_value;
+    write_stem<VEC>(a, idx, e, xn);
   }
 }
 
@@ -105,27 +85,14 @@ extern "C" int fidm_multistep_step(const fidm_multistep_args* a, fidm_stream_t s
     FIDM_REQUIRE(a->x_next != nullptr, FIDM_E_BADARG, "multistep_step: an injection needs x_next");
     FIDM_REQUIRE(a->gt && a->keep_mask && a->inject_noise, FIDM_E_BADARG,
                  "multistep_step: gt/keep_mask/inject_noise required for an injection");
-    FIDM_REQUIRE(a->mask_channels == 1 || a->mask_channels == a->channels, FIDM_E_BADARG,
-                 "multistep_step: mask_channels must be 1 or channels");
+    if (int rc = check_mask_channels(a, "multistep_step")) return rc;
   }
-  if (a->stem_out)
-    FIDM_REQUIRE(a->x_next != nullptr && a->stem_ld >= a->channels &&
-                     (a->stem_dtype == FIDM_F32 || a->stem_dtype == FIDM_BF16 || a->stem_dtype == FIDM_F16),
-                 FIDM_E_BADARG, "multistep_step: stem_out needs x_next, stem_ld >= channels and a dtype of F32 | BF16 | F16");
+  FIDM_REQUIRE(a->stem_out == nullptr || a->x_next != nullptr, FIDM_E_BADARG, "multistep_step: stem_out needs x_next");
+  if (int rc = check_stem(a, "multistep_step")) return rc;
   MultistepParams p;
   p.a = *a;
-  const bool vec4 = (a->hw % 4 == 0) && (((uintptr_t)a->x | (uintptr_t)a->model_out | (uintptr_t)a->m_prev |
-                                          (uintptr_t)a->m_out | (uintptr_t)a->x_next | (uintptr_t)a->gt |
-                                          (uintptr_t)a->keep_mask | (uintptr_t)a->inject_noise) % 16 == 0);
-  const long long total = (long long)a->batch * a->channels * (a->hw / (vec4 ? 4 : 1));
-  long long blocks = (total + 255) / 256;
-  const long long cap = (long long)num_sms() * 16;
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
-  if (vec4)
-    multistep_step_kernel<4><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(p);
-  else
-    multistep_step_kernel<1><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(p);
-  FIDM_CHECK_LAUNCH("multistep_step");
-  return 0;
+  const bool vec4 = vec4_ok(a->hw, a->x, a->model_out, a->m_prev, a->m_out, a->x_next, a->gt, a->keep_mask,
+                            a->inject_noise);
+  return launch_sampler(multistep_step_kernel<4>, multistep_step_kernel<1>, vec4,
+                        (long long)a->batch * a->channels * a->hw, p, stream, "multistep_step");
 }

@@ -9,7 +9,7 @@
 // sum below is an explicit __fmul_rn/__fadd_rn/__fsub_rn/__fdiv_rn -- the compiler may not contract
 // them into FMAs.  With identical model output and noise the DDIM path is bit-identical to the
 // reference; the DDPM path differs only by the ulp of expf.
-#include "common.cuh"
+#include "sampler_common.cuh"
 
 namespace fidm {
 
@@ -26,11 +26,9 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams p) {
   const long long total = (long long)a.batch * a.channels * hw_v;
   for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
-    const int pv = (int)(idx % hw_v);
-    const int bc = (int)(idx / hw_v);
-    const int c = bc % a.channels;
-    const int b = bc / a.channels;
-    const long long off = ((long long)b * a.channels + c) * a.hw + (long long)pv * VEC;
+    const SamplerElem e = sampler_elem<VEC>(idx, a.channels, a.hw, a.mask_channels);
+    const int b = e.b, c = e.c;
+    const long long off = e.off;
 
     int t_upd = a.t_update, t_inj = a.t_inject;
     if (a.t_dev) {
@@ -45,9 +43,7 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams p) {
     const bool need_var = upd && a.var_type != FIDM_VAR_FIXED && (a.sampler == FIDM_SAMPLER_DDPM || a.logvar_out != nullptr);
     const bool need_z = upd && (a.z != nullptr);
     const int oc = (a.var_type == FIDM_VAR_FIXED) ? a.channels : 2 * a.channels;
-    const long long ooff = ((long long)b * oc + c) * a.hw + (long long)pv * VEC;
-    const int mc = (a.mask_channels == 1) ? 0 : c;
-    const long long moff = ((long long)b * a.mask_channels + mc) * a.hw + (long long)pv * VEC;
+    const long long ooff = ((long long)b * oc + c) * a.hw + (long long)e.pv * VEC;
     float xs[VEC], mo[VEC], vv[VEC], zz[VEC], g[VEC], n[VEC], m[VEC];
     load_vec<float, VEC>(a.x + off, xs);
     if (upd) load_vec<float, VEC>(a.model_out + ooff, mo);
@@ -56,7 +52,7 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams p) {
     if (inj) {
       load_vec<float, VEC>(a.gt + off, g);
       load_vec<float, VEC>(a.inject_noise + off, n);
-      load_vec<float, VEC>(a.keep_mask + moff, m);
+      load_vec<float, VEC>(a.keep_mask + e.moff, m);
     }
     float smp[VEC], x0v[VEC];
 
@@ -129,37 +125,16 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams p) {
       for (int i = 0; i < VEC; ++i) smp[i] = xs[i];
     }
 
-    if (a.mode != FIDM_STEP_UPDATE_ONLY) {
-      // apply_inpainting_injection (:139-155): x = m*wg + (1-m)*x, wg = a*gt + s*n
+    if (inj) {
+      // apply_inpainting_injection (:139-155)
       const float* cf = a.coef + (long long)t_inj * FIDM_COEF_COLS;
       const float ca = a.cumulative ? cf[FIDM_C_SQRT_AB] : cf[FIDM_C_SQRT_AB_F32];
       const float cs = a.cumulative ? cf[FIDM_C_SQRT_1MAB] : cf[FIDM_C_SQRT_1MAB_F32];
-      float xn[VEC];
 #pragma unroll
-      for (int i = 0; i < VEC; ++i) {
-        const float wg = __fadd_rn(__fmul_rn(ca, g[i]), __fmul_rn(cs, n[i]));
-        xn[i] = __fadd_rn(__fmul_rn(m[i], wg), __fmul_rn(__fsub_rn(1.0f, m[i]), smp[i]));
-      }
-      if (a.x_next) store_vec<float, VEC>(a.x_next + off, xn);
-#pragma unroll
-      for (int i = 0; i < VEC; ++i) smp[i] = xn[i];
-    } else if (a.x_next) {
-      store_vec<float, VEC>(a.x_next + off, smp);
+      for (int i = 0; i < VEC; ++i) smp[i] = inject(smp[i], m[i], g[i], n[i], ca, cs);
     }
-    // Step-boundary fusion: the next evaluation's stem input (channel c of every pixel of the NHWC network input) and
-    // its timestep are written here -- the same roundings as the pack kernel (layout.cu), so the fused loop is
-    // bit-identical to pack + evaluate.
-    if (a.stem_out) {
-      const long long px = (long long)b * a.hw + (long long)pv * VEC;
-#pragma unroll
-      for (int i = 0; i < VEC; ++i) {
-        const long long e = (px + i) * a.stem_ld + c;
-        if (a.stem_dtype == FIDM_F16) reinterpret_cast<__half*>(a.stem_out)[e] = from_f32<__half>(smp[i]);
-        else if (a.stem_dtype == FIDM_BF16) reinterpret_cast<__nv_bfloat16*>(a.stem_out)[e] = from_f32<__nv_bfloat16>(smp[i]);
-        else reinterpret_cast<float*>(a.stem_out)[e] = smp[i];
-      }
-    }
-    if (a.t_out && idx < a.batch) a.t_out[idx] = a.t_out_value;
+    if (a.x_next) store_vec<float, VEC>(a.x_next + off, smp);
+    write_stem<VEC>(a, idx, e, smp);
   }
 }
 
@@ -171,8 +146,7 @@ extern "C" int fidm_sampler_step(const fidm_step_args* a, fidm_stream_t stream) 
   FIDM_REQUIRE(a->batch > 0 && a->channels > 0 && a->hw > 0, FIDM_E_BADARG, "sampler_step: empty shape");
   FIDM_REQUIRE(a->mode >= 0 && a->mode <= 2, FIDM_E_BADARG, "sampler_step: bad mode %d", a->mode);
   FIDM_REQUIRE(a->coef && a->x, FIDM_E_BADARG, "sampler_step: coef/x are required");
-  FIDM_REQUIRE(a->mask_channels == 1 || a->mask_channels == a->channels, FIDM_E_BADARG,
-               "sampler_step: mask_channels must be 1 or channels");
+  if (int rc = check_mask_channels(a, "sampler_step")) return rc;
   if (a->mode != FIDM_STEP_INJECT_ONLY) {
     FIDM_REQUIRE(a->model_out != nullptr, FIDM_E_BADARG, "sampler_step: model_out required for an update");
     FIDM_REQUIRE(a->t_dev || (a->t_update >= 0 && a->t_update < a->num_timesteps), FIDM_E_BADARG,
@@ -184,24 +158,11 @@ extern "C" int fidm_sampler_step(const fidm_step_args* a, fidm_stream_t stream) 
     FIDM_REQUIRE(a->t_dev || (a->t_inject >= 0 && a->t_inject < a->num_timesteps), FIDM_E_BADARG,
                  "sampler_step: t_inject %d out of range [0,%d)", a->t_inject, a->num_timesteps);
   }
-  if (a->stem_out)
-    FIDM_REQUIRE(a->stem_ld >= a->channels && (a->stem_dtype == FIDM_F32 || a->stem_dtype == FIDM_BF16 || a->stem_dtype == FIDM_F16),
-                 FIDM_E_BADARG, "sampler_step: stem_out needs stem_ld >= channels and a dtype of F32 | BF16 | F16");
+  if (int rc = check_stem(a, "sampler_step")) return rc;
   StepParams p;
   p.a = *a;
-  const bool vec4 = (a->hw % 4 == 0) && (((uintptr_t)a->x | (uintptr_t)a->model_out | (uintptr_t)a->z |
-                                          (uintptr_t)a->gt | (uintptr_t)a->keep_mask | (uintptr_t)a->inject_noise |
-                                          (uintptr_t)a->sample | (uintptr_t)a->pred_xstart | (uintptr_t)a->x_next |
-                                          (uintptr_t)a->mean_out | (uintptr_t)a->logvar_out) % 16 == 0);
-  const long long total = (long long)a->batch * a->channels * (a->hw / (vec4 ? 4 : 1));
-  long long blocks = (total + 255) / 256;
-  const long long cap = (long long)num_sms() * 16;
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
-  if (vec4)
-    sampler_step_kernel<4><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(p);
-  else
-    sampler_step_kernel<1><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(p);
-  FIDM_CHECK_LAUNCH("sampler_step");
-  return 0;
+  const bool vec4 = vec4_ok(a->hw, a->x, a->model_out, a->z, a->gt, a->keep_mask, a->inject_noise, a->sample,
+                            a->pred_xstart, a->x_next, a->mean_out, a->logvar_out);
+  return launch_sampler(sampler_step_kernel<4>, sampler_step_kernel<1>, vec4,
+                        (long long)a->batch * a->channels * a->hw, p, stream, "sampler_step");
 }

@@ -39,6 +39,46 @@ def _extract_into_tensor(arr, timesteps, broadcast_shape):
     return vals.expand(broadcast_shape)
 
 
+def _f32(t):
+    """`t` detached, as the fp32 contiguous tensor the sampler kernels read (`t` itself when it already is one)."""
+    if t is None:
+        return None
+    t = t.detach()
+    if t.dtype != torch.float32 or not t.is_contiguous():
+        t = t.to(torch.float32).contiguous()
+    return t
+
+
+def _set_injection(a, x, gt, keep, inject_noise):
+    """Point the known-region fields of a sampler arg struct (StepArgs, MultistepArgs, ResampleArgs) at fp32 copies of
+    gt, keep and inject_noise.  Returns the copies: the caller holds them until the launch."""
+    gt, keep, inject_noise = _f32(gt), _f32(keep), _f32(inject_noise)
+    assert gt.shape == x.shape and inject_noise.shape == x.shape
+    assert keep.shape[0] == x.shape[0] and keep.shape[2:] == x.shape[2:], tuple(keep.shape)
+    a.gt, a.keep_mask, a.inject_noise = L.ptr(gt), L.ptr(keep), L.ptr(inject_noise)
+    a.mask_channels = keep.shape[1]
+    return gt, keep, inject_noise
+
+
+def _set_stem(a, stem, t_next):
+    """Step-boundary fusion fields of a sampler arg struct: stem = (NHWC network input, timestep tensor) of an engine
+    plan receives the new state and, when t_next is given, the next timestep."""
+    if stem is not None:
+        x_in, t_in = stem
+        a.stem_out, a.stem_dtype, a.stem_ld = L.ptr(x_in), L.dtype_code(x_in.dtype), x_in.shape[-1]
+        if t_next is not None:
+            a.t_out, a.t_out_value = L.ptr(t_in), float(t_next)
+
+
+def _known_region(model_kwargs, use_inpainting_injection):
+    """(gt, gt_keep_mask) from model_kwargs when the injection is on and both are given, else (None, None)."""
+    if use_inpainting_injection and model_kwargs:
+        gt, keep = model_kwargs.get("gt"), model_kwargs.get("gt_keep_mask")
+        if gt is not None and keep is not None:
+            return gt, keep
+    return None, None
+
+
 _MEAN_CODE = {ModelMeanType.PREVIOUS_X: L.MEAN_PREVIOUS_X, ModelMeanType.START_X: L.MEAN_START_X,
               ModelMeanType.EPSILON: L.MEAN_EPSILON}
 _VAR_CODE = {ModelVarType.LEARNED: L.VAR_LEARNED, ModelVarType.LEARNED_RANGE: L.VAR_LEARNED_RANGE,
@@ -141,18 +181,7 @@ class GaussianDiffusion:
         a.t_update = -1 if t is None else int(t)
         a.t_inject = -1 if t_inject is None else int(t_inject)
         coef = script_table if script_table is not None else self._coef(x.device, eta if ddim else 0.0)
-        keepalive = [coef]
-
-        def c(tn, name, shape=None):
-            if tn is None:
-                return None
-            tn = tn.detach()
-            if tn.dtype != torch.float32 or not tn.is_contiguous():
-                tn = tn.to(torch.float32).contiguous()
-            keepalive.append(tn)
-            return tn
-
-        x = c(x, "x")
+        x = _f32(x)
         a.coef, a.x = L.ptr(coef), L.ptr(x)
         if t_dev is not None:
             t_dev = t_dev.detach().to(device=x.device, dtype=torch.int64).contiguous()
@@ -162,26 +191,20 @@ class GaussianDiffusion:
             lo, hi = (int(v) for v in torch.stack(torch.aminmax(t_dev)).tolist())
             if lo < (1 if mode == L.STEP_UPDATE_INJECT else 0) or hi >= a.num_timesteps:
                 raise IndexError(f"timesteps [{lo}, {hi}] out of range for a {a.num_timesteps}-step table")
-            keepalive.append(t_dev)
             a.t_dev = L.ptr(t_dev)
         if mode != L.STEP_INJECT_ONLY:
-            model_out = c(model_out, "model_out")
+            model_out, z = _f32(model_out), _f32(z)
             want_ch = Cn if a.var_type == L.VAR_FIXED else 2 * Cn
             if script_table is not None and model_out.shape[1] == Cn:
                 a.var_type = L.VAR_FIXED          # scripts accept 3- or 6-channel outputs (:515-520)
                 want_ch = Cn
             assert model_out.shape == (B, want_ch) + tuple(x.shape[2:]), \
                 f"model output shape {tuple(model_out.shape)} != {(B, want_ch) + tuple(x.shape[2:])}"
-            a.model_out = L.ptr(model_out)
-            a.z = L.ptr(c(z, "z"))
+            a.model_out, a.z = L.ptr(model_out), L.ptr(z)
+        a.mask_channels = 1
         if mode != L.STEP_UPDATE_ONLY:
-            gt, keep, inject_noise = c(gt, "gt"), c(keep, "keep"), c(inject_noise, "noise")
-            assert gt.shape == x.shape and inject_noise.shape == x.shape
-            assert keep.shape[0] == B and keep.shape[1] in (1, Cn) and keep.shape[2:] == x.shape[2:]
-            a.gt, a.keep_mask, a.inject_noise = L.ptr(gt), L.ptr(keep), L.ptr(inject_noise)
-            a.mask_channels = keep.shape[1]
-        else:
-            a.mask_channels = 1
+            gt, keep, inject_noise = _set_injection(a, x, gt, keep, inject_noise)
+            assert keep.shape[1] in (1, Cn), tuple(keep.shape)
         out = {}
         for flag, key, field in ((want_sample, "sample", "sample"), (want_x0, "pred_xstart", "pred_xstart"),
                                  (want_next, "x_next", "x_next"), (want_mean, "mean", "mean_out"),
@@ -189,12 +212,7 @@ class GaussianDiffusion:
             if flag:
                 out[key] = next_buf if (key == "x_next" and next_buf is not None) else torch.empty_like(x)
                 setattr(a, field, L.ptr(out[key]))
-        if stem is not None:
-            x_in, t_in = stem
-            a.stem_out, a.stem_dtype, a.stem_ld = L.ptr(x_in), L.dtype_code(x_in.dtype), x_in.shape[-1]
-            if t_next is not None:
-                a.t_out, a.t_out_value = L.ptr(t_in), float(t_next)
-            keepalive += [x_in, t_in]
+        _set_stem(a, stem, t_next)
         L.check(L.lib().fidm_sampler_step(C.byref(a), L.stream()), "sampler_step")
         return out
 
@@ -359,12 +377,11 @@ class GaussianDiffusion:
 
     # ------------------------------------------------------------------ single reverse steps
     def _maybe_inject(self, x, t, model_kwargs, on, schedule, cumulative):
-        if on and model_kwargs:
-            gt, keep = model_kwargs.get("gt"), model_kwargs.get("gt_keep_mask")
-            if gt is not None and keep is not None:
-                return self.apply_inpainting_injection(x, t, gt, keep, use_cumulative_noise=cumulative,
-                                                       injection_schedule=schedule)
-        return x
+        gt, keep = _known_region(model_kwargs, on)
+        if gt is None:
+            return x
+        return self.apply_inpainting_injection(x, t, gt, keep, use_cumulative_noise=cumulative,
+                                               injection_schedule=schedule)
 
     def p_sample(self, model, x, t, clip_denoised=True, denoised_fn=None, cond_fn=None, model_kwargs=None,
                  use_inpainting_injection=False, injection_schedule="all", use_cumulative_noise=True):
@@ -410,25 +427,89 @@ class GaussianDiffusion:
         return {"sample": r["sample"], "pred_xstart": r["pred_xstart"]}
 
     # ------------------------------------------------------------------ loops
-    def _loop(self, ddim, model, shape, noise, clip_denoised, denoised_fn, cond_fn, model_kwargs, device,
-              progress, eta, use_inpainting_injection, injection_schedule, use_cumulative_noise,
-              progressive):
-        """Shared fused loop: per step one model call and ONE K4 launch ([update t] -> [inject t-1])."""
+    def _x_T(self, model, shape, noise, device):
+        """The device default and x_T of every loop: `noise`, or one randn(shape) draw; FidmError for a CPU x_T."""
         if device is None:
             device = next(model.parameters()).device
         assert isinstance(shape, (tuple, list))
         img = noise if noise is not None else torch.randn(*shape, device=device)
         L.require_cuda(img)
+        return device, img
+
+    def _loop_start(self, model, shape, noise, device, mk, gt, keep, t_first, injection_schedule, cumulative):
+        """Prologue of the fused loops (K4, K6, K7).  gt / keep: the known region, None without injection; the
+        injection noise is drawn like `gt` as given.  Returns (x, inj_noise, evaluate, stem, bufs):
+        x, the fp32 contiguous state the first evaluation (at t_first) sees, after the injection on x_T;
+        inj_noise(ts), the injection noise at ts; evaluate(x, t), the model output at t;
+        stem, the engine plan's (network input, timestep tensor) or None; bufs, two state buffers to alternate
+        between on the plan, or None (x is bufs[0] after an injection on the plan)."""
+        device, img = self._x_T(model, shape, noise, device)
+
+        def inj_noise(ts):
+            return self._cached_noise(gt, ts) if cumulative else torch.randn_like(gt)
+
+        # Step-boundary fusion: when `model` is this package's model_fn (train_inpainting.InpaintingModelFn around a
+        # DiffusionInpaintingModel), the step kernels write the next evaluation's stem channels and timestep themselves
+        # and the UNet output is read where the head left it: a step is [graph replay, randn, kernel] -- no pack, no
+        # copies, no clone.
+        plan = None
+        fused_plan = getattr(model, "fused_plan", None)
+        if fused_plan is not None and os.environ.get("FIDM_FUSED_STEP", "1") != "0":
+            plan = fused_plan(tuple(shape), img, self._t_value(t_first), mk)
+
+        def evaluate(x, t):
+            if plan is not None:
+                return plan.run()                            # stem input and timestep are already in place
+            return self._call_model(model, x, torch.full((shape[0],), t, device=device, dtype=torch.long), mk)
+
+        # the kernels write the state in NCHW order: buffers allocated like a channels_last x_T would scramble it
+        img = _f32(img)
+        stem = (plan.x_in, plan.t_in) if plan is not None else None
+        bufs = [torch.empty_like(img), torch.empty_like(img)] if plan is not None else None
+        if gt is None or self._injection_gated(t_first, injection_schedule):
+            return img, inj_noise, evaluate, stem, bufs
+        x = self._step(L.STEP_INJECT_ONLY, img, t_inject=t_first, gt=gt, keep=keep, inject_noise=inj_noise(t_first),
+                       cumulative=cumulative, want_next=True, stem=stem, next_buf=bufs[0] if bufs else None)["x_next"]
+        return x, inj_noise, evaluate, stem, bufs
+
+    def _update_inject(self, x, i, model_output, z, gt, keep, inj_noise, stem, next_buf, *, ddim, eta, clip,
+                       cumulative, injection_schedule, want_out):
+        """One K4 launch of a fused loop: the update at i, the injection at i - 1 unless it is gated, and the next
+        evaluation's stem input.  `z` is drawn by the caller, before the injection noise.  Returns (K4's outputs, the
+        state the next evaluation sees)."""
+        nxt = i - 1
+        do_inj = gt is not None and nxt >= 0 and not self._injection_gated(nxt, injection_schedule)
+        fused = stem is not None
+        r = self._step(L.STEP_UPDATE_INJECT if do_inj else L.STEP_UPDATE_ONLY, x, t=i, t_inject=nxt,
+                       model_out=model_output, z=z if (not ddim or eta != 0.0) else None,
+                       gt=gt if do_inj else None, keep=keep if do_inj else None,
+                       inject_noise=inj_noise(nxt) if do_inj else None,
+                       ddim=ddim, eta=eta, clip=clip, cumulative=cumulative,
+                       want_sample=want_out or (not do_inj and not fused), want_x0=want_out,
+                       want_next=do_inj or fused,
+                       stem=stem if nxt >= 0 else None, t_next=self._t_value(nxt) if nxt >= 0 else None,
+                       next_buf=next_buf)
+        return r, (r["x_next"] if (do_inj or fused) else r["sample"])
+
+    def _last_sample(self, loop):
+        """Runs a loop generator to its end on a fresh injection-noise cache and returns its last "sample"."""
+        self.clear_gt_noise_cache()
+        final = None
+        for final in loop:
+            pass
+        return final["sample"]
+
+    def _loop(self, ddim, model, shape, noise, clip_denoised, denoised_fn, cond_fn, model_kwargs, device,
+              progress, eta, use_inpainting_injection, injection_schedule, use_cumulative_noise,
+              progressive):
+        """Shared fused loop: per step one model call and ONE K4 launch ([update t] -> [inject t-1])."""
         indices = list(range(self.num_timesteps))[::-1]
         if progress and tqdm is not None:
             indices = tqdm(indices)
         mk = model_kwargs
-        gt = keep = None
-        if use_inpainting_injection and mk:
-            gt, keep = mk.get("gt"), mk.get("gt_keep_mask")
-        inject = gt is not None and keep is not None
 
         if denoised_fn is not None or cond_fn is not None:       # unfused compatibility path
+            device, img = self._x_T(model, shape, noise, device)
             step = self.ddim_sample if ddim else self.p_sample
             extra = {"eta": eta} if ddim else {}
             for i in indices:
@@ -442,50 +523,19 @@ class GaussianDiffusion:
                     img = out["sample"]
             return
 
-        def inj_noise(ts):
-            return self._cached_noise(gt, ts) if use_cumulative_noise else torch.randn_like(gt)
-
-        t_value = self._t_value
-        B = shape[0]
-        T = self.num_timesteps
-        first = T - 1
-        # Step-boundary fusion: when `model` is this package's model_fn (train_inpainting.InpaintingModelFn around a
-        # DiffusionInpaintingModel), K4 writes the next evaluation's stem channels and timestep itself and reads the
-        # UNet output where the head left it: a step is [graph replay, randn, K4] -- no pack, no copies, no clone.
-        plan = None
-        fused_plan = getattr(model, "fused_plan", None)
-        if fused_plan is not None and os.environ.get("FIDM_FUSED_STEP", "1") != "0":
-            plan = fused_plan(tuple(shape), img, t_value(first), mk)
-        stem = (plan.x_in, plan.t_in) if plan is not None else None
-        bufs = [torch.empty_like(img), torch.empty_like(img)] if plan is not None else None
+        gt, keep = _known_region(mk, use_inpainting_injection)
+        x, inj_noise, evaluate, stem, bufs = self._loop_start(model, shape, noise, device, mk, gt, keep,
+                                                             self.num_timesteps - 1, injection_schedule,
+                                                             use_cumulative_noise)
         with torch.no_grad():
-            # injection for the first step happens on x_T itself
-            if inject and not self._injection_gated(first, injection_schedule):
-                x = self._step(L.STEP_INJECT_ONLY, img, t_inject=first, gt=gt, keep=keep,
-                               inject_noise=inj_noise(first), cumulative=use_cumulative_noise,
-                               want_next=True, stem=stem, next_buf=bufs[0] if bufs else None)["x_next"]
-            else:
-                x = img
             for k, i in enumerate(indices):
-                if plan is not None:
-                    model_output = plan.run()                        # stem input and timestep are already in place
-                else:
-                    t = torch.full((B,), i, device=device, dtype=torch.long)
-                    model_output = self._call_model(model, x, t, mk)
+                model_output = evaluate(x, i)
                 z = torch.randn_like(x)                              # RNG order: z_t, then n_{t-1}
-                nxt = i - 1
-                do_inj = inject and nxt >= 0 and not self._injection_gated(nxt, injection_schedule)
                 want_out = progressive or i == 0
-                r = self._step(L.STEP_UPDATE_INJECT if do_inj else L.STEP_UPDATE_ONLY, x, t=i, t_inject=nxt,
-                               model_out=model_output, z=z if (not ddim or eta != 0.0) else None,
-                               gt=gt if do_inj else None, keep=keep if do_inj else None,
-                               inject_noise=inj_noise(nxt) if do_inj else None,
-                               ddim=ddim, eta=eta, clip=clip_denoised, cumulative=use_cumulative_noise,
-                               want_sample=want_out or (not do_inj and plan is None), want_x0=want_out,
-                               want_next=do_inj or plan is not None,
-                               stem=stem if nxt >= 0 else None, t_next=t_value(nxt) if nxt >= 0 else None,
-                               next_buf=bufs[(k + 1) & 1] if bufs else None)
-                x = r["x_next"] if (do_inj or plan is not None) else r["sample"]
+                r, x = self._update_inject(x, i, model_output, z, gt, keep, inj_noise, stem,
+                                           bufs[(k + 1) & 1] if bufs else None, ddim=ddim, eta=eta, clip=clip_denoised,
+                                           cumulative=use_cumulative_noise, injection_schedule=injection_schedule,
+                                           want_out=want_out)
                 if want_out:
                     yield {"sample": r["sample"], "pred_xstart": r["pred_xstart"]}
 
@@ -511,25 +561,17 @@ class GaussianDiffusion:
                       model_kwargs=None, device=None, progress=False, use_inpainting_injection=False,
                       injection_schedule="all", use_cumulative_noise=True):
         """DDPM sampling with optional known-region injection (`:390-413`)."""
-        self.clear_gt_noise_cache()
-        final = None
-        for final in self._loop(False, model, shape, noise, clip_denoised, denoised_fn, cond_fn, model_kwargs,
-                                device, progress, 0.0, use_inpainting_injection, injection_schedule,
-                                use_cumulative_noise, False):
-            pass
-        return final["sample"]
+        return self._last_sample(self._loop(False, model, shape, noise, clip_denoised, denoised_fn, cond_fn,
+                                            model_kwargs, device, progress, 0.0, use_inpainting_injection,
+                                            injection_schedule, use_cumulative_noise, False))
 
     def ddim_sample_loop(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None, cond_fn=None,
                          model_kwargs=None, device=None, progress=False, eta=0.0,
                          use_inpainting_injection=False, injection_schedule="all", use_cumulative_noise=True):
         """DDIM sampling with optional known-region injection (`:487-506`)."""
-        self.clear_gt_noise_cache()
-        final = None
-        for final in self._loop(True, model, shape, noise, clip_denoised, denoised_fn, cond_fn, model_kwargs,
-                                device, progress, eta, use_inpainting_injection, injection_schedule,
-                                use_cumulative_noise, False):
-            pass
-        return final["sample"]
+        return self._last_sample(self._loop(True, model, shape, noise, clip_denoised, denoised_fn, cond_fn,
+                                            model_kwargs, device, progress, eta, use_inpainting_injection,
+                                            injection_schedule, use_cumulative_noise, False))
 
     # ------------------------------------------------------------------ DPM-Solver++ multistep (K6)
     def _dpm_table(self, device, steps, order, cumulative):
@@ -545,9 +587,7 @@ class GaussianDiffusion:
         of an engine plan receives the new state and `t_next` (step-boundary fusion, as in _step)."""
         L.require_cuda(x, model_out, m_prev, gt, keep, inject_noise)
         B, Cn = x.shape[0], x.shape[1]
-        model_out = model_out.detach()
-        if model_out.dtype != torch.float32 or not model_out.is_contiguous():
-            model_out = model_out.to(torch.float32).contiguous()
+        model_out = _f32(model_out)
         assert model_out.shape[0] == B and model_out.shape[2:] == x.shape[2:], tuple(model_out.shape)
         a = L.MultistepArgs()
         a.batch, a.channels, a.hw = B, Cn, x.numel() // (B * Cn)
@@ -558,17 +598,10 @@ class GaussianDiffusion:
         a.coef, a.x, a.model_out, a.m_prev, a.m_out, a.x_next = (L.ptr(v) for v in (tab, x, model_out, m_prev, m, nxt))
         a.mask_channels = 1
         if gt is not None:
-            a.inject, a.mask_channels = 1, keep.shape[1]
-            a.gt, a.keep_mask, a.inject_noise = L.ptr(gt), L.ptr(keep), L.ptr(inject_noise)
-        if stem is not None:
-            x_in, t_in = stem
-            a.stem_out, a.stem_dtype, a.stem_ld = L.ptr(x_in), L.dtype_code(x_in.dtype), x_in.shape[-1]
-            if t_next is not None:
-                a.t_out, a.t_out_value = L.ptr(t_in), float(t_next)
-        try:
-            L.check(L.lib().fidm_multistep_step(C.byref(a), L.stream()), "multistep_step")
-        except ValueError as e:      # an argument the library refuses: the caller passed something this path cannot run
-            raise L.FidmError(str(e)) from None
+            a.inject = 1
+            gt, keep, inject_noise = _set_injection(a, x, gt, keep, inject_noise)
+        _set_stem(a, stem, t_next)
+        L.check(L.lib().fidm_multistep_step(C.byref(a), L.stream()), "multistep_step")
         return m, nxt
 
     def _dpm_solver_loop(self, model, shape, steps, order, noise, clip_denoised, model_kwargs, device, progress,
@@ -578,52 +611,26 @@ class GaussianDiffusion:
             raise NotImplementedError("DPM-Solver++ needs an eps or x0 prediction; PREVIOUS_X models are not supported")
         grid = dpm_solver.timestep_grid(self.num_timesteps, steps)
         orders = dpm_solver.step_orders(steps, order)
-        if device is None:
-            device = next(model.parameters()).device
-        assert isinstance(shape, (tuple, list))
-        img = noise if noise is not None else torch.randn(*shape, device=device)
-        L.require_cuda(img)
-        tab = self._dpm_table(img.device, steps, order, use_cumulative_noise)
         mk = model_kwargs
-        gt = keep = None
-        if use_inpainting_injection and mk:
-            gt, keep = mk.get("gt"), mk.get("gt_keep_mask")
-        inject = gt is not None and keep is not None
-        if inject:
-            gt, keep = (v.detach().to(torch.float32).contiguous() for v in (gt, keep))
-
-        def inj_noise(ts):
-            return self._cached_noise(gt, ts) if use_cumulative_noise else torch.randn_like(gt)
-
-        B = shape[0]
-        plan = None
-        fused_plan = getattr(model, "fused_plan", None)
-        if fused_plan is not None and os.environ.get("FIDM_FUSED_STEP", "1") != "0":
-            plan = fused_plan(tuple(shape), img, self._t_value(int(grid[0])), mk)
-        stem = (plan.x_in, plan.t_in) if plan is not None else None
+        gt, keep = _known_region(mk, use_inpainting_injection)
+        if gt is not None:           # once per loop; the injection noise is drawn like the fp32 copy
+            gt, keep = _f32(gt), _f32(keep)
+        x, inj_noise, evaluate, stem, _ = self._loop_start(model, shape, noise, device, mk, gt, keep, int(grid[0]),
+                                                            injection_schedule, use_cumulative_noise)
+        tab = self._dpm_table(x.device, steps, order, use_cumulative_noise)
         ks = range(steps)
         if progress and tqdm is not None:
             ks = tqdm(ks)
         with torch.no_grad():
-            t0 = int(grid[0])
-            if inject and not self._injection_gated(t0, injection_schedule):      # injection on x_T itself
-                x = self._step(L.STEP_INJECT_ONLY, img, t_inject=t0, gt=gt, keep=keep, inject_noise=inj_noise(t0),
-                               cumulative=use_cumulative_noise, want_next=True, stem=stem)["x_next"]
-            else:
-                x = img.detach().to(torch.float32).contiguous()
             m_prev = None
             for k in ks:
-                if plan is not None:
-                    model_output = plan.run()                    # stem input and timestep are already in place
-                else:
-                    t = torch.full((B,), int(grid[k]), device=device, dtype=torch.long)
-                    model_output = self._call_model(model, x, t, mk)
+                model_output = evaluate(x, int(grid[k]))
                 if k == steps - 1:                               # t = 0: the sample is the x0 prediction
                     m, _ = self._multistep(tab, k, x, model_output, want_next=False, clip=clip_denoised)
                     yield {"sample": m, "pred_xstart": m}
                     break
                 nxt = int(grid[k + 1])
-                do_inj = inject and not self._injection_gated(nxt, injection_schedule)
+                do_inj = gt is not None and not self._injection_gated(nxt, injection_schedule)
                 m, x = self._multistep(tab, k, x, model_output, m_prev=m_prev if orders[k] == 2 else None,
                                        clip=clip_denoised, gt=gt if do_inj else None, keep=keep if do_inj else None,
                                        inject_noise=inj_noise(nxt) if do_inj else None, stem=stem,
@@ -648,13 +655,9 @@ class GaussianDiffusion:
         round(linspace(T - 1, 0, steps)) of this diffusion's own table, with the class path's known-region injection
         (on x_T, then after every update) and RNG draw order (randn(shape), then one injection noise per injection;
         the solver itself draws nothing).  Returns the x0 prediction at t = 0."""
-        self.clear_gt_noise_cache()
-        final = None
-        for final in self._dpm_solver_loop(model, shape, steps, order, noise, clip_denoised, model_kwargs, device,
-                                           progress, use_inpainting_injection, injection_schedule,
-                                           use_cumulative_noise):
-            pass
-        return final["sample"]
+        return self._last_sample(self._dpm_solver_loop(model, shape, steps, order, noise, clip_denoised, model_kwargs,
+                                                       device, progress, use_inpainting_injection, injection_schedule,
+                                                       use_cumulative_noise))
 
     # ------------------------------------------------------------------ RePaint resampling (K4 + K7)
     def _resample(self, x, u, undo_a, undo_s, *, t_inject=None, gt=None, keep=None, inject_noise=None, cumulative=True,
@@ -663,16 +666,7 @@ class GaussianDiffusion:
         table's coefficients; stem = (NHWC network input, timestep tensor) of an engine plan receives the new state and
         `t_next` (step-boundary fusion, as in _step).  Returns the new state (next_buf when given)."""
         L.require_cuda(x, u, gt, keep, inject_noise)
-        keepalive = []
-
-        def c(tn):
-            tn = tn.detach()
-            if tn.dtype != torch.float32 or not tn.is_contiguous():
-                tn = tn.to(torch.float32).contiguous()
-            keepalive.append(tn)
-            return tn
-
-        x, u = c(x), c(u)
+        x, u = _f32(x), _f32(u)
         assert u.shape == x.shape, (tuple(u.shape), tuple(x.shape))
         B, Cn = x.shape[0], x.shape[1]
         a = L.ResampleArgs()
@@ -682,25 +676,15 @@ class GaussianDiffusion:
         a.x, a.noise, a.x_next = L.ptr(x), L.ptr(u), L.ptr(out)
         a.mask_channels = 1
         if t_inject is not None:
-            gt, keep, inject_noise = c(gt), c(keep), c(inject_noise)
-            assert gt.shape == x.shape and inject_noise.shape == x.shape
-            assert keep.shape[0] == B and keep.shape[2:] == x.shape[2:], tuple(keep.shape)
+            gt, keep, inject_noise = _set_injection(a, x, gt, keep, inject_noise)
             if "host" not in self._coef_cache:
                 self._coef_cache["host"] = self.coefficient_table(0.0)
             cls = self._coef_cache["host"]
             ia, is_ = (L.C_SQRT_AB, L.C_SQRT_1MAB) if cumulative else (L.C_SQRT_AB_F32, L.C_SQRT_1MAB_F32)
-            a.inject, a.mask_channels = 1, keep.shape[1]
+            a.inject = 1
             a.inject_a, a.inject_s = float(cls[t_inject, ia]), float(cls[t_inject, is_])
-            a.gt, a.keep_mask, a.inject_noise = L.ptr(gt), L.ptr(keep), L.ptr(inject_noise)
-        if stem is not None:
-            x_in, t_in = stem
-            a.stem_out, a.stem_dtype, a.stem_ld = L.ptr(x_in), L.dtype_code(x_in.dtype), x_in.shape[-1]
-            if t_next is not None:
-                a.t_out, a.t_out_value = L.ptr(t_in), float(t_next)
-        try:
-            L.check(L.lib().fidm_resample_undo(C.byref(a), L.stream()), "resample_undo")
-        except ValueError as e:      # an argument the library refuses: the caller passed something this path cannot run
-            raise L.FidmError(str(e)) from None
+        _set_stem(a, stem, t_next)
+        L.check(L.lib().fidm_resample_undo(C.byref(a), L.stream()), "resample_undo")
         return out
 
     def _repaint_plan(self, jump_length, jump_n_sample, model_kwargs, use_inpainting_injection):
@@ -716,57 +700,22 @@ class GaussianDiffusion:
                       injection_schedule, use_cumulative_noise, progressive):
         """Per evaluation one model call and one K4 launch; when a jump follows the evaluation, K4 only updates and
         one K7 launch re-noises to t_up, injects at t_up and writes the next stem input."""
-        if device is None:
-            device = next(model.parameters()).device
-        assert isinstance(shape, (tuple, list))
-        img = noise if noise is not None else torch.randn(*shape, device=device)
-        L.require_cuda(img)
         mk = model_kwargs
         gt, keep = mk["gt"], mk["gt_keep_mask"]
-
-        def inj_noise(ts):
-            return self._cached_noise(gt, ts) if use_cumulative_noise else torch.randn_like(gt)
-
-        t_value = self._t_value
-        B = shape[0]
-        first = evals[0].t
-        plan = None
-        fused_plan = getattr(model, "fused_plan", None)
-        if fused_plan is not None and os.environ.get("FIDM_FUSED_STEP", "1") != "0":
-            plan = fused_plan(tuple(shape), img, t_value(first), mk)
-        stem = (plan.x_in, plan.t_in) if plan is not None else None
-        bufs = [torch.empty_like(img), torch.empty_like(img)] if plan is not None else None
+        x, inj_noise, evaluate, stem, bufs = self._loop_start(model, shape, noise, device, mk, gt, keep, evals[0].t,
+                                                             injection_schedule, use_cumulative_noise)
         if progress and tqdm is not None:
             evals = tqdm(evals)
         with torch.no_grad():
-            # injection for the first evaluation happens on x_T itself
-            if not self._injection_gated(first, injection_schedule):
-                x = self._step(L.STEP_INJECT_ONLY, img, t_inject=first, gt=gt, keep=keep,
-                               inject_noise=inj_noise(first), cumulative=use_cumulative_noise,
-                               want_next=True, stem=stem, next_buf=bufs[0] if bufs else None)["x_next"]
-            else:
-                x = img
             for k, (i, t_up, undo_a, undo_s) in enumerate(evals):
-                if plan is not None:
-                    model_output = plan.run()                        # stem input and timestep are already in place
-                else:
-                    t = torch.full((B,), i, device=device, dtype=torch.long)
-                    model_output = self._call_model(model, x, t, mk)
+                model_output = evaluate(x, i)
                 z = torch.randn_like(x)                              # RNG order: z_t, [u], then n of the next t
                 want_out = progressive or i == 0
                 nbuf = bufs[(k + 1) & 1] if bufs else None
                 if t_up is None:                                     # as _loop's DDPM step
-                    nxt = i - 1
-                    do_inj = nxt >= 0 and not self._injection_gated(nxt, injection_schedule)
-                    r = self._step(L.STEP_UPDATE_INJECT if do_inj else L.STEP_UPDATE_ONLY, x, t=i, t_inject=nxt,
-                                   model_out=model_output, z=z, gt=gt if do_inj else None,
-                                   keep=keep if do_inj else None, inject_noise=inj_noise(nxt) if do_inj else None,
-                                   ddim=False, clip=clip_denoised, cumulative=use_cumulative_noise,
-                                   want_sample=want_out or (not do_inj and plan is None), want_x0=want_out,
-                                   want_next=do_inj or plan is not None,
-                                   stem=stem if nxt >= 0 else None, t_next=t_value(nxt) if nxt >= 0 else None,
-                                   next_buf=nbuf)
-                    x = r["x_next"] if (do_inj or plan is not None) else r["sample"]
+                    r, x = self._update_inject(x, i, model_output, z, gt, keep, inj_noise, stem, nbuf, ddim=False,
+                                               eta=0.0, clip=clip_denoised, cumulative=use_cumulative_noise,
+                                               injection_schedule=injection_schedule, want_out=want_out)
                 else:
                     r = self._step(L.STEP_UPDATE_ONLY, x, t=i, model_out=model_output, z=z, ddim=False,
                                    clip=clip_denoised, want_sample=True, want_x0=want_out)
@@ -774,7 +723,7 @@ class GaussianDiffusion:
                     do_inj = not self._injection_gated(t_up, injection_schedule)
                     x = self._resample(r["sample"], u, undo_a, undo_s, t_inject=t_up if do_inj else None,
                                        gt=gt, keep=keep, inject_noise=inj_noise(t_up) if do_inj else None,
-                                       cumulative=use_cumulative_noise, stem=stem, t_next=t_value(t_up),
+                                       cumulative=use_cumulative_noise, stem=stem, t_next=self._t_value(t_up),
                                        next_buf=nbuf)
                 if want_out:
                     yield {"sample": r["sample"], "pred_xstart": r["pred_xstart"], "t": i}
@@ -801,12 +750,8 @@ class GaussianDiffusion:
         the undo noise if a jump follows, and the injection noise of the next evaluation (with use_cumulative_noise
         a revisited timestep reuses its cached noise).  Returns the sample at t = 0, not re-blended."""
         evals = self._repaint_plan(jump_length, jump_n_sample, model_kwargs, use_inpainting_injection)
-        self.clear_gt_noise_cache()
-        final = None
-        for final in self._repaint_loop(evals, model, shape, noise, clip_denoised, model_kwargs, device, progress,
-                                        injection_schedule, use_cumulative_noise, False):
-            pass
-        return final["sample"]
+        return self._last_sample(self._repaint_loop(evals, model, shape, noise, clip_denoised, model_kwargs, device,
+                                                    progress, injection_schedule, use_cumulative_noise, False))
 
     def sample_with_advanced_inpainting(self, model, shape, gt=None, gt_keep_mask=None, use_ddim=True, eta=0.0,
                                         progress=True, device=None, injection_schedule="all",

@@ -1,8 +1,6 @@
 """CPU: DPM-Solver++ multistep host logic -- the grid, the per-step coefficient table against the float64 D-form of
-oracle/dpm_solver_oracle.py, the C struct mirror, and the solver's convergence order on the analytic model."""
+oracle/dpm_solver_oracle.py, and the solver's convergence order on the analytic model."""
 import math
-import os
-import re
 
 import numpy as np
 import pytest
@@ -11,8 +9,6 @@ import torch
 import fidm_b200 as F
 from fidm_b200 import _lib, dpm_solver
 from oracle import dpm_solver_oracle as O
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.mark.parametrize("T,N", [(1000, 2), (1000, 20), (1000, 25), (1000, 999), (1000, 1000), (100, 100), (7, 3)])
@@ -85,25 +81,6 @@ def test_table_reuses_the_class_path_fp32_values(cumulative):
     assert torch.equal(tab[:-1, _lib.MS_INJ_A], cls[g[1:], ia]) and torch.equal(tab[:-1, _lib.MS_INJ_S], cls[g[1:], is_])
     rows = dpm_solver.update_rows(d.alphas_cumprod, g.numpy(), 2)
     assert torch.equal(tab[:, _lib.MS_A:_lib.MS_B1 + 1], torch.from_numpy(rows).float())
-
-
-def test_multistep_struct_matches_header_field_order():
-    text = open(os.path.join(ROOT, "include", "fidm_b200.h")).read()
-    body = re.search(r"typedef struct fidm_multistep_args \{(.*?)\} fidm_multistep_args;", text, flags=re.S).group(1)
-    body = re.sub(r"/\*.*?\*/", "", body, flags=re.S)
-    names = []
-    for decl in body.split(";"):
-        decl = decl.strip()
-        if not decl:
-            continue
-        decl = re.sub(r"^(const\s+)?(int32_t|int64_t|float|double|void)\s*\**", "", decl)
-        for part in decl.split(","):
-            names.append(re.sub(r"\[.*\]", "", part.replace("*", "").strip()))
-    assert names == [f[0] for f in _lib.MultistepArgs._fields_]
-    cols = int(re.search(r"#define FIDM_MS_COLS (\d+)", text).group(1))
-    assert cols == _lib.MS_COLS
-    for name in ("X0_C1", "X0_C2", "A", "B0", "B1", "INJ_A", "INJ_S"):
-        assert int(re.search(r"FIDM_MS_%s = (\d+)" % name, text).group(1)) == getattr(_lib, "MS_" + name)
 
 
 def _rms_errors(sched, order, Ns):

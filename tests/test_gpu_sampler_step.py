@@ -100,6 +100,40 @@ def test_step_argument_errors(cuda_lib):
         d._step(L.STEP_UPDATE_ONLY, x, t=3, model_out=torch.zeros(1, 3, 8, 8, device="cuda"), want_sample=True)
 
 
+@pytest.mark.parametrize("schedule", ["all", "low"])
+@pytest.mark.parametrize("loop", ["ddim", "ddpm", "repaint", "dpm_solver"])
+def test_fused_loops_equal_for_channels_last_noise(cuda_lib, loop, schedule, monkeypatch):
+    """T64 (synthetic weights) on the engine plan: a channels_last x_T gives every loop bit for bit what the same x_T
+    in NCHW order gives.  The kernels write NCHW state, so the loops must not allocate their state like x_T."""
+    import fidm_b200 as F
+    from fidm_b200.utils.synth import synth_batch, synth_state_dict
+    monkeypatch.setenv("FIDM_FUSED_STEP", "1")
+    dev = torch.device("cuda:0")
+    cfg = F.CONFIGS["T64"]
+    model = F.DiffusionInpaintingModel(F.UNetModel(**dict(cfg, in_channels=3)))
+    model.load_state_dict(synth_state_dict(cfg, seed=2), strict=True)
+    fn = F.InpaintingModelFn(model.to(dev))
+    plans = []
+    inner = fn.fused_plan
+    fn.fused_plan = lambda *a: plans.append(inner(*a)) or plans[-1]
+    d = F.create_gaussian_diffusion(steps=20, learn_sigma=True, noise_schedule="cosine")
+    data = synth_batch(2, 64, seed=6, device=dev)
+    shape = (2, 3, 64, 64)
+    noise = torch.randn(shape, device=dev, generator=torch.Generator(device=dev).manual_seed(1))
+    kw = dict(model_kwargs={"gt": data["gt"], "gt_keep_mask": data["gt_keep_mask"]}, device=dev,
+              use_inpainting_injection=True, injection_schedule=schedule)
+    run = {"ddim": lambda x_T: d.ddim_sample_loop(fn, shape, noise=x_T, **kw),
+           "ddpm": lambda x_T: d.p_sample_loop(fn, shape, noise=x_T, **kw),
+           "repaint": lambda x_T: d.repaint_sample_loop(fn, shape, jump_length=4, jump_n_sample=2, noise=x_T, **kw),
+           "dpm_solver": lambda x_T: d.dpm_solver_sample_loop(fn, shape, steps=8, noise=x_T, **kw)}[loop]
+    outs = []
+    for x_T in (noise, noise.contiguous(memory_format=torch.channels_last)):
+        torch.manual_seed(4)
+        outs.append(run(x_T))
+    assert len(plans) == 2 and all(p is not None for p in plans)      # both runs were fused
+    assert torch.isfinite(outs[0]).all() and torch.equal(outs[1], outs[0]), (loop, schedule)
+
+
 def test_pack_unpack_roundtrip(cuda_lib):
     from fidm_b200 import ops
     dev = "cuda"

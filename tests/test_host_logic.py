@@ -34,7 +34,8 @@ def test_library_exports_every_declared_symbol():
 
 def test_ctypes_structs_match_header_field_order():
     text = open(os.path.join(ROOT, "include", "fidm_b200.h")).read()
-    for cname, struct in (("fidm_step_args", _lib.StepArgs), ("fidm_gn_args", _lib.GnArgs),
+    for cname, struct in (("fidm_step_args", _lib.StepArgs), ("fidm_multistep_args", _lib.MultistepArgs),
+                          ("fidm_resample_args", _lib.ResampleArgs), ("fidm_gn_args", _lib.GnArgs),
                           ("fidm_conv_args", _lib.ConvArgs), ("fidm_attn_args", _lib.AttnArgs),
                           ("fidm_pack_args", _lib.PackArgs)):
         body = re.search(r"typedef struct %s \{(.*?)\} %s;" % (cname, cname), text, flags=re.S).group(1)
@@ -48,6 +49,11 @@ def test_ctypes_structs_match_header_field_order():
             for part in decl.split(","):
                 names.append(re.sub(r"\[.*\]", "", part.replace("*", "").strip()))
         assert names == [f[0] for f in struct._fields_], cname
+    cols = int(re.search(r"#define FIDM_MS_COLS (\d+)", text).group(1))
+    assert cols == _lib.MS_COLS
+    for name in ("X0_C1", "X0_C2", "A", "B0", "B1", "INJ_A", "INJ_S"):
+        assert int(re.search(r"FIDM_MS_%s = (\d+)" % name, text).group(1)) == getattr(_lib, "MS_" + name)
+    assert "fidm_resample_undo" in _lib.SYMBOLS
 
 
 def test_no_cpu_fallback():
