@@ -22,6 +22,7 @@ SAMPLER_DDPM, SAMPLER_DDIM, SAMPLER_DDIM_SCRIPT = 0, 1, 2
 MEAN_PREVIOUS_X, MEAN_START_X, MEAN_EPSILON = 0, 1, 2
 VAR_LEARNED, VAR_FIXED, VAR_LEARNED_RANGE = 0, 1, 2
 RESAMPLE_NONE, RESAMPLE_DOWN, RESAMPLE_UP = 0, 1, 2
+NOISE_XT, NOISE_STEP, NOISE_INJECT, NOISE_INJECT_FRESH, NOISE_UNDO = range(5)
 
 i32, vp, fp, dp = C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p
 
@@ -51,6 +52,10 @@ class ResampleArgs(C.Structure):
                 ("inject", i32), ("inject_a", C.c_float), ("inject_s", C.c_float),
                 ("gt", fp), ("keep_mask", fp), ("inject_noise", fp),
                 ("stem_out", vp), ("stem_dtype", i32), ("stem_ld", i32), ("t_out", fp), ("t_out_value", C.c_float)]
+
+
+class SeededNoise(C.Structure):
+    _fields_ = [("seeds", vp), ("draw", i32), ("inject_tag", i32), ("inject_draw", i32)]
 
 
 class PackArgs(C.Structure):
@@ -95,6 +100,10 @@ SYMBOLS = {
     "fidm_sampler_step": (C.c_int, [_P(StepArgs), vp]),
     "fidm_multistep_step": (C.c_int, [_P(MultistepArgs), vp]),
     "fidm_resample_undo": (C.c_int, [_P(ResampleArgs), vp]),
+    "fidm_sampler_step_seeded": (C.c_int, [_P(StepArgs), _P(SeededNoise), vp]),
+    "fidm_multistep_step_seeded": (C.c_int, [_P(MultistepArgs), _P(SeededNoise), vp]),
+    "fidm_resample_undo_seeded": (C.c_int, [_P(ResampleArgs), _P(SeededNoise), vp]),
+    "fidm_randn_seeded": (C.c_int, [fp, vp, i32, C.c_int64, i32, i32, vp]),
     "fidm_pack_nchw_to_nhwc": (C.c_int, [_P(PackArgs), vp]),
     "fidm_unpack_nhwc_to_nchw": (C.c_int, [vp, i32, i32, fp, i32, i32, i32, vp]),
     "fidm_prepare_inputs_u8": (C.c_int, [vp, vp, fp, fp, fp, fp, i32, i32, vp]),

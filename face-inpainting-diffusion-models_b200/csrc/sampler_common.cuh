@@ -2,6 +2,7 @@
 // The fused-versus-unfused tests and the oracles compare these kernels bit for bit, so each piece exists once.
 #pragma once
 #include "common.cuh"
+#include "philox.cuh"
 
 namespace fidm {
 
@@ -24,6 +25,14 @@ __device__ __forceinline__ SamplerElem sampler_elem(long long idx, int channels,
   const int mc = (mask_channels == 1) ? 0 : e.c;
   e.moff = ((long long)e.b * mask_channels + mc) * hw + (long long)e.pv * VEC;
   return e;
+}
+
+// Seeded mode: the VEC normals of element e under its image's seed, draw (tag, draw) -- what fidm_randn_seeded writes
+// at the same place of a [batch][channels][hw] buffer.
+template <int VEC>
+__device__ __forceinline__ void seeded_elem_normals(const fidm_seeded_noise& s, const SamplerElem& e, int hw, int tag,
+                                                    int draw, float (&n)[VEC]) {
+  seeded_normals<VEC>(s.seeds[e.b], (long long)e.c * hw + (long long)e.pv * VEC, (uint32_t)tag, (uint32_t)draw, n);
 }
 
 // Known-region injection (apply_inpainting_injection): m*wg + (1-m)*v, wg = ca*gt + cs*n, one fp32 rounding per
@@ -68,6 +77,15 @@ template <typename Args>
 inline int check_mask_channels(const Args* a, const char* who) {
   FIDM_REQUIRE(a->mask_channels == 1 || a->mask_channels == a->channels, FIDM_E_BADARG,
                "%s: mask_channels must be 1 or channels", who);
+  return 0;
+}
+
+// The seeded entries: `s` and its seeds are required, and the injection draw must be a valid one when `inject`.
+inline int check_seeded(const fidm_seeded_noise* s, bool inject, const char* who) {
+  FIDM_REQUIRE(s != nullptr && s->seeds != nullptr, FIDM_E_BADARG, "%s: seeded noise and its seeds are required", who);
+  if (inject)
+    FIDM_REQUIRE((s->inject_tag == FIDM_NOISE_INJECT || s->inject_tag == FIDM_NOISE_INJECT_FRESH) && s->inject_draw >= 0,
+                 FIDM_E_BADARG, "%s: the injection needs tag INJECT | INJECT_FRESH and a draw >= 0", who);
   return 0;
 }
 

@@ -6,18 +6,26 @@
 //
 // Rounding contract (as sampler_step.cu): every product and sum is an explicit __fmul_rn / __fadd_rn / __fsub_rn, so
 // the compiler may not contract them into FMAs and oracle/dpm_solver_oracle.py can mirror the kernel bit for bit.
+//
+// SEEDED (fidm_multistep_step_seeded): the injection noise is generated in registers (philox.cuh) instead of read.
 #include "sampler_common.cuh"
 
 namespace fidm {
 
+template <bool SEEDED>
 struct MultistepParams {
   fidm_multistep_args a;
+};
+template <>
+struct MultistepParams<true> {
+  fidm_multistep_args a;
+  fidm_seeded_noise s;
 };
 
 __device__ __forceinline__ float ms_clamp1(float v) { return fminf(fmaxf(v, -1.0f), 1.0f); }
 
-template <int VEC>
-__global__ void __launch_bounds__(256) multistep_step_kernel(const MultistepParams p) {
+template <int VEC, bool SEEDED>
+__global__ void __launch_bounds__(256) multistep_step_kernel(const MultistepParams<SEEDED> p) {
   const fidm_multistep_args& a = p.a;
   const float* cf = a.coef + (long long)a.step * FIDM_MS_COLS;
   const float c1 = cf[FIDM_MS_X0_C1], c2 = cf[FIDM_MS_X0_C2];
@@ -41,7 +49,10 @@ __global__ void __launch_bounds__(256) multistep_step_kernel(const MultistepPara
     if (upd && second) load_vec<float, VEC>(a.m_prev + off, mp);
     if (inj) {
       load_vec<float, VEC>(a.gt + off, g);
-      load_vec<float, VEC>(a.inject_noise + off, n);
+      if constexpr (SEEDED)
+        seeded_elem_normals<VEC>(p.s, e, a.hw, p.s.inject_tag, p.s.inject_draw, n);
+      else
+        load_vec<float, VEC>(a.inject_noise + off, n);
       load_vec<float, VEC>(a.keep_mask + e.moff, m);
     }
 
@@ -66,33 +77,50 @@ __global__ void __launch_bounds__(256) multistep_step_kernel(const MultistepPara
   }
 }
 
+// The unseeded (s == nullptr) and seeded entries; `who` prefixes the error text.
+static int multistep_step(const fidm_multistep_args* a, const fidm_seeded_noise* s, fidm_stream_t stream,
+                          const char* who) {
+  FIDM_REQUIRE(a != nullptr, FIDM_E_BADARG, "%s: null args", who);
+  FIDM_REQUIRE(a->batch > 0 && a->channels > 0 && a->hw > 0, FIDM_E_BADARG, "%s: empty shape", who);
+  FIDM_REQUIRE(a->mean_type == FIDM_MEAN_EPSILON || a->mean_type == FIDM_MEAN_START_X, FIDM_E_BADARG,
+               "%s: mean_type must be EPSILON or START_X", who);
+  FIDM_REQUIRE(a->out_channels == a->channels || a->out_channels == 2 * a->channels, FIDM_E_BADARG,
+               "%s: out_channels must be channels or 2*channels", who);
+  FIDM_REQUIRE(a->coef && a->x && a->model_out && a->m_out, FIDM_E_BADARG,
+               "%s: coef/x/model_out/m_out are required", who);
+  FIDM_REQUIRE(a->steps > 0 && a->step >= 0 && a->step < a->steps, FIDM_E_BADARG,
+               "%s: step %d out of range [0,%d)", who, a->step, a->steps);
+  FIDM_REQUIRE(a->m_prev == nullptr || a->step > 0, FIDM_E_BADARG, "%s: step 0 has no m_prev", who);
+  if (s) {
+    if (int rc = check_seeded(s, a->inject != 0, who)) return rc;
+    FIDM_REQUIRE(a->inject_noise == nullptr, FIDM_E_BADARG, "%s: inject_noise must be NULL", who);
+  }
+  if (a->inject) {
+    FIDM_REQUIRE(a->x_next != nullptr, FIDM_E_BADARG, "%s: an injection needs x_next", who);
+    FIDM_REQUIRE(a->gt && a->keep_mask && (s || a->inject_noise), FIDM_E_BADARG,
+                 "%s: gt/keep_mask/inject_noise required for an injection", who);
+    if (int rc = check_mask_channels(a, who)) return rc;
+  }
+  FIDM_REQUIRE(a->stem_out == nullptr || a->x_next != nullptr, FIDM_E_BADARG, "%s: stem_out needs x_next", who);
+  if (int rc = check_stem(a, who)) return rc;
+  const bool vec4 = vec4_ok(a->hw, a->x, a->model_out, a->m_prev, a->m_out, a->x_next, a->gt, a->keep_mask,
+                            a->inject_noise);
+  const long long elems = (long long)a->batch * a->channels * a->hw;
+  if (s)
+    return launch_sampler(multistep_step_kernel<4, true>, multistep_step_kernel<1, true>, vec4, elems,
+                          MultistepParams<true>{*a, *s}, stream, who);
+  return launch_sampler(multistep_step_kernel<4, false>, multistep_step_kernel<1, false>, vec4, elems,
+                        MultistepParams<false>{*a}, stream, who);
+}
+
 }  // namespace fidm
 
 extern "C" int fidm_multistep_step(const fidm_multistep_args* a, fidm_stream_t stream) {
-  using namespace fidm;
-  FIDM_REQUIRE(a != nullptr, FIDM_E_BADARG, "multistep_step: null args");
-  FIDM_REQUIRE(a->batch > 0 && a->channels > 0 && a->hw > 0, FIDM_E_BADARG, "multistep_step: empty shape");
-  FIDM_REQUIRE(a->mean_type == FIDM_MEAN_EPSILON || a->mean_type == FIDM_MEAN_START_X, FIDM_E_BADARG,
-               "multistep_step: mean_type must be EPSILON or START_X");
-  FIDM_REQUIRE(a->out_channels == a->channels || a->out_channels == 2 * a->channels, FIDM_E_BADARG,
-               "multistep_step: out_channels must be channels or 2*channels");
-  FIDM_REQUIRE(a->coef && a->x && a->model_out && a->m_out, FIDM_E_BADARG,
-               "multistep_step: coef/x/model_out/m_out are required");
-  FIDM_REQUIRE(a->steps > 0 && a->step >= 0 && a->step < a->steps, FIDM_E_BADARG,
-               "multistep_step: step %d out of range [0,%d)", a->step, a->steps);
-  FIDM_REQUIRE(a->m_prev == nullptr || a->step > 0, FIDM_E_BADARG, "multistep_step: step 0 has no m_prev");
-  if (a->inject) {
-    FIDM_REQUIRE(a->x_next != nullptr, FIDM_E_BADARG, "multistep_step: an injection needs x_next");
-    FIDM_REQUIRE(a->gt && a->keep_mask && a->inject_noise, FIDM_E_BADARG,
-                 "multistep_step: gt/keep_mask/inject_noise required for an injection");
-    if (int rc = check_mask_channels(a, "multistep_step")) return rc;
-  }
-  FIDM_REQUIRE(a->stem_out == nullptr || a->x_next != nullptr, FIDM_E_BADARG, "multistep_step: stem_out needs x_next");
-  if (int rc = check_stem(a, "multistep_step")) return rc;
-  MultistepParams p;
-  p.a = *a;
-  const bool vec4 = vec4_ok(a->hw, a->x, a->model_out, a->m_prev, a->m_out, a->x_next, a->gt, a->keep_mask,
-                            a->inject_noise);
-  return launch_sampler(multistep_step_kernel<4>, multistep_step_kernel<1>, vec4,
-                        (long long)a->batch * a->channels * a->hw, p, stream, "multistep_step");
+  return fidm::multistep_step(a, nullptr, stream, "multistep_step");
+}
+
+extern "C" int fidm_multistep_step_seeded(const fidm_multistep_args* a, const fidm_seeded_noise* s,
+                                          fidm_stream_t stream) {
+  FIDM_REQUIRE(s != nullptr, FIDM_E_BADARG, "multistep_step_seeded: seeded noise is required");
+  return fidm::multistep_step(a, s, stream, "multistep_step_seeded");
 }

@@ -9,18 +9,27 @@
 // sum below is an explicit __fmul_rn/__fadd_rn/__fsub_rn/__fdiv_rn -- the compiler may not contract
 // them into FMAs.  With identical model output and noise the DDIM path is bit-identical to the
 // reference; the DDPM path differs only by the ulp of expf.
+//
+// SEEDED (fidm_sampler_step_seeded): the step noise z and the injection noise are not read but generated in registers
+// (philox.cuh), with the values fidm_randn_seeded writes for the same draws: DDIM eta=0 then moves 52 B per pixel.
 #include "sampler_common.cuh"
 
 namespace fidm {
 
+template <bool SEEDED>
 struct StepParams {
   fidm_step_args a;
+};
+template <>
+struct StepParams<true> {
+  fidm_step_args a;
+  fidm_seeded_noise s;
 };
 
 __device__ __forceinline__ float clamp1(float v) { return fminf(fmaxf(v, -1.0f), 1.0f); }
 
-template <int VEC>
-__global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams p) {
+template <int VEC, bool SEEDED>
+__global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams<SEEDED> p) {
   const fidm_step_args& a = p.a;
   const int hw_v = a.hw / VEC;
   const long long total = (long long)a.batch * a.channels * hw_v;
@@ -31,7 +40,7 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams p) {
     const long long off = e.off;
 
     int t_upd = a.t_update, t_inj = a.t_inject;
-    if (a.t_dev) {
+    if (!SEEDED && a.t_dev) {
       t_upd = (int)a.t_dev[b];
       t_inj = (a.mode == FIDM_STEP_INJECT_ONLY) ? t_upd : t_upd - 1;
     }
@@ -41,17 +50,28 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams p) {
     // the log-variance (DDIM: 64 B per pixel instead of 76).
     const bool upd = a.mode != FIDM_STEP_INJECT_ONLY, inj = a.mode != FIDM_STEP_UPDATE_ONLY;
     const bool need_var = upd && a.var_type != FIDM_VAR_FIXED && (a.sampler == FIDM_SAMPLER_DDPM || a.logvar_out != nullptr);
-    const bool need_z = upd && (a.z != nullptr);
+    bool has_z;
+    if constexpr (SEEDED) has_z = p.s.draw >= 0;
+    else has_z = a.z != nullptr;
+    const bool need_z = upd && has_z;
     const int oc = (a.var_type == FIDM_VAR_FIXED) ? a.channels : 2 * a.channels;
     const long long ooff = ((long long)b * oc + c) * a.hw + (long long)e.pv * VEC;
     float xs[VEC], mo[VEC], vv[VEC], zz[VEC], g[VEC], n[VEC], m[VEC];
     load_vec<float, VEC>(a.x + off, xs);
     if (upd) load_vec<float, VEC>(a.model_out + ooff, mo);
     if (need_var) load_vec<float, VEC>(a.model_out + ooff + (long long)a.channels * a.hw, vv);
-    if (need_z) load_vec<float, VEC>(a.z + off, zz);
+    if (need_z) {
+      if constexpr (SEEDED)
+        seeded_elem_normals<VEC>(p.s, e, a.hw, FIDM_NOISE_STEP, p.s.draw, zz);
+      else
+        load_vec<float, VEC>(a.z + off, zz);
+    }
     if (inj) {
       load_vec<float, VEC>(a.gt + off, g);
-      load_vec<float, VEC>(a.inject_noise + off, n);
+      if constexpr (SEEDED)
+        seeded_elem_normals<VEC>(p.s, e, a.hw, p.s.inject_tag, p.s.inject_draw, n);
+      else
+        load_vec<float, VEC>(a.inject_noise + off, n);
       load_vec<float, VEC>(a.keep_mask + e.moff, m);
     }
     float smp[VEC], x0v[VEC];
@@ -138,31 +158,48 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams p) {
   }
 }
 
+// The unseeded (s == nullptr) and seeded entries; `who` prefixes the error text.
+static int sampler_step(const fidm_step_args* a, const fidm_seeded_noise* s, fidm_stream_t stream, const char* who) {
+  FIDM_REQUIRE(a != nullptr, FIDM_E_BADARG, "%s: null args", who);
+  FIDM_REQUIRE(a->batch > 0 && a->channels > 0 && a->hw > 0, FIDM_E_BADARG, "%s: empty shape", who);
+  FIDM_REQUIRE(a->mode >= 0 && a->mode <= 2, FIDM_E_BADARG, "%s: bad mode %d", who, a->mode);
+  FIDM_REQUIRE(a->coef && a->x, FIDM_E_BADARG, "%s: coef/x are required", who);
+  if (int rc = check_mask_channels(a, who)) return rc;
+  if (s) {
+    if (int rc = check_seeded(s, a->mode != FIDM_STEP_UPDATE_ONLY, who)) return rc;
+    FIDM_REQUIRE(a->z == nullptr && a->inject_noise == nullptr && a->t_dev == nullptr, FIDM_E_BADARG,
+                 "%s: z/inject_noise/t_dev must be NULL", who);
+    FIDM_REQUIRE(s->draw >= -1, FIDM_E_BADARG, "%s: step noise draw %d < -1", who, s->draw);
+  }
+  if (a->mode != FIDM_STEP_INJECT_ONLY) {
+    FIDM_REQUIRE(a->model_out != nullptr, FIDM_E_BADARG, "%s: model_out required for an update", who);
+    FIDM_REQUIRE(a->t_dev || (a->t_update >= 0 && a->t_update < a->num_timesteps), FIDM_E_BADARG,
+                 "%s: t_update %d out of range [0,%d)", who, a->t_update, a->num_timesteps);
+  }
+  if (a->mode != FIDM_STEP_UPDATE_ONLY) {
+    FIDM_REQUIRE(a->gt && a->keep_mask && (s || a->inject_noise), FIDM_E_BADARG,
+                 "%s: gt/keep_mask/inject_noise required for an injection", who);
+    FIDM_REQUIRE(a->t_dev || (a->t_inject >= 0 && a->t_inject < a->num_timesteps), FIDM_E_BADARG,
+                 "%s: t_inject %d out of range [0,%d)", who, a->t_inject, a->num_timesteps);
+  }
+  if (int rc = check_stem(a, who)) return rc;
+  const bool vec4 = vec4_ok(a->hw, a->x, a->model_out, a->z, a->gt, a->keep_mask, a->inject_noise, a->sample,
+                            a->pred_xstart, a->x_next, a->mean_out, a->logvar_out);
+  const long long elems = (long long)a->batch * a->channels * a->hw;
+  if (s)
+    return launch_sampler(sampler_step_kernel<4, true>, sampler_step_kernel<1, true>, vec4, elems,
+                          StepParams<true>{*a, *s}, stream, who);
+  return launch_sampler(sampler_step_kernel<4, false>, sampler_step_kernel<1, false>, vec4, elems,
+                        StepParams<false>{*a}, stream, who);
+}
+
 }  // namespace fidm
 
 extern "C" int fidm_sampler_step(const fidm_step_args* a, fidm_stream_t stream) {
-  using namespace fidm;
-  FIDM_REQUIRE(a != nullptr, FIDM_E_BADARG, "sampler_step: null args");
-  FIDM_REQUIRE(a->batch > 0 && a->channels > 0 && a->hw > 0, FIDM_E_BADARG, "sampler_step: empty shape");
-  FIDM_REQUIRE(a->mode >= 0 && a->mode <= 2, FIDM_E_BADARG, "sampler_step: bad mode %d", a->mode);
-  FIDM_REQUIRE(a->coef && a->x, FIDM_E_BADARG, "sampler_step: coef/x are required");
-  if (int rc = check_mask_channels(a, "sampler_step")) return rc;
-  if (a->mode != FIDM_STEP_INJECT_ONLY) {
-    FIDM_REQUIRE(a->model_out != nullptr, FIDM_E_BADARG, "sampler_step: model_out required for an update");
-    FIDM_REQUIRE(a->t_dev || (a->t_update >= 0 && a->t_update < a->num_timesteps), FIDM_E_BADARG,
-                 "sampler_step: t_update %d out of range [0,%d)", a->t_update, a->num_timesteps);
-  }
-  if (a->mode != FIDM_STEP_UPDATE_ONLY) {
-    FIDM_REQUIRE(a->gt && a->keep_mask && a->inject_noise, FIDM_E_BADARG,
-                 "sampler_step: gt/keep_mask/inject_noise required for an injection");
-    FIDM_REQUIRE(a->t_dev || (a->t_inject >= 0 && a->t_inject < a->num_timesteps), FIDM_E_BADARG,
-                 "sampler_step: t_inject %d out of range [0,%d)", a->t_inject, a->num_timesteps);
-  }
-  if (int rc = check_stem(a, "sampler_step")) return rc;
-  StepParams p;
-  p.a = *a;
-  const bool vec4 = vec4_ok(a->hw, a->x, a->model_out, a->z, a->gt, a->keep_mask, a->inject_noise, a->sample,
-                            a->pred_xstart, a->x_next, a->mean_out, a->logvar_out);
-  return launch_sampler(sampler_step_kernel<4>, sampler_step_kernel<1>, vec4,
-                        (long long)a->batch * a->channels * a->hw, p, stream, "sampler_step");
+  return fidm::sampler_step(a, nullptr, stream, "sampler_step");
+}
+
+extern "C" int fidm_sampler_step_seeded(const fidm_step_args* a, const fidm_seeded_noise* s, fidm_stream_t stream) {
+  FIDM_REQUIRE(s != nullptr, FIDM_E_BADARG, "sampler_step_seeded: seeded noise is required");
+  return fidm::sampler_step(a, s, stream, "sampler_step_seeded");
 }

@@ -3,7 +3,8 @@
 Drop-in for the sampling half of the reference's class (`gaussian_diffusion.py:27-538, 640-700`):
 same constructor, attribute names, method names, argument order and defaults, same RNG draw order
 (`randn(shape)` once, then per step `randn_like(gt)` on an injection-cache miss and `randn_like(x)`),
-so seeding torch's generator reproduces the reference's noise on the same device.
+so seeding torch's generator reproduces the reference's noise on the same device.  With `seeds=` the fused loops instead
+generate every noise value inside the sampler kernels from per-image seeds (seeded.py), independent of the batch.
 
 What differs is the execution.  Per step the reference launches ~40 elementwise ATen kernels,
 re-uploads 14 coefficient tables and synchronises on `.item()` (`:131`); here a step is ONE fused
@@ -22,7 +23,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from . import dpm_solver, repaint
+from . import dpm_solver, repaint, seeded
 from .losses import LossType, ModelMeanType, ModelVarType  # noqa: F401
 
 try:  # tqdm is only used when progress=True, as in the reference
@@ -53,7 +54,7 @@ def _set_injection(a, x, gt, keep, inject_noise):
     """Point the known-region fields of a sampler arg struct (StepArgs, MultistepArgs, ResampleArgs) at fp32 copies of
     gt, keep and inject_noise.  Returns the copies: the caller holds them until the launch."""
     gt, keep, inject_noise = _f32(gt), _f32(keep), _f32(inject_noise)
-    assert gt.shape == x.shape and inject_noise.shape == x.shape
+    assert gt.shape == x.shape and (inject_noise is None or inject_noise.shape == x.shape)
     assert keep.shape[0] == x.shape[0] and keep.shape[2:] == x.shape[2:], tuple(keep.shape)
     a.gt, a.keep_mask, a.inject_noise = L.ptr(gt), L.ptr(keep), L.ptr(inject_noise)
     a.mask_channels = keep.shape[1]
@@ -77,6 +78,22 @@ def _known_region(model_kwargs, use_inpainting_injection):
         if gt is not None and keep is not None:
             return gt, keep
     return None, None
+
+
+class _TorchDraws:
+    """The noise of one unseeded loop: torch's generator, in the reference's draw order (the injection noise through
+    the per-timestep cache when cumulative, drawn like `gt`)."""
+
+    def __init__(self, diffusion, gt, cumulative):
+        self.diffusion, self.gt, self.cumulative = diffusion, gt, cumulative
+
+    def inject(self, ts):
+        return self.diffusion._cached_noise(self.gt, ts) if self.cumulative else torch.randn_like(self.gt)
+
+    def step(self, x, k):
+        return torch.randn_like(x)
+
+    undo = step
 
 
 _MEAN_CODE = {ModelMeanType.PREVIOUS_X: L.MEAN_PREVIOUS_X, ModelMeanType.START_X: L.MEAN_START_X,
@@ -165,7 +182,11 @@ class GaussianDiffusion:
               stem=None, t_next=None, next_buf=None):
         """One K4 launch.  stem = (NHWC network-input tensor, timestep tensor) of an engine plan: the state after this call
         is also written as the first channels of the stem input and `t_next` into the timestep tensor (step-boundary
-        fusion); next_buf: preallocated fp32 tensor for x_next."""
+        fusion); next_buf: preallocated fp32 tensor for x_next.  z / inject_noise may be seeded.Draw values: the launch is
+        then the seeded entry, which generates them in the kernel."""
+        sn = seeded.launch_args(z, inject_noise)
+        if sn is not None:
+            z = inject_noise = None
         L.require_cuda(x, model_out, z, gt, keep, inject_noise)
         B, Cn = x.shape[0], x.shape[1]
         hw = x.numel() // (B * Cn)
@@ -213,7 +234,10 @@ class GaussianDiffusion:
                 out[key] = next_buf if (key == "x_next" and next_buf is not None) else torch.empty_like(x)
                 setattr(a, field, L.ptr(out[key]))
         _set_stem(a, stem, t_next)
-        L.check(L.lib().fidm_sampler_step(C.byref(a), L.stream()), "sampler_step")
+        if sn is None:
+            L.check(L.lib().fidm_sampler_step(C.byref(a), L.stream()), "sampler_step")
+        else:
+            L.check(L.lib().fidm_sampler_step_seeded(C.byref(a), C.byref(sn), L.stream()), "sampler_step_seeded")
         return out
 
     # ------------------------------------------------------------------ forward process helpers
@@ -427,26 +451,35 @@ class GaussianDiffusion:
         return {"sample": r["sample"], "pred_xstart": r["pred_xstart"]}
 
     # ------------------------------------------------------------------ loops
-    def _x_T(self, model, shape, noise, device):
-        """The device default and x_T of every loop: `noise`, or one randn(shape) draw; FidmError for a CPU x_T."""
+    def _x_T(self, model, shape, noise, device, seeds=None):
+        """The device default and x_T of every loop: `noise`, or one randn(shape) draw, or with `seeds` (checked CPU
+        tensor) the seeded draw (XT, 0); FidmError for a CPU x_T.  Returns (device, x_T, seeds on the device)."""
         if device is None:
             device = next(model.parameters()).device
         assert isinstance(shape, (tuple, list))
-        img = noise if noise is not None else torch.randn(*shape, device=device)
+        if seeds is not None:
+            seeds = seeds.to(device)
+        if noise is not None:
+            img = noise
+        elif seeds is None:
+            img = torch.randn(*shape, device=device)
+        else:
+            img = seeded.randn(seeds, shape, L.NOISE_XT, 0)
         L.require_cuda(img)
-        return device, img
+        return device, img, seeds
 
-    def _loop_start(self, model, shape, noise, device, mk, gt, keep, t_first, injection_schedule, cumulative):
+    def _loop_start(self, model, shape, noise, device, mk, gt, keep, t_first, injection_schedule, cumulative, seeds):
         """Prologue of the fused loops (K4, K6, K7).  gt / keep: the known region, None without injection; the
-        injection noise is drawn like `gt` as given.  Returns (x, inj_noise, evaluate, stem, bufs):
+        injection noise is drawn like `gt` as given.  Returns (x, rng, evaluate, stem, bufs):
         x, the fp32 contiguous state the first evaluation (at t_first) sees, after the injection on x_T;
-        inj_noise(ts), the injection noise at ts; evaluate(x, t), the model output at t;
-        stem, the engine plan's (network input, timestep tensor) or None; bufs, two state buffers to alternate
-        between on the plan, or None (x is bufs[0] after an injection on the plan)."""
-        device, img = self._x_T(model, shape, noise, device)
-
-        def inj_noise(ts):
-            return self._cached_noise(gt, ts) if cumulative else torch.randn_like(gt)
+        rng, the loop's noise: rng.inject(ts) at timestep ts, rng.step(x, k) and rng.undo(x, k) of evaluation k -- torch
+        tensors, or with `seeds` seeded.Draw values that the launchers turn into seeded launches;
+        evaluate(x, t), the model output at t; stem, the engine plan's (network input, timestep tensor) or None;
+        bufs, two state buffers to alternate between on the plan, or None (x is bufs[0] after an injection on the plan)."""
+        if seeds is not None:
+            seeds = seeded.check_seeds(seeds, shape[0])
+        device, img, seeds = self._x_T(model, shape, noise, device, seeds)
+        rng = _TorchDraws(self, gt, cumulative) if seeds is None else seeded.SeededDraws(seeds, cumulative)
 
         # Step-boundary fusion: when `model` is this package's model_fn (train_inpainting.InpaintingModelFn around a
         # DiffusionInpaintingModel), the step kernels write the next evaluation's stem channels and timestep themselves
@@ -467,10 +500,10 @@ class GaussianDiffusion:
         stem = (plan.x_in, plan.t_in) if plan is not None else None
         bufs = [torch.empty_like(img), torch.empty_like(img)] if plan is not None else None
         if gt is None or self._injection_gated(t_first, injection_schedule):
-            return img, inj_noise, evaluate, stem, bufs
-        x = self._step(L.STEP_INJECT_ONLY, img, t_inject=t_first, gt=gt, keep=keep, inject_noise=inj_noise(t_first),
+            return img, rng, evaluate, stem, bufs
+        x = self._step(L.STEP_INJECT_ONLY, img, t_inject=t_first, gt=gt, keep=keep, inject_noise=rng.inject(t_first),
                        cumulative=cumulative, want_next=True, stem=stem, next_buf=bufs[0] if bufs else None)["x_next"]
-        return x, inj_noise, evaluate, stem, bufs
+        return x, rng, evaluate, stem, bufs
 
     def _update_inject(self, x, i, model_output, z, gt, keep, inj_noise, stem, next_buf, *, ddim, eta, clip,
                        cumulative, injection_schedule, want_out):
@@ -501,7 +534,7 @@ class GaussianDiffusion:
 
     def _loop(self, ddim, model, shape, noise, clip_denoised, denoised_fn, cond_fn, model_kwargs, device,
               progress, eta, use_inpainting_injection, injection_schedule, use_cumulative_noise,
-              progressive):
+              progressive, seeds):
         """Shared fused loop: per step one model call and ONE K4 launch ([update t] -> [inject t-1])."""
         indices = list(range(self.num_timesteps))[::-1]
         if progress and tqdm is not None:
@@ -509,7 +542,10 @@ class GaussianDiffusion:
         mk = model_kwargs
 
         if denoised_fn is not None or cond_fn is not None:       # unfused compatibility path
-            device, img = self._x_T(model, shape, noise, device)
+            if seeds is not None:
+                raise NotImplementedError("seeds are not supported with denoised_fn / cond_fn: that unfused path "
+                                          "draws from torch's generator")
+            device, img, _ = self._x_T(model, shape, noise, device)
             step = self.ddim_sample if ddim else self.p_sample
             extra = {"eta": eta} if ddim else {}
             for i in indices:
@@ -524,15 +560,15 @@ class GaussianDiffusion:
             return
 
         gt, keep = _known_region(mk, use_inpainting_injection)
-        x, inj_noise, evaluate, stem, bufs = self._loop_start(model, shape, noise, device, mk, gt, keep,
-                                                             self.num_timesteps - 1, injection_schedule,
-                                                             use_cumulative_noise)
+        x, rng, evaluate, stem, bufs = self._loop_start(model, shape, noise, device, mk, gt, keep,
+                                                       self.num_timesteps - 1, injection_schedule,
+                                                       use_cumulative_noise, seeds)
         with torch.no_grad():
             for k, i in enumerate(indices):
                 model_output = evaluate(x, i)
-                z = torch.randn_like(x)                              # RNG order: z_t, then n_{t-1}
+                z = rng.step(x, k)                                   # RNG order: z_t, then n_{t-1}
                 want_out = progressive or i == 0
-                r, x = self._update_inject(x, i, model_output, z, gt, keep, inj_noise, stem,
+                r, x = self._update_inject(x, i, model_output, z, gt, keep, rng.inject, stem,
                                            bufs[(k + 1) & 1] if bufs else None, ddim=ddim, eta=eta, clip=clip_denoised,
                                            cumulative=use_cumulative_noise, injection_schedule=injection_schedule,
                                            want_out=want_out)
@@ -542,36 +578,40 @@ class GaussianDiffusion:
     def p_sample_loop_progressive(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None,
                                   cond_fn=None, model_kwargs=None, device=None, progress=False,
                                   use_inpainting_injection=False, injection_schedule="all",
-                                  use_cumulative_noise=True):
+                                  use_cumulative_noise=True, seeds=None):
         """Generator over the per-step dicts {"sample", "pred_xstart"} (`:415-445`)."""
         yield from self._loop(False, model, shape, noise, clip_denoised, denoised_fn, cond_fn, model_kwargs,
                               device, progress, 0.0, use_inpainting_injection, injection_schedule,
-                              use_cumulative_noise, True)
+                              use_cumulative_noise, True, seeds)
 
     def ddim_sample_loop_progressive(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None,
                                      cond_fn=None, model_kwargs=None, device=None, progress=False, eta=0.0,
                                      use_inpainting_injection=False, injection_schedule="all",
-                                     use_cumulative_noise=True):
+                                     use_cumulative_noise=True, seeds=None):
         """Generator over the per-step dicts {"sample", "pred_xstart"} (`:508-538`)."""
         yield from self._loop(True, model, shape, noise, clip_denoised, denoised_fn, cond_fn, model_kwargs,
                               device, progress, eta, use_inpainting_injection, injection_schedule,
-                              use_cumulative_noise, True)
+                              use_cumulative_noise, True, seeds)
 
     def p_sample_loop(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None, cond_fn=None,
                       model_kwargs=None, device=None, progress=False, use_inpainting_injection=False,
-                      injection_schedule="all", use_cumulative_noise=True):
-        """DDPM sampling with optional known-region injection (`:390-413`)."""
+                      injection_schedule="all", use_cumulative_noise=True, seeds=None):
+        """DDPM sampling with optional known-region injection (`:390-413`).  seeds: one uint64 per image (a sequence
+        of ints or an int64 / uint64 tensor) -- every noise value is then generated from the image's own seed inside
+        the sampler kernels (seeded.py), so an image's result does not depend on its batch; torch's generator is not
+        used.  The same holds for every loop of this class."""
         return self._last_sample(self._loop(False, model, shape, noise, clip_denoised, denoised_fn, cond_fn,
                                             model_kwargs, device, progress, 0.0, use_inpainting_injection,
-                                            injection_schedule, use_cumulative_noise, False))
+                                            injection_schedule, use_cumulative_noise, False, seeds))
 
     def ddim_sample_loop(self, model, shape, noise=None, clip_denoised=True, denoised_fn=None, cond_fn=None,
                          model_kwargs=None, device=None, progress=False, eta=0.0,
-                         use_inpainting_injection=False, injection_schedule="all", use_cumulative_noise=True):
-        """DDIM sampling with optional known-region injection (`:487-506`)."""
+                         use_inpainting_injection=False, injection_schedule="all", use_cumulative_noise=True,
+                         seeds=None):
+        """DDIM sampling with optional known-region injection (`:487-506`); seeds as in p_sample_loop."""
         return self._last_sample(self._loop(True, model, shape, noise, clip_denoised, denoised_fn, cond_fn,
                                             model_kwargs, device, progress, eta, use_inpainting_injection,
-                                            injection_schedule, use_cumulative_noise, False))
+                                            injection_schedule, use_cumulative_noise, False, seeds))
 
     # ------------------------------------------------------------------ DPM-Solver++ multistep (K6)
     def _dpm_table(self, device, steps, order, cumulative):
@@ -584,7 +624,11 @@ class GaussianDiffusion:
                    inject_noise=None, stem=None, t_next=None):
         """One K6 launch with row `step` of the table `tab`: returns (m_k, state at t_{k+1} or None).  m_prev selects
         the second-order update; gt / keep / inject_noise the injection; stem = (NHWC network input, timestep tensor)
-        of an engine plan receives the new state and `t_next` (step-boundary fusion, as in _step)."""
+        of an engine plan receives the new state and `t_next` (step-boundary fusion, as in _step).  inject_noise may be a
+        seeded.Draw (a seeded launch)."""
+        sn = seeded.launch_args(None, inject_noise)
+        if sn is not None:
+            inject_noise = None
         L.require_cuda(x, model_out, m_prev, gt, keep, inject_noise)
         B, Cn = x.shape[0], x.shape[1]
         model_out = _f32(model_out)
@@ -601,11 +645,14 @@ class GaussianDiffusion:
             a.inject = 1
             gt, keep, inject_noise = _set_injection(a, x, gt, keep, inject_noise)
         _set_stem(a, stem, t_next)
-        L.check(L.lib().fidm_multistep_step(C.byref(a), L.stream()), "multistep_step")
+        if sn is None:
+            L.check(L.lib().fidm_multistep_step(C.byref(a), L.stream()), "multistep_step")
+        else:
+            L.check(L.lib().fidm_multistep_step_seeded(C.byref(a), C.byref(sn), L.stream()), "multistep_step_seeded")
         return m, nxt
 
     def _dpm_solver_loop(self, model, shape, steps, order, noise, clip_denoised, model_kwargs, device, progress,
-                         use_inpainting_injection, injection_schedule, use_cumulative_noise):
+                         use_inpainting_injection, injection_schedule, use_cumulative_noise, seeds):
         """Per evaluation one model call and ONE K6 launch (x0 prediction, update, injection, next stem input)."""
         if self.model_mean_type == ModelMeanType.PREVIOUS_X:
             raise NotImplementedError("DPM-Solver++ needs an eps or x0 prediction; PREVIOUS_X models are not supported")
@@ -615,8 +662,8 @@ class GaussianDiffusion:
         gt, keep = _known_region(mk, use_inpainting_injection)
         if gt is not None:           # once per loop; the injection noise is drawn like the fp32 copy
             gt, keep = _f32(gt), _f32(keep)
-        x, inj_noise, evaluate, stem, _ = self._loop_start(model, shape, noise, device, mk, gt, keep, int(grid[0]),
-                                                            injection_schedule, use_cumulative_noise)
+        x, rng, evaluate, stem, _ = self._loop_start(model, shape, noise, device, mk, gt, keep, int(grid[0]),
+                                                      injection_schedule, use_cumulative_noise, seeds)
         tab = self._dpm_table(x.device, steps, order, use_cumulative_noise)
         ks = range(steps)
         if progress and tqdm is not None:
@@ -633,7 +680,7 @@ class GaussianDiffusion:
                 do_inj = gt is not None and not self._injection_gated(nxt, injection_schedule)
                 m, x = self._multistep(tab, k, x, model_output, m_prev=m_prev if orders[k] == 2 else None,
                                        clip=clip_denoised, gt=gt if do_inj else None, keep=keep if do_inj else None,
-                                       inject_noise=inj_noise(nxt) if do_inj else None, stem=stem,
+                                       inject_noise=rng.inject(nxt) if do_inj else None, stem=stem,
                                        t_next=self._t_value(nxt))
                 m_prev = m
                 yield {"sample": x, "pred_xstart": m}
@@ -641,33 +688,38 @@ class GaussianDiffusion:
     def dpm_solver_sample_loop_progressive(self, model, shape, steps=20, order=2, noise=None, clip_denoised=True,
                                            model_kwargs=None, device=None, progress=False,
                                            use_inpainting_injection=False, injection_schedule="all",
-                                           use_cumulative_noise=True):
+                                           use_cumulative_noise=True, seeds=None):
         """Generator over one dict {"sample", "pred_xstart"} per model evaluation of dpm_solver_sample_loop:
         "sample" is the state the next evaluation sees (after the injection), and the x0 prediction at t = 0 for the
         last one; "pred_xstart" is the x0 prediction of that evaluation.  Every yielded tensor is a fresh buffer."""
         yield from self._dpm_solver_loop(model, shape, steps, order, noise, clip_denoised, model_kwargs, device,
-                                         progress, use_inpainting_injection, injection_schedule, use_cumulative_noise)
+                                         progress, use_inpainting_injection, injection_schedule, use_cumulative_noise,
+                                         seeds)
 
     def dpm_solver_sample_loop(self, model, shape, steps=20, order=2, noise=None, clip_denoised=True,
                                model_kwargs=None, device=None, progress=False, use_inpainting_injection=False,
-                               injection_schedule="all", use_cumulative_noise=True):
+                               injection_schedule="all", use_cumulative_noise=True, seeds=None):
         """DPM-Solver++ (multistep, `order` 1 or 2) in `steps` model evaluations on the timesteps
         round(linspace(T - 1, 0, steps)) of this diffusion's own table, with the class path's known-region injection
         (on x_T, then after every update) and RNG draw order (randn(shape), then one injection noise per injection;
-        the solver itself draws nothing).  Returns the x0 prediction at t = 0."""
+        the solver itself draws nothing; seeds as in p_sample_loop).  Returns the x0 prediction at t = 0."""
         return self._last_sample(self._dpm_solver_loop(model, shape, steps, order, noise, clip_denoised, model_kwargs,
                                                        device, progress, use_inpainting_injection, injection_schedule,
-                                                       use_cumulative_noise))
+                                                       use_cumulative_noise, seeds))
 
     # ------------------------------------------------------------------ RePaint resampling (K4 + K7)
     def _resample(self, x, u, undo_a, undo_s, *, t_inject=None, gt=None, keep=None, inject_noise=None, cumulative=True,
                   stem=None, t_next=None, next_buf=None):
         """One K7 launch: x' = undo_a*x + undo_s*u, then (t_inject not None) the injection at t_inject with the class
         table's coefficients; stem = (NHWC network input, timestep tensor) of an engine plan receives the new state and
-        `t_next` (step-boundary fusion, as in _step).  Returns the new state (next_buf when given)."""
+        `t_next` (step-boundary fusion, as in _step).  u / inject_noise may be seeded.Draw values (a seeded launch).
+        Returns the new state (next_buf when given)."""
+        sn = seeded.launch_args(u, inject_noise)
+        if sn is not None:
+            u = inject_noise = None
         L.require_cuda(x, u, gt, keep, inject_noise)
         x, u = _f32(x), _f32(u)
-        assert u.shape == x.shape, (tuple(u.shape), tuple(x.shape))
+        assert u is None or u.shape == x.shape, (tuple(u.shape), tuple(x.shape))
         B, Cn = x.shape[0], x.shape[1]
         a = L.ResampleArgs()
         a.batch, a.channels, a.hw = B, Cn, x.numel() // (B * Cn)
@@ -684,12 +736,17 @@ class GaussianDiffusion:
             a.inject = 1
             a.inject_a, a.inject_s = float(cls[t_inject, ia]), float(cls[t_inject, is_])
         _set_stem(a, stem, t_next)
-        L.check(L.lib().fidm_resample_undo(C.byref(a), L.stream()), "resample_undo")
+        if sn is None:
+            L.check(L.lib().fidm_resample_undo(C.byref(a), L.stream()), "resample_undo")
+        else:
+            L.check(L.lib().fidm_resample_undo_seeded(C.byref(a), C.byref(sn), L.stream()), "resample_undo_seeded")
         return out
 
-    def _repaint_plan(self, jump_length, jump_n_sample, model_kwargs, use_inpainting_injection):
+    def _repaint_plan(self, jump_length, jump_n_sample, model_kwargs, use_inpainting_injection, shape, seeds):
         """The evaluation plan, after every argument check (raises ValueError before any RNG draw or GPU work)."""
         plan = repaint.evaluation_plan(self.alphas_cumprod, jump_length, jump_n_sample)
+        if seeds is not None:
+            seeded.check_seeds(seeds, shape[0])
         if not use_inpainting_injection:
             raise ValueError("RePaint resampling needs the known-region injection (use_inpainting_injection=True)")
         if not model_kwargs or model_kwargs.get("gt") is None or model_kwargs.get("gt_keep_mask") is None:
@@ -697,32 +754,32 @@ class GaussianDiffusion:
         return plan
 
     def _repaint_loop(self, evals, model, shape, noise, clip_denoised, model_kwargs, device, progress,
-                      injection_schedule, use_cumulative_noise, progressive):
+                      injection_schedule, use_cumulative_noise, progressive, seeds):
         """Per evaluation one model call and one K4 launch; when a jump follows the evaluation, K4 only updates and
         one K7 launch re-noises to t_up, injects at t_up and writes the next stem input."""
         mk = model_kwargs
         gt, keep = mk["gt"], mk["gt_keep_mask"]
-        x, inj_noise, evaluate, stem, bufs = self._loop_start(model, shape, noise, device, mk, gt, keep, evals[0].t,
-                                                             injection_schedule, use_cumulative_noise)
+        x, rng, evaluate, stem, bufs = self._loop_start(model, shape, noise, device, mk, gt, keep, evals[0].t,
+                                                       injection_schedule, use_cumulative_noise, seeds)
         if progress and tqdm is not None:
             evals = tqdm(evals)
         with torch.no_grad():
             for k, (i, t_up, undo_a, undo_s) in enumerate(evals):
                 model_output = evaluate(x, i)
-                z = torch.randn_like(x)                              # RNG order: z_t, [u], then n of the next t
+                z = rng.step(x, k)                                   # RNG order: z_t, [u], then n of the next t
                 want_out = progressive or i == 0
                 nbuf = bufs[(k + 1) & 1] if bufs else None
                 if t_up is None:                                     # as _loop's DDPM step
-                    r, x = self._update_inject(x, i, model_output, z, gt, keep, inj_noise, stem, nbuf, ddim=False,
+                    r, x = self._update_inject(x, i, model_output, z, gt, keep, rng.inject, stem, nbuf, ddim=False,
                                                eta=0.0, clip=clip_denoised, cumulative=use_cumulative_noise,
                                                injection_schedule=injection_schedule, want_out=want_out)
                 else:
                     r = self._step(L.STEP_UPDATE_ONLY, x, t=i, model_out=model_output, z=z, ddim=False,
                                    clip=clip_denoised, want_sample=True, want_x0=want_out)
-                    u = torch.randn_like(x)
+                    u = rng.undo(x, k)
                     do_inj = not self._injection_gated(t_up, injection_schedule)
                     x = self._resample(r["sample"], u, undo_a, undo_s, t_inject=t_up if do_inj else None,
-                                       gt=gt, keep=keep, inject_noise=inj_noise(t_up) if do_inj else None,
+                                       gt=gt, keep=keep, inject_noise=rng.inject(t_up) if do_inj else None,
                                        cumulative=use_cumulative_noise, stem=stem, t_next=self._t_value(t_up),
                                        next_buf=nbuf)
                 if want_out:
@@ -731,27 +788,28 @@ class GaussianDiffusion:
     def repaint_sample_loop_progressive(self, model, shape, jump_length=10, jump_n_sample=10, noise=None,
                                         clip_denoised=True, model_kwargs=None, device=None, progress=False,
                                         use_inpainting_injection=True, injection_schedule="all",
-                                        use_cumulative_noise=True):
+                                        use_cumulative_noise=True, seeds=None):
         """Generator over one dict {"sample", "pred_xstart", "t"} per model evaluation of repaint_sample_loop:
         "sample" is the DDPM output of the evaluation at timestep "t", before any undo or injection.  The arguments
         are checked when this is called, before the first draw."""
-        evals = self._repaint_plan(jump_length, jump_n_sample, model_kwargs, use_inpainting_injection)
+        evals = self._repaint_plan(jump_length, jump_n_sample, model_kwargs, use_inpainting_injection, shape, seeds)
         return self._repaint_loop(evals, model, shape, noise, clip_denoised, model_kwargs, device, progress,
-                                  injection_schedule, use_cumulative_noise, True)
+                                  injection_schedule, use_cumulative_noise, True, seeds)
 
     def repaint_sample_loop(self, model, shape, jump_length=10, jump_n_sample=10, noise=None, clip_denoised=True,
                             model_kwargs=None, device=None, progress=False, use_inpainting_injection=True,
-                            injection_schedule="all", use_cumulative_noise=True):
+                            injection_schedule="all", use_cumulative_noise=True, seeds=None):
         """DDPM sampling with RePaint resampling (Lugmayr et al. 2022): the class path's DDPM step and known-region
         injection, on RePaint's jump schedule (repaint.py) -- every `jump_length` timesteps the state is re-noised
         back up `jump_length` levels and denoised again, `jump_n_sample - 1` times, so that the hole can agree with
         the known region.  T + (jump_n_sample - 1) * jump_length * len(range(0, T - jump_length, jump_length)) model
         evaluations.  RNG draw order: randn(shape), the injection noise at T - 1, then per evaluation the step noise,
         the undo noise if a jump follows, and the injection noise of the next evaluation (with use_cumulative_noise
-        a revisited timestep reuses its cached noise).  Returns the sample at t = 0, not re-blended."""
-        evals = self._repaint_plan(jump_length, jump_n_sample, model_kwargs, use_inpainting_injection)
+        a revisited timestep reuses its cached noise; seeds as in p_sample_loop).  Returns the sample at t = 0, not
+        re-blended."""
+        evals = self._repaint_plan(jump_length, jump_n_sample, model_kwargs, use_inpainting_injection, shape, seeds)
         return self._last_sample(self._repaint_loop(evals, model, shape, noise, clip_denoised, model_kwargs, device,
-                                                    progress, injection_schedule, use_cumulative_noise, False))
+                                                    progress, injection_schedule, use_cumulative_noise, False, seeds))
 
     def sample_with_advanced_inpainting(self, model, shape, gt=None, gt_keep_mask=None, use_ddim=True, eta=0.0,
                                         progress=True, device=None, injection_schedule="all",

@@ -9,6 +9,8 @@ the CPU tests of the host logic).
 import torch
 import torch.distributed as dist
 
+from .seeded import check_seeds
+
 
 def shard_bounds(batch, rank, world_size):
     """[start, stop) of `rank`'s contiguous slice; sizes differ by at most one."""
@@ -38,9 +40,12 @@ def gather_batch(local, batch):
     return torch.cat([bufs[r][: b - a] for r, (a, b) in enumerate(sizes)], dim=0)
 
 
-def sample_sharded(diffusion, model_fn, gt, gt_keep_mask, *, ddim=True, eta=0.0, seed=0, sampler=None, **loop_kwargs):
+def sample_sharded(diffusion, model_fn, gt, gt_keep_mask, *, ddim=True, eta=0.0, seed=0, sampler=None, seeds=None,
+                   **loop_kwargs):
     """Run the inpainting loop on this rank's slice of (gt, gt_keep_mask) and gather the results.
-    Per-rank generator seed = seed + rank (parity is checked shard by shard against the oracle).
+    Per-rank generator seed = seed + rank (parity is checked shard by shard against the oracle).  seeds: one uint64 per
+    image of the whole batch (see GaussianDiffusion.p_sample_loop); each rank then runs its slice of them, `seed` is
+    not used, and every image comes out as it would on one GPU.
     sampler: "ddim" | "ddpm" | "dpm_solver" | "repaint" (None: "ddim" if `ddim` else "ddpm"); `eta` is used by
     "ddim" only, and loop_kwargs go to the chosen loop (steps / order, jump_length / jump_n_sample, ...)."""
     if sampler is None:
@@ -54,10 +59,14 @@ def sample_sharded(diffusion, model_fn, gt, gt_keep_mask, *, ddim=True, eta=0.0,
     if gt.shape[0] < world:
         # an empty shard would make its rank fail in the loop while the others wait in all_gather
         raise ValueError(f"batch {gt.shape[0]} < world size {world}: every rank needs at least one image")
+    if seeds is not None:
+        lo, hi = shard_bounds(gt.shape[0], rank, world)
+        loop_kwargs["seeds"] = check_seeds(seeds, gt.shape[0])[lo:hi].view(torch.uint64)
     g, k = shard(gt, rank, world), shard(gt_keep_mask, rank, world)
-    torch.manual_seed(seed + rank)
-    if g.is_cuda:
-        torch.cuda.manual_seed(seed + rank)
+    if seeds is None:
+        torch.manual_seed(seed + rank)
+        if g.is_cuda:
+            torch.cuda.manual_seed(seed + rank)
     extra = {"eta": eta} if sampler == "ddim" else {}
     out = loops[sampler](model_fn, tuple(g.shape), model_kwargs={"gt": g, "gt_keep_mask": k}, device=g.device,
                          use_inpainting_injection=True, **extra, **loop_kwargs)

@@ -192,6 +192,34 @@ typedef struct fidm_resample_args {
 int fidm_resample_undo(const fidm_resample_args* a, fidm_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Per-image seeded noise.  Every Gaussian value is a function of (the image's uint64 seed, the element's flat NCHW
+ * index j within its image, a tag, a draw) only -- Philox4x32-10 keyed by the seed with counter (j >> 2, draw, tag, 0)
+ * and Box-Muller, specified in csrc/philox.cuh -- so an image's noise does not depend on its batch, its position in it
+ * or the number of GPUs.  The _seeded entries below are the K4 / K6 / K7 entries with their noise tensors generated in
+ * registers instead of read: each takes the same arg struct, requires its noise pointers (z, inject_noise, noise) to
+ * be NULL, and reads the draws from `s`.  fidm_randn_seeded fills a buffer with the same values.
+ * Draws of the sampling loops: x_T (XT, 0); step noise of the k-th evaluation (STEP, k); cumulative injection noise at
+ * timestep t (INJECT, t); the i-th fresh injection of a loop (INJECT_FRESH, i); RePaint undo noise after evaluation k
+ * (UNDO, k).
+ * ---------------------------------------------------------------------------------------------- */
+enum { FIDM_NOISE_XT = 0, FIDM_NOISE_STEP = 1, FIDM_NOISE_INJECT = 2, FIDM_NOISE_INJECT_FRESH = 3, FIDM_NOISE_UNDO = 4 };
+typedef struct fidm_seeded_noise {
+  const uint64_t* seeds;                /* device [batch]: seed of each image */
+  int32_t draw;                         /* K4: draw of the step noise (tag STEP; -1: none, as z == NULL);
+                                           K7: draw of the undo noise (tag UNDO); K6: unused */
+  int32_t inject_tag, inject_draw;      /* the injection noise: FIDM_NOISE_INJECT | FIDM_NOISE_INJECT_FRESH, draw */
+} fidm_seeded_noise;
+/* K4 with a->z and a->inject_noise NULL; a->t_dev must be NULL (one timestep for the whole batch) */
+int fidm_sampler_step_seeded(const fidm_step_args* a, const fidm_seeded_noise* s, fidm_stream_t stream);
+/* K6 with a->inject_noise NULL */
+int fidm_multistep_step_seeded(const fidm_multistep_args* a, const fidm_seeded_noise* s, fidm_stream_t stream);
+/* K7 with a->noise and a->inject_noise NULL */
+int fidm_resample_undo_seeded(const fidm_resample_args* a, const fidm_seeded_noise* s, fidm_stream_t stream);
+/* out[b][j] = the normal of element j of image b under seeds[b], draw (tag, draw); out is [batch][elems_per_image] */
+int fidm_randn_seeded(float* out, const uint64_t* seeds, int32_t batch, int64_t elems_per_image, int32_t tag,
+                      int32_t draw, fidm_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Layout converters.  Replace torch.cat([x, masked_image, mask.repeat(1,3,1,1)], 1) of
  * unet.py:199 and the NCHW activations of the reference with one NHWC (bf16|fp32) tensor padded to
  * `c_pad` channels (zeros).  Up to 3 fp32 NCHW sources; a source with repeat>1 is broadcast.
