@@ -23,6 +23,8 @@ MEAN_PREVIOUS_X, MEAN_START_X, MEAN_EPSILON = 0, 1, 2
 VAR_LEARNED, VAR_FIXED, VAR_LEARNED_RANGE = 0, 1, 2
 RESAMPLE_NONE, RESAMPLE_DOWN, RESAMPLE_UP = 0, 1, 2
 NOISE_XT, NOISE_STEP, NOISE_INJECT, NOISE_INJECT_FRESH, NOISE_UNDO = range(5)
+MAX_SLOTS = 128
+SLOT_IDLE, SLOT_ADMIT = -1, -2
 
 i32, vp, fp, dp = C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p
 
@@ -56,6 +58,11 @@ class ResampleArgs(C.Structure):
 
 class SeededNoise(C.Structure):
     _fields_ = [("seeds", vp), ("draw", i32), ("inject_tag", i32), ("inject_draw", i32)]
+
+
+class SlotArgs(C.Structure):
+    _fields_ = [("t_value", fp), ("inject_draw", vp), ("out", fp), ("step_noise", i32),
+                ("action", i32 * MAX_SLOTS), ("seeds", C.c_uint64 * MAX_SLOTS)]
 
 
 class PackArgs(C.Structure):
@@ -104,6 +111,7 @@ SYMBOLS = {
     "fidm_multistep_step_seeded": (C.c_int, [_P(MultistepArgs), _P(SeededNoise), vp]),
     "fidm_resample_undo_seeded": (C.c_int, [_P(ResampleArgs), _P(SeededNoise), vp]),
     "fidm_randn_seeded": (C.c_int, [fp, vp, i32, C.c_int64, i32, i32, vp]),
+    "fidm_sampler_step_slots": (C.c_int, [_P(StepArgs), _P(SlotArgs), vp]),
     "fidm_pack_nchw_to_nhwc": (C.c_int, [_P(PackArgs), vp]),
     "fidm_unpack_nhwc_to_nchw": (C.c_int, [vp, i32, i32, fp, i32, i32, i32, vp]),
     "fidm_prepare_inputs_u8": (C.c_int, [vp, vp, fp, fp, fp, fp, i32, i32, vp]),

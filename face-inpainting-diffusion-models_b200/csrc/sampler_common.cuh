@@ -1,4 +1,5 @@
-// Pieces shared by the sampler kernels K4 (sampler_step.cu), K6 (sampler_multistep.cu) and K7 (sampler_resample.cu).
+// Pieces shared by the sampler kernels K4 and K8 (sampler_step.cu), K6 (sampler_multistep.cu) and K7
+// (sampler_resample.cu).
 // The fused-versus-unfused tests and the oracles compare these kernels bit for bit, so each piece exists once.
 #pragma once
 #include "common.cuh"
@@ -42,11 +43,11 @@ __device__ __forceinline__ float inject(float v, float m, float g, float n, floa
   return __fadd_rn(__fmul_rn(m, wg), __fmul_rn(__fsub_rn(1.0f, m), v));
 }
 
-// Step-boundary fusion: the next evaluation's stem input (channel c of VEC pixels of the NHWC network input) and its
-// timestep.  The roundings are the pack kernel's (layout.cu), so a fused loop is bit-identical to pack + evaluate.
-// Args is any of the three sampler arg structs; they share these field names.
+// Step-boundary fusion: the next evaluation's stem input (channel c of VEC pixels of the NHWC network input, store_stem)
+// and its timestep (write_stem: one value for the whole batch).  The roundings are the pack kernel's (layout.cu), so a
+// fused loop is bit-identical to pack + evaluate.  Args is any of the sampler arg structs; they share these field names.
 template <int VEC, typename Args>
-__device__ __forceinline__ void write_stem(const Args& a, long long idx, const SamplerElem& e, const float (&v)[VEC]) {
+__device__ __forceinline__ void store_stem(const Args& a, const SamplerElem& e, const float (&v)[VEC]) {
   if (a.stem_out) {
     const long long px = (long long)e.b * a.hw + (long long)e.pv * VEC;
 #pragma unroll
@@ -60,6 +61,11 @@ __device__ __forceinline__ void write_stem(const Args& a, long long idx, const S
         reinterpret_cast<float*>(a.stem_out)[s] = v[i];
     }
   }
+}
+
+template <int VEC, typename Args>
+__device__ __forceinline__ void write_stem(const Args& a, long long idx, const SamplerElem& e, const float (&v)[VEC]) {
+  store_stem<VEC>(a, e, v);
   if (a.t_out && idx < a.batch) a.t_out[idx] = a.t_out_value;
 }
 

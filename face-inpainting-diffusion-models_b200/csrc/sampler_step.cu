@@ -12,6 +12,10 @@
 //
 // SEEDED (fidm_sampler_step_seeded): the step noise z and the injection noise are not read but generated in registers
 // (philox.cuh), with the values fidm_randn_seeded writes for the same draws: DDIM eta=0 then moves 52 B per pixel.
+//
+// K8 (fidm_sampler_step_slots, continuous batching) is the same element body with SLOTS set: the action, the timesteps,
+// the seed and the draws come per slot from the launch parameters, x_T is generated for an admitted slot, and a slot
+// updated at t = 0 writes its sample to a separate buffer.  The update and injection arithmetic is K4's own code.
 #include "sampler_common.cuh"
 
 namespace fidm {
@@ -25,11 +29,24 @@ struct StepParams<true> {
   fidm_step_args a;
   fidm_seeded_noise s;
 };
+struct SlotParams {
+  fidm_step_args a;
+  fidm_slot_args s;
+};
+// The parameters of K4 (SLOTS false) and K8 (SLOTS and SEEDED true).
+template <bool SEEDED, bool SLOTS>
+struct KernelParams {
+  using type = StepParams<SEEDED>;
+};
+template <>
+struct KernelParams<true, true> {
+  using type = SlotParams;
+};
 
 __device__ __forceinline__ float clamp1(float v) { return fminf(fmaxf(v, -1.0f), 1.0f); }
 
-template <int VEC, bool SEEDED>
-__global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams<SEEDED> p) {
+template <int VEC, bool SEEDED, bool SLOTS>
+__global__ void __launch_bounds__(256) sampler_step_kernel(const typename KernelParams<SEEDED, SLOTS>::type p) {
   const fidm_step_args& a = p.a;
   const int hw_v = a.hw / VEC;
   const long long total = (long long)a.batch * a.channels * hw_v;
@@ -39,7 +56,17 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams<SEED
     const int b = e.b, c = e.c;
     const long long off = e.off;
 
+    // K8: the slot's action -- idle, admit (x_T, injection at T-1), or update at t and injection at t-1 -- and the
+    // draw of its injection (< 0: none)
+    int act = 0, slot_inj_draw = -1;
     int t_upd = a.t_update, t_inj = a.t_inject;
+    if constexpr (SLOTS) {
+      act = p.s.action[b];
+      if (act == FIDM_SLOT_IDLE) continue;
+      t_upd = act;
+      t_inj = (act == FIDM_SLOT_ADMIT) ? a.num_timesteps - 1 : act - 1;
+      if (t_inj >= 0) slot_inj_draw = p.s.inject_draw[t_inj];
+    }
     if (!SEEDED && a.t_dev) {
       t_upd = (int)a.t_dev[b];
       t_inj = (a.mode == FIDM_STEP_INJECT_ONLY) ? t_upd : t_upd - 1;
@@ -48,27 +75,41 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams<SEED
     // Every load of this element is issued up front (one memory round trip instead of two dependent ones), and only
     // what the mode needs is read: the variance channels are skipped when neither the DDPM update nor a caller wants
     // the log-variance (DDIM: 64 B per pixel instead of 76).
-    const bool upd = a.mode != FIDM_STEP_INJECT_ONLY, inj = a.mode != FIDM_STEP_UPDATE_ONLY;
+    const bool upd = SLOTS ? act != FIDM_SLOT_ADMIT : a.mode != FIDM_STEP_INJECT_ONLY;
+    const bool inj = SLOTS ? slot_inj_draw >= 0 : a.mode != FIDM_STEP_UPDATE_ONLY;
     const bool need_var = upd && a.var_type != FIDM_VAR_FIXED && (a.sampler == FIDM_SAMPLER_DDPM || a.logvar_out != nullptr);
     bool has_z;
-    if constexpr (SEEDED) has_z = p.s.draw >= 0;
+    if constexpr (SLOTS) has_z = p.s.step_noise != 0;
+    else if constexpr (SEEDED) has_z = p.s.draw >= 0;
     else has_z = a.z != nullptr;
     const bool need_z = upd && has_z;
     const int oc = (a.var_type == FIDM_VAR_FIXED) ? a.channels : 2 * a.channels;
     const long long ooff = ((long long)b * oc + c) * a.hw + (long long)e.pv * VEC;
     float xs[VEC], mo[VEC], vv[VEC], zz[VEC], g[VEC], n[VEC], m[VEC];
-    load_vec<float, VEC>(a.x + off, xs);
+    // K8's draws are those of the slot's seed at the element's flat index j within its image
+    uint64_t seed = 0;
+    long long j = 0;
+    if constexpr (SLOTS) {
+      seed = p.s.seeds[b];
+      j = (long long)c * a.hw + (long long)e.pv * VEC;
+    }
+    if (!SLOTS || upd) load_vec<float, VEC>(a.x + off, xs);
+    else seeded_normals<VEC>(seed, j, FIDM_NOISE_XT, 0u, xs);         // admit: x_T
     if (upd) load_vec<float, VEC>(a.model_out + ooff, mo);
     if (need_var) load_vec<float, VEC>(a.model_out + ooff + (long long)a.channels * a.hw, vv);
     if (need_z) {
-      if constexpr (SEEDED)
+      if constexpr (SLOTS)
+        seeded_normals<VEC>(seed, j, FIDM_NOISE_STEP, (uint32_t)(a.num_timesteps - 1 - t_upd), zz);
+      else if constexpr (SEEDED)
         seeded_elem_normals<VEC>(p.s, e, a.hw, FIDM_NOISE_STEP, p.s.draw, zz);
       else
         load_vec<float, VEC>(a.z + off, zz);
     }
     if (inj) {
       load_vec<float, VEC>(a.gt + off, g);
-      if constexpr (SEEDED)
+      if constexpr (SLOTS)
+        seeded_normals<VEC>(seed, j, a.cumulative ? FIDM_NOISE_INJECT : FIDM_NOISE_INJECT_FRESH, (uint32_t)slot_inj_draw, n);
+      else if constexpr (SEEDED)
         seeded_elem_normals<VEC>(p.s, e, a.hw, p.s.inject_tag, p.s.inject_draw, n);
       else
         load_vec<float, VEC>(a.inject_noise + off, n);
@@ -136,10 +177,12 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams<SEED
           smp[i] = __fadd_rn(mean, __fmul_rn(__fmul_rn(nz, sd), z));
         }
       }
-      if (a.sample) store_vec<float, VEC>(a.sample + off, smp);
-      if (a.pred_xstart) store_vec<float, VEC>(a.pred_xstart + off, x0v);
-      if (a.mean_out) store_vec<float, VEC>(a.mean_out + off, mv);
-      if (a.logvar_out) store_vec<float, VEC>(a.logvar_out + off, lv);
+      if constexpr (!SLOTS) {
+        if (a.sample) store_vec<float, VEC>(a.sample + off, smp);
+        if (a.pred_xstart) store_vec<float, VEC>(a.pred_xstart + off, x0v);
+        if (a.mean_out) store_vec<float, VEC>(a.mean_out + off, mv);
+        if (a.logvar_out) store_vec<float, VEC>(a.logvar_out + off, lv);
+      }
     } else {
 #pragma unroll
       for (int i = 0; i < VEC; ++i) smp[i] = xs[i];
@@ -153,8 +196,18 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const StepParams<SEED
 #pragma unroll
       for (int i = 0; i < VEC; ++i) smp[i] = inject(smp[i], m[i], g[i], n[i], ca, cs);
     }
-    if (a.x_next) store_vec<float, VEC>(a.x_next + off, smp);
-    write_stem<VEC>(a, idx, e, smp);
+    if constexpr (SLOTS) {
+      if (upd && t_upd == 0) {                     // the request's result: kept apart until the host collects it
+        store_vec<float, VEC>(p.s.out + off, smp);
+        continue;
+      }
+      store_vec<float, VEC>(a.x_next + off, smp);
+      store_stem<VEC>(a, e, smp);
+      if (a.t_out && c == 0 && e.pv == 0) a.t_out[b] = p.s.t_value[t_inj];
+    } else {
+      if (a.x_next) store_vec<float, VEC>(a.x_next + off, smp);
+      write_stem<VEC>(a, idx, e, smp);
+    }
   }
 }
 
@@ -187,13 +240,47 @@ static int sampler_step(const fidm_step_args* a, const fidm_seeded_noise* s, fid
                             a->pred_xstart, a->x_next, a->mean_out, a->logvar_out);
   const long long elems = (long long)a->batch * a->channels * a->hw;
   if (s)
-    return launch_sampler(sampler_step_kernel<4, true>, sampler_step_kernel<1, true>, vec4, elems,
+    return launch_sampler(sampler_step_kernel<4, true, false>, sampler_step_kernel<1, true, false>, vec4, elems,
                           StepParams<true>{*a, *s}, stream, who);
-  return launch_sampler(sampler_step_kernel<4, false>, sampler_step_kernel<1, false>, vec4, elems,
+  return launch_sampler(sampler_step_kernel<4, false, false>, sampler_step_kernel<1, false, false>, vec4, elems,
                         StepParams<false>{*a}, stream, who);
 }
 
+static int sampler_step_slots(const fidm_step_args* a, const fidm_slot_args* s, fidm_stream_t stream) {
+  const char* who = "sampler_step_slots";
+  FIDM_REQUIRE(a != nullptr && s != nullptr, FIDM_E_BADARG, "%s: null args", who);
+  FIDM_REQUIRE(a->batch >= 1 && a->batch <= FIDM_MAX_SLOTS, FIDM_E_BADARG, "%s: %d slots outside [1, %d]", who,
+               a->batch, FIDM_MAX_SLOTS);
+  FIDM_REQUIRE(a->channels > 0 && a->hw > 0 && a->num_timesteps > 0, FIDM_E_BADARG, "%s: empty shape", who);
+  FIDM_REQUIRE(a->sampler == FIDM_SAMPLER_DDPM || a->sampler == FIDM_SAMPLER_DDIM, FIDM_E_BADARG,
+               "%s: sampler must be DDPM | DDIM", who);
+  FIDM_REQUIRE(a->coef && a->x && a->x_next && a->gt && a->keep_mask && s->out && s->t_value && s->inject_draw,
+               FIDM_E_BADARG, "%s: coef/x/x_next/gt/keep_mask/out/t_value/inject_draw are required", who);
+  FIDM_REQUIRE(a->z == nullptr && a->inject_noise == nullptr && a->t_dev == nullptr, FIDM_E_BADARG,
+               "%s: z/inject_noise/t_dev must be NULL", who);
+  FIDM_REQUIRE(!a->sample && !a->pred_xstart && !a->mean_out && !a->logvar_out, FIDM_E_BADARG,
+               "%s: sample/pred_xstart/mean_out/logvar_out must be NULL", who);
+  if (int rc = check_mask_channels(a, who)) return rc;
+  bool any_update = false;
+  for (int b = 0; b < a->batch; ++b) {
+    const int act = s->action[b];
+    FIDM_REQUIRE(act == FIDM_SLOT_IDLE || act == FIDM_SLOT_ADMIT || (act >= 0 && act < a->num_timesteps), FIDM_E_BADARG,
+                 "%s: slot %d: action %d is not IDLE, ADMIT or a timestep in [0,%d)", who, b, act, a->num_timesteps);
+    any_update |= act >= 0;
+  }
+  FIDM_REQUIRE(!any_update || a->model_out != nullptr, FIDM_E_BADARG, "%s: model_out required for an update", who);
+  if (int rc = check_stem(a, who)) return rc;
+  const bool vec4 = vec4_ok(a->hw, a->x, a->model_out, a->gt, a->keep_mask, a->x_next, s->out);
+  const long long elems = (long long)a->batch * a->channels * a->hw;
+  return launch_sampler(sampler_step_kernel<4, true, true>, sampler_step_kernel<1, true, true>, vec4, elems,
+                        SlotParams{*a, *s}, stream, who);
+}
+
 }  // namespace fidm
+
+extern "C" int fidm_sampler_step_slots(const fidm_step_args* a, const fidm_slot_args* s, fidm_stream_t stream) {
+  return fidm::sampler_step_slots(a, s, stream);
+}
 
 extern "C" int fidm_sampler_step(const fidm_step_args* a, fidm_stream_t stream) {
   return fidm::sampler_step(a, nullptr, stream, "sampler_step");

@@ -619,6 +619,25 @@ class Plan:
         L.check(self.lib.fidm_pack_nchw_to_nhwc(a, L.stream()), "pack")
         self.t_in.copy_(timesteps[batch_offset:batch_offset + self.B], non_blocking=True)
 
+    def load_slot(self, slot, sources, c0):
+        """Pack the fp32 NCHW `sources` [(tensor [1, channels, H, W], channels, repeat)] of ONE image into image `slot`
+        of the network input, from channel c0 on: the pack kernel with a destination offset.  The other images, the
+        channels outside the sources and the timesteps are left alone (continuous batching admits one request per slot
+        while the sampler step kernel writes the state channels)."""
+        a = L.PackArgs()
+        hw = self.H * self.W
+        a.batch, a.hw, a.n_src = 1, hw, len(sources)
+        total_c = 0
+        for i, (t, c, r) in enumerate(sources):
+            assert t.is_contiguous() and t.dtype == torch.float32 and t.numel() == c * hw, (tuple(t.shape), c)
+            a.src[i] = t.data_ptr()
+            a.src_channels[i], a.src_repeat[i] = c, r
+            total_c += c * r
+        assert 0 <= slot < self.B and c0 + total_c <= 16, (slot, c0, total_c)
+        a.dst = self.x_in.data_ptr() + (slot * hw * STEM_CIN_PAD + c0) * self.x_in.element_size()
+        a.dst_dtype, a.ld_dst, a.c_pad = L.dtype_code(self.x_in.dtype), STEM_CIN_PAD, total_c
+        L.check(self.lib.fidm_pack_nchw_to_nhwc(a, L.stream()), "pack")
+
     def _launch(self, ops):
         st = L.stream()
         for fn, args in ops:

@@ -811,6 +811,20 @@ class GaussianDiffusion:
         return self._last_sample(self._repaint_loop(evals, model, shape, noise, clip_denoised, model_kwargs, device,
                                                     progress, injection_schedule, use_cumulative_noise, False, seeds))
 
+    # ------------------------------------------------------------------ continuous batching (K8)
+    def continuous_sampler(self, model, slots=8, image_size=(256, 256), sampler="ddim", eta=0.0, clip_denoised=True,
+                           use_inpainting_injection=True, injection_schedule="all", use_cumulative_noise=True,
+                           channels=3, device=None, denoised_fn=None, cond_fn=None):
+        """A continuous-batching sampler (continuous.py) over `slots` images of `image_size`: requests of one image
+        each, submitted with their own seed at any time, each run through ddim_sample_loop ("ddim", any eta) or
+        p_sample_loop ("ddpm") on this diffusion's T timesteps, its result bit-identical to that loop run alone with
+        seeds=[seed].  Arguments are checked here and at submit, before any launch."""
+        from .continuous import ContinuousSampler
+        return ContinuousSampler(self, model, slots=slots, image_size=image_size, sampler=sampler, eta=eta,
+                                 clip_denoised=clip_denoised, use_inpainting_injection=use_inpainting_injection,
+                                 injection_schedule=injection_schedule, use_cumulative_noise=use_cumulative_noise,
+                                 channels=channels, device=device, denoised_fn=denoised_fn, cond_fn=cond_fn)
+
     def sample_with_advanced_inpainting(self, model, shape, gt=None, gt_keep_mask=None, use_ddim=True, eta=0.0,
                                         progress=True, device=None, injection_schedule="all",
                                         use_cumulative_noise=True):

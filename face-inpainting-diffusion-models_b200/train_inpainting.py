@@ -60,6 +60,11 @@ def create_model_and_diffusion(checkpoint_path, device, img_size=256):
     return model, diffusion, {"missing_keys": missing, "unexpected_keys": unexpected}
 
 
+def conditioning(gt, gt_keep_mask):
+    """(masked_image, mask) the UNet is fed for the known image gt and its keep mask (test_inp_ddim_100.py:373-385)."""
+    return gt * gt_keep_mask + torch.zeros_like(gt) * (1 - gt_keep_mask), 1 - gt_keep_mask
+
+
 class InpaintingModelFn:
     """The `model_fn` closure every working call site of the reference wraps the model in
     (test_inp_ddim_100.py:373-385): swallows `gt` / `gt_keep_mask`, feeds the UNet
@@ -86,7 +91,7 @@ class InpaintingModelFn:
         # the cache holds references, so identity (not an address that could be recycled) is compared
         k = self._key
         if k is None or k[0] is not gt or k[1] is not gt_keep_mask or k[2:] != (gt._version, gt_keep_mask._version):
-            self._cond = (gt * gt_keep_mask + torch.zeros_like(gt) * (1 - gt_keep_mask), 1 - gt_keep_mask)
+            self._cond = conditioning(gt, gt_keep_mask)
             self._key = (gt, gt_keep_mask, gt._version, gt_keep_mask._version)
         return self._cond
 
@@ -115,6 +120,20 @@ class InpaintingModelFn:
         if not (x.is_cuda and x.dtype == torch.float32 and tuple(x.shape) == tuple(shape)):
             return None
         return inner.fused_plan(x, t_first, masked_image, mask)
+
+    def slot_plan(self, batch, channels, height, width):
+        """Continuous-batching hook (continuous.py): the engine plan of `batch` slots, whose state channels and
+        timesteps the sampler step kernel writes, or None: the caller uses __call__ per iteration."""
+        inner = self.model
+        if getattr(inner, "slot_plan", None) is None:
+            return None
+        return inner.slot_plan(batch, channels, height, width)
+
+    def load_slot(self, plan, slot, gt, gt_keep_mask):
+        """Pack the conditioning channels of one request (gt [1, C, H, W], keep [1, 1 or C, H, W]) into slot `slot` of
+        a plan from slot_plan."""
+        masked_image, mask = conditioning(gt, gt_keep_mask)
+        self.model.load_slot(plan, slot, masked_image, mask)
 
 
 def sample_with_advanced_inpainting(model, diffusion, masked_images, masks, device, num_steps=50, use_ddim=True,

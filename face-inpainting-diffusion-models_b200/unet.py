@@ -185,6 +185,22 @@ class DiffusionInpaintingModel(nn.Module):
         plan.load_inputs(srcs, torch.full((n,), float(t_value), device=x.device, dtype=torch.float32))
         return plan
 
+    def slot_plan(self, batch, channels, height, width):
+        """The engine plan of `batch` slots for continuous batching (continuous.py), or None when the network input
+        [x | masked_image | mask x3] does not fit the 16-channel stem pack or the batch is split into micro-batches.
+        The plan is the one the loops of this batch size use: the caller owns its inputs while it has work."""
+        if 2 * channels + 3 > 16 or self.base_model.micro_batches > 1:
+            return None
+        return self.base_model.plan_for(batch, height, width)
+
+    def load_slot(self, plan, slot, masked_image, mask):
+        """Pack one image's conditioning channels (masked image, mask x3: unet.py:199) into image `slot` of the plan's
+        network input, behind the state channels that the sampler step kernel writes."""
+        c = masked_image.shape[1]
+        rep = 3 if mask.shape[1] == 1 else 1
+        plan.load_slot(slot, [(t.detach().to(torch.float32).contiguous(), t.shape[1], r)
+                              for t, r in ((masked_image, 1), (mask, rep))], c)
+
     def forward(self, x, t, masked_image, mask):
         """cat([x, masked_image, mask x3]) -> base UNet (unet.py:197-200); the concat is fused into the
         NCHW->NHWC pack kernel."""

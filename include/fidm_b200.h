@@ -200,7 +200,7 @@ int fidm_resample_undo(const fidm_resample_args* a, fidm_stream_t stream);
  * be NULL, and reads the draws from `s`.  fidm_randn_seeded fills a buffer with the same values.
  * Draws of the sampling loops: x_T (XT, 0); step noise of the k-th evaluation (STEP, k); cumulative injection noise at
  * timestep t (INJECT, t); the i-th fresh injection of a loop (INJECT_FRESH, i); RePaint undo noise after evaluation k
- * (UNDO, k).
+ * (UNDO, k).  K8 (below) takes the same draws per slot.
  * ---------------------------------------------------------------------------------------------- */
 enum { FIDM_NOISE_XT = 0, FIDM_NOISE_STEP = 1, FIDM_NOISE_INJECT = 2, FIDM_NOISE_INJECT_FRESH = 3, FIDM_NOISE_UNDO = 4 };
 typedef struct fidm_seeded_noise {
@@ -218,6 +218,36 @@ int fidm_resample_undo_seeded(const fidm_resample_args* a, const fidm_seeded_noi
 /* out[b][j] = the normal of element j of image b under seeds[b], draw (tag, draw); out is [batch][elems_per_image] */
 int fidm_randn_seeded(float* out, const uint64_t* seeds, int32_t batch, int64_t elems_per_image, int32_t tag,
                       int32_t draw, fidm_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * K8  per-slot sampler step (continuous batching).  The state [batch][channels][hw] is a fixed set of `batch` SLOTS,
+ * each holding its own seeded request at its own timestep; one launch takes, per slot, the action in s->action:
+ *   FIDM_SLOT_IDLE   nothing is read or written for the slot (state, stem, t_out, out);
+ *   FIDM_SLOT_ADMIT  x_T = draw (XT, 0) under the slot's seed, then the injection at T-1 (unless inject_draw[T-1] < 0),
+ *                    written as the state, the stem channels and t_out[b] = t_value[T-1] -- a seeded loop's prologue;
+ *   t >= 0           K4's seeded STEP_UPDATE_INJECT / STEP_UPDATE_ONLY at t for the slot: step noise (STEP, T-1-t) when
+ *                    s->step_noise, injection at t-1 with draw (INJECT | INJECT_FRESH as a->cumulative,
+ *                    inject_draw[t-1]) unless that is < 0; state, stem and t_out[b] = t_value[t-1] are written, and at
+ *                    t = 0 the sample goes to out[b] instead (state, stem and t_out are left alone).
+ * Every value is bit-identical to what fidm_sampler_step_seeded computes for that image alone (T = a->num_timesteps).
+ * Fields of `a` used: the shape (batch = number of slots, at most FIDM_MAX_SLOTS), sampler (DDPM | DDIM), mean_type,
+ * var_type, clip_denoised, cumulative, mask_channels, num_timesteps, coef, x, model_out (read for updates), gt,
+ * keep_mask, x_next (may equal x: each element is read and written by the same thread), stem_out / stem_dtype /
+ * stem_ld and t_out; mode, t_update, t_inject and t_out_value are ignored, and z, inject_noise, t_dev, sample,
+ * pred_xstart, mean_out and logvar_out must be NULL.  The per-slot control travels by value in the launch parameters:
+ * the host owns the schedule, and no launch reads control state that it or another launch writes.
+ * ---------------------------------------------------------------------------------------------- */
+#define FIDM_MAX_SLOTS 128
+enum { FIDM_SLOT_IDLE = -1, FIDM_SLOT_ADMIT = -2 };
+typedef struct fidm_slot_args {
+  const float* t_value;                 /* device [num_timesteps]: what the model sees for t (_scale_timesteps) */
+  const int32_t* inject_draw;           /* device [num_timesteps]: draw of the injection at t; -1: no injection at t */
+  float* out;                           /* [batch][channels][hw]: the sample of a slot updated at t = 0 */
+  int32_t step_noise;                   /* 1: updates draw step noise (DDPM, DDIM with eta > 0) */
+  int32_t action[FIDM_MAX_SLOTS];       /* per slot: FIDM_SLOT_IDLE | FIDM_SLOT_ADMIT | t (update at t) */
+  uint64_t seeds[FIDM_MAX_SLOTS];       /* per slot: the request's seed */
+} fidm_slot_args;
+int fidm_sampler_step_slots(const fidm_step_args* a, const fidm_slot_args* s, fidm_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Layout converters.  Replace torch.cat([x, masked_image, mask.repeat(1,3,1,1)], 1) of

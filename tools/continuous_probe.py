@@ -1,0 +1,262 @@
+"""Continuous batching on ADM256: one JSON line on stdout.
+
+Workload: ADM256 bf16 (synthetic weights), 256x256, DDIM-50 on a 50-step cosine diffusion, injection on, seeded,
+64 requests with procedural masks covering 5-60 % (utils.synth).  Alternated within each of --rounds rounds (the
+median is reported):
+  (a) each request alone through ddim_sample_loop at batch 1;
+  (b) lockstep ddim_sample_loop batches of 8 (the bound when all requests are known up front);
+  (c) the continuous sampler, 8 slots, all 64 requests queued at once;
+  (d) the continuous sampler fed a deterministic Poisson arrival trace at --load of (b)'s rate.
+For each: images/s, per-request latency from submit (or arrival) to result-ready (p50 / p95, CUDA events recorded at
+completion), mean slot occupancy, and ms per iteration minus ms per evaluation alone (graph replay of the plan at
+that batch), which is the host and sampler-step overhead.  Then K8 (all slots updating, DDIM eta=0, bf16 stem)
+against the seeded K4 at batch 8 and 64, each in a CUDA graph of 20 launches, beside a 2 GiB device-to-device copy.
+The card's name, power limit and clocks are read (not set) in the same call.
+
+    python tools/continuous_probe.py [--rounds 3] [--load 0.8]
+"""
+import argparse
+import ctypes
+import json
+import os
+import random
+import statistics
+import sys
+import time
+
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tools"))
+
+from repaint_probe import copy_gbs, event_ms, gpu_info  # noqa: E402
+
+B, S, T, N = 8, 256, 50, 64
+
+
+def _pct(v, q):
+    v = sorted(v)
+    return v[min(len(v) - 1, int(round(q * (len(v) - 1))))]
+
+
+class _Clock:
+    """GPU time since a synchronised origin, read from events (ms), and the host clock with the same origin (s)."""
+
+    def __init__(self):
+        torch.cuda.synchronize()
+        self.e0 = torch.cuda.Event(enable_timing=True)
+        self.e0.record()
+        self.t0 = time.perf_counter()
+
+    def mark(self):
+        e = torch.cuda.Event(enable_timing=True)
+        e.record()
+        return e
+
+    def ms(self, e):
+        return self.e0.elapsed_time(e)
+
+
+def run_alone(d, fn, gts, keeps, seeds):
+    clk, done = _Clock(), []
+    for k in range(N):
+        d.ddim_sample_loop(fn, (1, 3, S, S), model_kwargs={"gt": gts[k:k + 1], "gt_keep_mask": keeps[k:k + 1]},
+                           device=gts.device, use_inpainting_injection=True, seeds=[seeds[k]])
+        done.append(clk.mark())
+    torch.cuda.synchronize()
+    lat = [clk.ms(e) for e in done]
+    return {"wall_ms": lat[-1], "latency_ms": lat, "occupancy": 1.0, "iterations": N * T}
+
+
+def run_lockstep(d, fn, gts, keeps, seeds):
+    clk, done = _Clock(), []
+    for j in range(0, N, B):
+        d.ddim_sample_loop(fn, (B, 3, S, S), model_kwargs={"gt": gts[j:j + B], "gt_keep_mask": keeps[j:j + B]},
+                           device=gts.device, use_inpainting_injection=True, seeds=seeds[j:j + B])
+        done += [clk.mark()] * B
+    torch.cuda.synchronize()
+    lat = [clk.ms(e) for e in done]
+    return {"wall_ms": lat[-1], "latency_ms": lat, "occupancy": 1.0, "iterations": N // B * T}
+
+
+def run_continuous(d, fn, gts, keeps, seeds, arrivals_s=None):
+    """arrivals_s: host seconds after the origin at which each request arrives (None: all queued at the origin)."""
+    cs = d.continuous_sampler(fn, slots=B, image_size=(S, S), sampler="ddim")
+    clk = _Clock()
+    arrive_ms, done, tickets = {}, {}, {}
+    k, iters, busy = 0, 0, 0
+    while k < N or cs.pending():
+        now = time.perf_counter() - clk.t0
+        while k < N and (arrivals_s is None or arrivals_s[k] <= now):
+            tk = cs.submit(gts[k], keeps[k], seeds[k])
+            tickets[tk] = k
+            arrive_ms[tk] = 0.0 if arrivals_s is None else arrivals_s[k] * 1e3
+            k += 1
+        if not cs.pending():
+            time.sleep(max(0.0, arrivals_s[k] - now))
+            continue
+        busy += min(B, cs.pending())          # slots busy in this iteration (admissions included)
+        for tk, _ in cs.step():
+            done[tk] = clk.mark()
+        iters += 1
+    torch.cuda.synchronize()
+    lat = [clk.ms(done[tk]) - arrive_ms[tk] for tk in tickets]
+    return {"wall_ms": max(clk.ms(e) for e in done.values()), "latency_ms": lat, "occupancy": busy / (iters * B),
+            "iterations": iters}
+
+
+def eval_ms(fn, batch):
+    """ms per evaluation alone: graph replay of the plan of this batch size."""
+    plan = fn.model.base_model.plan_for(batch, S, S)
+    plan.run()
+    return min(event_ms(plan.run, 20) for _ in range(3))
+
+
+def k8_probe(d, batch, dev):
+    """us per step, DDIM eta=0 update + cumulative injection + bf16 stem write: seeded K4 against K8, CUDA graph of 20."""
+    from fidm_b200 import _lib as L
+    from fidm_b200 import continuous, seeded
+    g = torch.Generator(device=dev).manual_seed(batch)
+    x = torch.randn(batch, 3, S, S, device=dev, generator=g)
+    mo = torch.randn(batch, 6, S, S, device=dev, generator=g)
+    gt = torch.rand(batch, 3, S, S, device=dev, generator=g)
+    keep = (torch.rand(batch, 3, S, S, device=dev, generator=g) > 0.5).float()
+    nxt = torch.empty_like(x)
+    x_in = torch.zeros(batch, S, S, 16, device=dev, dtype=torch.bfloat16)
+    t_in = torch.zeros(batch, device=dev)
+    seeds = seeded.check_seeds(list(range(batch)), batch).to(dev)
+    t = 30
+
+    def k4():
+        d._step(L.STEP_UPDATE_INJECT, x, t=t, t_inject=t - 1, model_out=mo, gt=gt, keep=keep,
+                inject_noise=seeded.Draw(seeds, L.NOISE_INJECT, t - 1), ddim=True, want_next=True,
+                stem=(x_in, t_in), t_next=float(t - 1), next_buf=nxt)
+
+    from fidm_b200.gaussian_diffusion import _MEAN_CODE, _VAR_CODE
+    a = L.StepArgs()
+    a.batch, a.channels, a.hw = batch, 3, S * S
+    a.sampler, a.mean_type, a.var_type = L.SAMPLER_DDIM, _MEAN_CODE[d.model_mean_type], _VAR_CODE[d.model_var_type]
+    a.clip_denoised, a.cumulative, a.mask_channels, a.num_timesteps = 1, 1, 3, d.num_timesteps
+    coef = d._coef(dev, 0.0)
+    tv = torch.tensor([d._t_value(v) for v in range(d.num_timesteps)], dtype=torch.float32, device=dev)
+    inj = torch.tensor(continuous.injection_draws(d, "all", True), dtype=torch.int32, device=dev)
+    out = torch.empty_like(x)
+    a.coef, a.x, a.model_out, a.gt, a.keep_mask, a.x_next = (L.ptr(v) for v in (coef, x, mo, gt, keep, nxt))
+    a.stem_out, a.stem_dtype, a.stem_ld, a.t_out = L.ptr(x_in), L.BF16, 16, L.ptr(t_in)
+    s = L.SlotArgs()
+    s.t_value, s.inject_draw, s.out = L.ptr(tv), L.ptr(inj), L.ptr(out)
+    for b in range(batch):
+        s.action[b], s.seeds[b] = t, b
+
+    def k8():
+        L.check(L.lib().fidm_sampler_step_slots(ctypes.byref(a), ctypes.byref(s), L.stream()), "sampler_step_slots")
+
+    # read x 12, model_out 12 (of 24: the variance half is not read by DDIM), gt 12, keep 12; write x 12, stem 6 B
+    nbytes = batch * S * S * (12 + 12 + 12 + 12 + 12 + 6)
+    res = {"batch": batch, "bytes_per_step": nbytes}
+    for name, fn in (("seeded_k4", k4), ("k8", k8)):
+        for _ in range(3):
+            fn()
+        stream = torch.cuda.Stream()
+        stream.wait_stream(torch.cuda.current_stream())
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.stream(stream):
+            with torch.cuda.graph(graph):
+                for _ in range(20):
+                    fn()
+        torch.cuda.current_stream().wait_stream(stream)
+        graph.replay()
+        ms = min(event_ms(graph.replay, 10) for _ in range(3)) / 20
+        res[name] = {"us_per_step": round(ms * 1e3, 2), "gbs": round(nbytes / (ms * 1e-3) / 1e9, 1)}
+        del graph
+    k4()
+    ref, ref_stem, ref_t = nxt.clone(), x_in.clone(), t_in.clone()
+    nxt.zero_(), x_in.zero_(), t_in.zero_()
+    k8()
+    res["k8_equals_k4"] = bool(torch.equal(nxt, ref) and torch.equal(x_in, ref_stem) and torch.equal(t_in, ref_t))
+    return res
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--rounds", type=int, default=3, help="alternating timing rounds (the median is reported)")
+    ap.add_argument("--load", type=float, default=0.8, help="Poisson arrival rate of (d) as a fraction of (b)'s rate")
+    args = ap.parse_args()
+    import fidm_b200 as F
+    from fidm_b200.utils.synth import synth_batch, synth_state_dict
+    dev = torch.device("cuda", 0)
+    F._lib.check(F._lib.lib().fidm_device_supported(0), "device")
+    info = gpu_info()
+    cfg = F.CONFIGS["ADM256"]
+    model = F.DiffusionInpaintingModel(F.UNetModel(**dict(cfg, in_channels=3)))
+    model.load_state_dict(synth_state_dict(cfg, seed=0), strict=True)
+    model.to(dev)
+    model.base_model.set_precision("bf16")
+    fn = F.InpaintingModelFn(model)
+    d = F.create_gaussian_diffusion(steps=T, learn_sigma=True, noise_schedule="cosine")
+    data = synth_batch(N, S, seed=100, device=dev)
+    gts, keeps = data["gt"], data["gt_keep_mask"]
+    seeds = list(range(5000, 5000 + N))
+    with torch.no_grad():
+        # warm-up: plans and graphs of batch 1 and 8, tables; checks that (c) reproduces (a) and (b)
+        lock = d.ddim_sample_loop(fn, (B, 3, S, S), model_kwargs={"gt": gts[:B], "gt_keep_mask": keeps[:B]},
+                                  device=dev, use_inpainting_injection=True, seeds=seeds[:B])
+        alone = d.ddim_sample_loop(fn, (1, 3, S, S), model_kwargs={"gt": gts[:1], "gt_keep_mask": keeps[:1]},
+                                   device=dev, use_inpainting_injection=True, seeds=seeds[:1])
+        cs = d.continuous_sampler(fn, slots=B, image_size=(S, S), sampler="ddim")
+        tk = [cs.submit(gts[k], keeps[k], seeds[k]) for k in range(B)]
+        res_c = cs.drain()
+        cont = torch.cat([res_c[t] for t in tk])
+        checks = {"continuous_equals_lockstep_b8": bool(torch.equal(cont, lock)),
+                  "continuous_equals_alone_b1": bool(torch.equal(cont[:1], alone)),
+                  "lockstep_b8_equals_alone_b1": bool(torch.equal(lock[:1], alone))}
+        ev = {1: eval_ms(fn, 1), B: eval_ms(fn, B)}
+        rate_b = None
+        runs = {"a_alone_b1": lambda: run_alone(d, fn, gts, keeps, seeds),
+                "b_lockstep_b8": lambda: run_lockstep(d, fn, gts, keeps, seeds),
+                "c_continuous_all_queued": lambda: run_continuous(d, fn, gts, keeps, seeds),
+                "d_continuous_poisson": None}
+        got = {name: [] for name in runs}
+        for r in range(args.rounds):
+            for name, run in runs.items():
+                if name == "d_continuous_poisson":
+                    rate = args.load * rate_b                       # requests per second
+                    rng = random.Random(r)
+                    arr, t = [], 0.0
+                    for _ in range(N):
+                        t += rng.expovariate(rate)
+                        arr.append(t)
+                    got[name].append(run_continuous(d, fn, gts, keeps, seeds, arr))
+                else:
+                    got[name].append(run())
+                if name == "b_lockstep_b8" and rate_b is None:
+                    rate_b = N / (got[name][-1]["wall_ms"] * 1e-3)
+        steps = [k8_probe(d, b, dev) for b in (8, 64)]
+    cp = copy_gbs(dev)
+    for st in steps:
+        for name in ("seeded_k4", "k8"):
+            st[name]["fraction_of_copy"] = round(st[name]["gbs"] / cp, 3)
+    out = {"probe": "continuous", "gpu": info,
+           "config": "ADM256 bf16, 256x256, DDIM-50 cosine, injection on, seeded, 8 slots, 64 requests (5-60 % holes), "
+                     "synthetic weights",
+           "checks": checks, "eval_ms_alone": {str(k): round(v, 3) for k, v in ev.items()},
+           "poisson_rate_per_s": round(args.load * rate_b, 3), "copy_gbs": cp, "step": steps, "runs": {}}
+    for name, rs in got.items():
+        batch = 1 if name == "a_alone_b1" else B
+        walls = [r["wall_ms"] for r in rs]
+        med = rs[walls.index(statistics.median_low(walls))]
+        out["runs"][name] = {
+            "images_per_s": round(N / (med["wall_ms"] * 1e-3), 3),
+            "all_images_per_s": [round(N / (w * 1e-3), 3) for w in walls],
+            "latency_p50_ms": round(_pct(med["latency_ms"], 0.5), 1),
+            "latency_p95_ms": round(_pct(med["latency_ms"], 0.95), 1),
+            "mean_slot_occupancy": round(med["occupancy"], 3),
+            "iterations": med["iterations"],
+            "ms_per_iteration": round(med["wall_ms"] / med["iterations"], 3),
+            "overhead_ms_per_iteration": round(med["wall_ms"] / med["iterations"] - ev[batch], 3)}
+    print(json.dumps(out))
+
+
+if __name__ == "__main__":
+    main()
