@@ -18,8 +18,8 @@
 //   * Weights stream through a TMA ring as in K1; the optional 1x1 skip source (nn.py:184,212) rides the same
 //     ring (one stage for its A box, one for its weights) as extra K iterations.
 //   * CTA pair (cta_group::2): each CTA transforms its own 128 pixel rows and stages half of the weight tile.
-//   * Epilogue = K1's (bias, timestep row, residual, bf16 TMA store into concat slices, fused GroupNorm statistics
-//     of the output).
+//   * Epilogue as K1's, from the same pieces (conv_epilogue.cuh): bias, timestep row, residual, bf16 TMA store into
+//     concat slices, fused GroupNorm statistics of the output.
 //   * UP: `up` ResBlocks (nn.py:190-195) -- the halo tile is the 6 x 10 box of the HALF-resolution stream it covers
 //     after a nearest 2x upsample; every source pixel is activated once and stored to its 2 x 2 halo positions.  The
 //     second conv of the block reads its identity skip at (h/2, w/2) (res_half).  BLOCK_N = 16: the 6-channel head
@@ -32,6 +32,8 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "conv_act.cuh"
+#include "conv_epilogue.cuh"
 #include "conv_host.cuh"
 #include "sm100_primitives.cuh"
 
@@ -82,53 +84,6 @@ constexpr int kSmemBytes = kOffBars + 256 + 1024;
 static_assert(kOffCopy % 1024 == 0 && kOffRing % 1024 == 0 && kOffStaging % 1024 == 0, "swizzle-atom alignment");
 static_assert(kSmemBytes <= 227 * 1024, "shared memory budget");
 }  // namespace halo
-
-__device__ __forceinline__ uint32_t ld_shared_u32x4(uint32_t addr, uint32_t& y, uint32_t& z, uint32_t& w) {
-  uint32_t x;
-  asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(x), "=r"(y), "=r"(z), "=r"(w) : "r"(addr));
-  return x;
-}
-__device__ __forceinline__ void st_shared_u32x4(uint32_t addr, uint4 v) {
-  asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-// silu(x*A + B) of two packed bf16 values -> two packed 16-bit results (fp16 or bf16).  h = x*A/2 + B/2, then
-// silu = h + h*tanh(h): one MUFU op per value.  (tanh.approx.f16x2 was tried: ptxas splits it into two MUFU.TANH.F16,
-// so it saves no MUFU issue slots and only costs accuracy.)
-template <bool OUT_F16>
-__device__ __forceinline__ uint32_t act_pair(uint32_t raw, float a0, float b0, float a1, float b1) {
-  const float h0 = fmaf(__uint_as_float(raw << 16), a0, b0);
-  const float h1 = fmaf(__uint_as_float(raw & 0xFFFF0000u), a1, b1);
-  float t0, t1;
-  asm("tanh.approx.f32 %0, %1;" : "=f"(t0) : "f"(h0));
-  asm("tanh.approx.f32 %0, %1;" : "=f"(t1) : "f"(h1));
-  const float y0 = fmaf(h0, t0, h0), y1 = fmaf(h1, t1, h1);
-  if (OUT_F16) {
-    // saturating: |GroupNorm output| <= sqrt(group size) (724 at 256^2), so gamma * (1 + scale) >~ 90 would overflow
-    // fp16 (65504) to inf and poison the whole image through the MMA; satfinite clamps at the cost of nothing
-    uint32_t o;
-    asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(o) : "f"(y1), "f"(y0));
-    return o;
-  }
-  const __nv_bfloat162 o = __floats2bfloat162_rn(y0, y1);
-  return *reinterpret_cast<const uint32_t*>(&o);
-}
-
-// FP8 operand (tcgen05 kind::f8f6f4, e4m3): silu(x*A + B) of two packed bf16 values -> two packed e4m3 bytes (channel 0 in
-// the low byte).  satfinite: e4m3 has no inf, values beyond 448 clamp.
-__device__ __forceinline__ uint32_t act_pair_e4m3(uint32_t raw, float a0, float b0, float a1, float b1) {
-  const float h0 = fmaf(__uint_as_float(raw << 16), a0, b0);
-  const float h1 = fmaf(__uint_as_float(raw & 0xFFFF0000u), a1, b1);
-  float t0, t1;
-  asm("tanh.approx.f32 %0, %1;" : "=f"(t0) : "f"(h0));
-  asm("tanh.approx.f32 %0, %1;" : "=f"(t1) : "f"(h1));
-  const float y0 = fmaf(h0, t0, h0), y1 = fmaf(h1, t1, h1);
-  unsigned short o;
-  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(o) : "f"(y1), "f"(y0));
-  return (uint32_t)o;
-}
-__device__ __forceinline__ void st_shared_u32x2(uint32_t addr, uint32_t x, uint32_t y) {
-  asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(addr), "r"(x), "r"(y) : "memory");
-}
 
 // OPK: operand kind staged by the transform and multiplied with the weights: 0 = bf16, 1 = fp16 (kind::f16),
 // 2 = fp8 e4m3 (kind::f8f6f4: a 128-byte operand row holds 128 channels, so a K slice is TWO 64-channel halo tiles;
@@ -383,12 +338,11 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_constan
           for (int i = 0; i < 4; ++i) {
             v[i] = make_uint4(0u, 0u, 0u, 0u);
             if (col_ok && lyq + 3 * i < kUpH && (unsigned)(lh + 3 * i) < (unsigned)Hs) {
-              uint32_t r1, r2, r3;
-              const uint32_t r0 = ld_shared_u32x4(ro[i] + roff, r1, r2, r3);
-              v[i].x = act_pair<OUT_F16>(r0, c[0].x, c[0].y, c[0].z, c[0].w);
-              v[i].y = act_pair<OUT_F16>(r1, c[1].x, c[1].y, c[1].z, c[1].w);
-              v[i].z = act_pair<OUT_F16>(r2, c[2].x, c[2].y, c[2].z, c[2].w);
-              v[i].w = act_pair<OUT_F16>(r3, c[3].x, c[3].y, c[3].z, c[3].w);
+              const uint4 r = ld_shared_u32x4(ro[i] + roff);
+              v[i].x = act_pair<OUT_F16>(r.x, c[0].x, c[0].y, c[0].z, c[0].w);
+              v[i].y = act_pair<OUT_F16>(r.y, c[1].x, c[1].y, c[1].z, c[1].w);
+              v[i].z = act_pair<OUT_F16>(r.z, c[2].x, c[2].y, c[2].z, c[2].w);
+              v[i].w = act_pair<OUT_F16>(r.w, c[3].x, c[3].y, c[3].z, c[3].w);
             }
           }
           if constexpr (PROF) pf_work += clock64() - pf_t;
@@ -474,10 +428,9 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_constan
             uint2 v8[9];
 #pragma unroll
             for (int i = 0; i < 9; ++i) {
-              uint32_t r1, r2, r3;
-              const uint32_t r0 = ld_shared_u32x4(((i & 1) ? ro_odd : ro_even) + roff + (i >> 1) * (4 * kHW * 128), r1, r2, r3);
-              v8[i].x = act_pair_e4m3(r0, c[0].x, c[0].y, c[0].z, c[0].w) | (act_pair_e4m3(r1, c[1].x, c[1].y, c[1].z, c[1].w) << 16);
-              v8[i].y = act_pair_e4m3(r2, c[2].x, c[2].y, c[2].z, c[2].w) | (act_pair_e4m3(r3, c[3].x, c[3].y, c[3].z, c[3].w) << 16);
+              const uint4 r = ld_shared_u32x4(((i & 1) ? ro_odd : ro_even) + roff + (i >> 1) * (4 * kHW * 128));
+              v8[i].x = act_pair_e4m3(r.x, c[0].x, c[0].y, c[0].z, c[0].w) | (act_pair_e4m3(r.y, c[1].x, c[1].y, c[1].z, c[1].w) << 16);
+              v8[i].y = act_pair_e4m3(r.z, c[2].x, c[2].y, c[2].z, c[2].w) | (act_pair_e4m3(r.w, c[3].x, c[3].y, c[3].z, c[3].w) << 16);
               const bool out = (i == 0) ? first_out : (i == 8) ? last_out : col_out;
               if (out) v8[i] = make_uint2(0u, 0u);
             }
@@ -511,12 +464,11 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_constan
           uint4 v[9];
 #pragma unroll
           for (int i = 0; i < 9; ++i) {
-            uint32_t r1, r2, r3;
-            const uint32_t r0 = ld_shared_u32x4(((i & 1) ? ro_odd : ro_even) + roff + (i >> 1) * (4 * kHW * 128), r1, r2, r3);
-            v[i].x = act_pair<OUT_F16>(r0, c[0].x, c[0].y, c[0].z, c[0].w);
-            v[i].y = act_pair<OUT_F16>(r1, c[1].x, c[1].y, c[1].z, c[1].w);
-            v[i].z = act_pair<OUT_F16>(r2, c[2].x, c[2].y, c[2].z, c[2].w);
-            v[i].w = act_pair<OUT_F16>(r3, c[3].x, c[3].y, c[3].z, c[3].w);
+            const uint4 r = ld_shared_u32x4(((i & 1) ? ro_odd : ro_even) + roff + (i >> 1) * (4 * kHW * 128));
+            v[i].x = act_pair<OUT_F16>(r.x, c[0].x, c[0].y, c[0].z, c[0].w);
+            v[i].y = act_pair<OUT_F16>(r.y, c[1].x, c[1].y, c[1].z, c[1].w);
+            v[i].z = act_pair<OUT_F16>(r.z, c[2].x, c[2].y, c[2].z, c[2].w);
+            v[i].w = act_pair<OUT_F16>(r.w, c[3].x, c[3].y, c[3].z, c[3].w);
             const bool out = (i == 0) ? first_out : (i == 8) ? last_out : col_out;
             if (out) v[i] = make_uint4(0u, 0u, 0u, 0u);
           }
@@ -546,7 +498,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_constan
       o[0] = (unsigned long long)(clock64() - pf_start); o[1] = pf_raw; o[2] = pf_ae; o[3] = pf_work;
     }
   } else {
-    // ==================================================================== epilogue (warps 0-7), as in K1
+    // ==================================================================== epilogue (warps 0-7), as in K1 (conv_epilogue.cuh)
     const int wg = warp >> 2, qw = warp & 3;          // warp (qw) may only touch TMEM lanes [32 qw, 32 qw + 32)
     const int row = qw * 32 + lane;                   // TMEM lane == pixel row of this CTA's box
     const uint32_t lane_sel = (uint32_t)(qw * 32) << 16;
@@ -580,19 +532,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_constan
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive_cluster(&tmem_empty[acc], 0);
-        if (wg == 0) {
-          const long long hw = (long long)p.H * p.W;
-          float* o = p.y_nchw + ((long long)n * p.cout_valid) * hw + (long long)(h0 + hl) * p.W + (w0 + wl);
-#pragma unroll
-          for (int q = 0; q < 16; ++q) {
-            if (q < p.cout_valid) {
-              float val = __uint_as_float(v16[q]);
-              if (p.bias) val += __ldg(p.bias + q);
-              if (p.row_add) val += __ldg(p.row_add + (long long)n * p.ld_row_add + q);
-              o[(long long)q * hw] = val;
-            }
-          }
-        }
+        if (wg == 0) epi::store_head16(p, v16, 0, n, h0 + hl, w0 + wl);
       } else {
 #pragma unroll 1
       for (int ch = wg; ch < BLOCK_N / 64; ch += 2) {
@@ -630,67 +570,19 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_constan
             f[4 * q] *= t.x; f[4 * q + 1] *= t.y; f[4 * q + 2] *= t.z; f[4 * q + 3] *= t.w;
           }
         }
-        if (p.bias) {
-          const float4* b4 = reinterpret_cast<const float4*>(p.bias + cbase);
-#pragma unroll
-          for (int q = 0; q < 16; ++q) {
-            const float4 t = __ldg(b4 + q);
-            f[4 * q] += t.x; f[4 * q + 1] += t.y; f[4 * q + 2] += t.z; f[4 * q + 3] += t.w;
-          }
-        }
-        if (p.row_add) {
-          const float4* r4 = reinterpret_cast<const float4*>(p.row_add + (long long)n * p.ld_row_add + cbase);
-#pragma unroll
-          for (int q = 0; q < 16; ++q) {
-            const float4 t = __ldg(r4 + q);
-            f[4 * q] += t.x; f[4 * q + 1] += t.y; f[4 * q + 2] += t.z; f[4 * q + 3] += t.w;
-          }
-        }
+        if (p.bias) epi::add_f32_row(f, p.bias + cbase);
+        if (p.row_add) epi::add_f32_row(f, p.row_add + (long long)n * p.ld_row_add + cbase);
         if (p.res_tma) {
           mbar_wait(&res_bar[wg], res_phase);
           res_phase ^= 1u;
-          const uint32_t rrow = smem_u32(stage_out) + row * 128;
-#pragma unroll
-          for (int q = 0; q < 8; ++q) {
-            uint32_t u1, u2, u3;
-            const uint32_t u0 = ld_shared_u32x4(rrow + ((q ^ (row & 7)) << 4), u1, u2, u3);
-            const uint32_t u[4] = {u0, u1, u2, u3};
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              f[8 * q + 2 * e] += __uint_as_float(u[e] << 16);
-              f[8 * q + 2 * e + 1] += __uint_as_float(u[e] & 0xFFFF0000u);
-            }
-          }
+          epi::add_bf16_row_smem(f, smem_u32(stage_out) + row * 128, row);
         } else if (p.residual) {
-          const uint4* rs = reinterpret_cast<const uint4*>(p.residual + pix * p.ld_res + cbase);
-#pragma unroll
-          for (int q = 0; q < 8; ++q) {
-            const uint4 t = __ldg(rs + q);
-            const uint32_t u[4] = {t.x, t.y, t.z, t.w};
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              f[8 * q + 2 * e] += __uint_as_float(u[e] << 16);
-              f[8 * q + 2 * e + 1] += __uint_as_float(u[e] & 0xFFFF0000u);
-            }
-          }
+          epi::add_bf16_row(f, p.residual + pix * p.ld_res + cbase);
         }
         // this warpgroup's staging tile was last read by the TMA store of its previous chunk
         if (issuer) bulk_wait_group_read<0>();
         named_bar_sync(bar_a, 128);
-        uint8_t* srow = stage_out + row * 128;
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-          uint4 pk;
-          __nv_bfloat162 b0 = __floats2bfloat162_rn(f[8 * u + 0], f[8 * u + 1]);
-          __nv_bfloat162 b1 = __floats2bfloat162_rn(f[8 * u + 2], f[8 * u + 3]);
-          __nv_bfloat162 b2 = __floats2bfloat162_rn(f[8 * u + 4], f[8 * u + 5]);
-          __nv_bfloat162 b3 = __floats2bfloat162_rn(f[8 * u + 6], f[8 * u + 7]);
-          pk.x = *reinterpret_cast<uint32_t*>(&b0);
-          pk.y = *reinterpret_cast<uint32_t*>(&b1);
-          pk.z = *reinterpret_cast<uint32_t*>(&b2);
-          pk.w = *reinterpret_cast<uint32_t*>(&b3);
-          *reinterpret_cast<uint4*>(srow + ((u ^ (row & 7)) << 4)) = pk;   // 128-byte swizzle
-        }
+        epi::stage_bf16_row(stage_out + row * 128, row, f);
         fence_proxy_async_smem();
         named_bar_sync(bar_b, 128);
         if (issuer) {
@@ -698,23 +590,13 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_constan
           bulk_commit_group();
         }
         if (p.colsum) {
-          // Fused GroupNorm statistics of the OUTPUT (for its consumer): per-channel (sum, sum of squares) of the
-          // bf16 tile just staged; rows 0-63 / 64-127 are separate partial rows (fixed-order fold later).
+          // Fused GroupNorm statistics of the OUTPUT (for its consumer), of the bf16 tile just staged; rows 0-63 /
+          // 64-127 are separate partial rows (fixed-order fold later).
           const int col = row & 63, half = row >> 6;
-          const uint32_t sb0 = smem_u32(stage_out) + (col & 7) * 2;
-          const int cu = col >> 3;
-          float s1 = 0.0f, s2 = 0.0f;
-#pragma unroll 8
-          for (int r = half * 64; r < half * 64 + 64; ++r) {
-            uint32_t rawv;
-            asm volatile("ld.shared.u16 %0, [%1];" : "=r"(rawv) : "r"(sb0 + r * 128 + ((cu ^ (r & 7)) << 4)));
-            const float val = __uint_as_float(rawv << 16);
-            s1 += val;
-            s2 = fmaf(val, val, s2);
-          }
+          const float2 st = epi::staged_col_stats(smem_u32(stage_out), col, half);
           const int slot = (m_blk % tiles_img) * 2 + half;
           float2* dst = reinterpret_cast<float2*>(p.colsum) + ((long long)n * p.colsum_slots + slot) * p.cout + cbase + col;
-          *dst = make_float2(s1, s2);
+          *dst = st;
         }
       }
       }  // BLOCK_N >= 64
@@ -758,13 +640,10 @@ static int launch_conv_halo_t(const fidm_conv_args& a, cudaStream_t st) {
   p.kc2 = a.x2 ? a.cin2 / 64 : 0;
   p.coef = reinterpret_cast<const float2*>(a.gn_coef); p.ld_coef = a.ld_gn_coef;
   p.w_scale = OPK == 2 ? a.w_scale : nullptr;
-  p.bias = a.bias; p.row_add = a.row_add; p.ld_row_add = a.ld_row_add;
-  p.residual = reinterpret_cast<const __nv_bfloat16*>(a.residual); p.ld_res = a.ld_res;
+  set_epilogue_params(p, a);
   p.res_half = a.residual_half_res;
   p.res_tma = (BLOCK_N >= 64 && a.residual && !a.residual_half_res) ? 1 : 0;
-  p.colsum = a.colsum; p.cout = a.cout;
   p.colsum_slots = p.tiles_w * p.tiles_h * 2;
-  p.y_nchw = a.y_nchw_f32 ? reinterpret_cast<float*>(a.y) : nullptr; p.cout_valid = a.cout_valid;
   p.prof = PROF ? g_prof : nullptr;
 
   CUtensorMap tmRaw, tmB, tmA2, tmB2, tmY, tmRes;
@@ -808,16 +687,12 @@ static int launch_conv_halo_t(const fidm_conv_args& a, cudaStream_t st) {
 
 int launch_conv_halo(const fidm_conv_args& a, cudaStream_t st) {
   if (a.halo_copy) return launch_conv_halo_swap(a, st, nullptr);      // un-normalized operand through the halo path (stem)
-  if (a.dtype != FIDM_E4M3 && conv_halo_swap_preferred(a)) {
-    FIDM_REQUIRE(a.gn_coef && a.ld_gn_coef >= a.cin && (uintptr_t)a.gn_coef % 16 == 0 && a.ld_gn_coef % 2 == 0, FIDM_E_BADARG,
-                 "conv (fused GroupNorm operand): gn_coef must be 16-byte aligned [batch][ld >= cin] float2");
-    return launch_conv_halo_swap(a, st, g_prof);
-  }
+  FIDM_REQUIRE(a.gn_coef && a.ld_gn_coef >= a.cin && (uintptr_t)a.gn_coef % 16 == 0 && a.ld_gn_coef % 2 == 0, FIDM_E_BADARG,
+               "conv (fused GroupNorm operand): gn_coef must be 16-byte aligned [batch][ld >= cin] float2");
+  if (a.dtype != FIDM_E4M3 && conv_halo_swap_preferred(a)) return launch_conv_halo_swap(a, st, g_prof);
   FIDM_REQUIRE(conv_halo_supported(a), FIDM_E_SHAPE,
                "conv (fused GroupNorm operand): needs 3x3 stride 1, H %% 16 == 0, W %% 16 == 0, cin %% 64 == 0, cout %% 128 == 0 "
                "(or the 16-wide fp32-NCHW head); e4m3 operands: cin %% 128 == 0, cout %% 256 == 0, w_scale, no upsampling");
-  FIDM_REQUIRE(a.gn_coef && a.ld_gn_coef >= a.cin && (uintptr_t)a.gn_coef % 16 == 0 && a.ld_gn_coef % 2 == 0, FIDM_E_BADARG,
-               "conv (fused GroupNorm operand): gn_coef must be 16-byte aligned [batch][ld >= cin] float2");
   const bool f16 = a.dtype == FIDM_F16;
   if (a.dtype == FIDM_E4M3) return launch_conv_halo_t<256, 2, false>(a, st);
   if (a.x_half_res) {

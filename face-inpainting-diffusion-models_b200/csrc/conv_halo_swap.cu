@@ -34,6 +34,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "conv_act.cuh"
 #include "conv_host.cuh"
 #include "sm100_primitives.cuh"
 
@@ -84,33 +85,6 @@ static_assert(kRawBytes <= kRawStride, "raw buffer");
 static_assert(kSmemBytes <= 227 * 1024, "shared memory budget");
 static_assert(kRingStages >= 4, "a skip-source slice needs up to 4 stages: alignment skip, two pixel boxes, weights");
 }  // namespace halo_s
-
-__device__ __forceinline__ uint32_t lds_u32x4(uint32_t addr, uint32_t& y, uint32_t& z, uint32_t& w) {
-  uint32_t x;
-  asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(x), "=r"(y), "=r"(z), "=r"(w) : "r"(addr));
-  return x;
-}
-__device__ __forceinline__ void sts_u32x4(uint32_t addr, uint4 v) {
-  asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-// silu(x*A + B) of two packed bf16 values -> two packed 16-bit results; see conv_halo.cu (one MUFU op per value,
-// saturating fp16 convert).
-template <bool OUT_F16>
-__device__ __forceinline__ uint32_t act_pair_s(uint32_t raw, float a0, float b0, float a1, float b1) {
-  const float h0 = fmaf(__uint_as_float(raw << 16), a0, b0);
-  const float h1 = fmaf(__uint_as_float(raw & 0xFFFF0000u), a1, b1);
-  float t0, t1;
-  asm("tanh.approx.f32 %0, %1;" : "=f"(t0) : "f"(h0));
-  asm("tanh.approx.f32 %0, %1;" : "=f"(t1) : "f"(h1));
-  const float y0 = fmaf(h0, t0, h0), y1 = fmaf(h1, t1, h1);
-  uint32_t o;
-  if (OUT_F16) {
-    asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(o) : "f"(y1), "f"(y0));
-  } else {
-    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(o) : "f"(y1), "f"(y0));
-  }
-  return o;
-}
 
 // ACT = false: the operand is x itself (16-bit, already in the weights' dtype) -- the stem convolution, which has no
 // GroupNorm in front of it (unet.py:55) but the same 3x3 structure; the transform is then a plain shifted copy.
@@ -385,12 +359,11 @@ conv_halo_swap_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_co
           for (int i = 0; i < 4; ++i) {
             v[i] = make_uint4(0u, 0u, 0u, 0u);
             if (col_ok && lyq + 3 * i < kUp && (unsigned)(lh + 3 * i) < (unsigned)Hs) {
-              uint32_t r1, r2, r3;
-              const uint32_t r0 = lds_u32x4(ro[i], r1, r2, r3);
-              v[i].x = act_pair_s<OUT_F16>(r0, c[0].x, c[0].y, c[0].z, c[0].w);
-              v[i].y = act_pair_s<OUT_F16>(r1, c[1].x, c[1].y, c[1].z, c[1].w);
-              v[i].z = act_pair_s<OUT_F16>(r2, c[2].x, c[2].y, c[2].z, c[2].w);
-              v[i].w = act_pair_s<OUT_F16>(r3, c[3].x, c[3].y, c[3].z, c[3].w);
+              const uint4 r = ld_shared_u32x4(ro[i]);
+              v[i].x = act_pair<OUT_F16>(r.x, c[0].x, c[0].y, c[0].z, c[0].w);
+              v[i].y = act_pair<OUT_F16>(r.y, c[1].x, c[1].y, c[1].z, c[1].w);
+              v[i].z = act_pair<OUT_F16>(r.z, c[2].x, c[2].y, c[2].z, c[2].w);
+              v[i].w = act_pair<OUT_F16>(r.w, c[3].x, c[3].y, c[3].z, c[3].w);
             }
           }
           PF_ADD(pf_work);
@@ -406,8 +379,8 @@ conv_halo_swap_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_co
                 for (int i = 0; i < 4; ++i) {
                   const int ly = lyq + 3 * i;                         // source row of the box, 0..9
                   if (ly < kUp) {
-                    if (ly >= 1) sts_u32x4(sb[xk][s] - 2048 + i * (6 * 2048), v[i]);     // halo row 2 ly - 1
-                    if (ly <= 8) sts_u32x4(sb[xk][s] + i * (6 * 2048), v[i]);            // halo row 2 ly
+                    if (ly >= 1) st_shared_u32x4(sb[xk][s] - 2048 + i * (6 * 2048), v[i]);     // halo row 2 ly - 1
+                    if (ly <= 8) st_shared_u32x4(sb[xk][s] + i * (6 * 2048), v[i]);            // halo row 2 ly
                   }
                 }
               }
@@ -468,17 +441,16 @@ conv_halo_swap_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_co
 #pragma unroll
         for (int i = 0; i < 9; ++i) {
           const uint32_t sw = (uint32_t)((px0 + i * kHalo) & 7) << 4;
-          uint32_t r1, r2, r3;
-          const uint32_t r0 = lds_u32x4(raw0 + i * (kHalo * 128) + (j16 ^ sw), r1, r2, r3);
+          const uint4 r = ld_shared_u32x4(raw0 + i * (kHalo * 128) + (j16 ^ sw));
           if constexpr (ACT) {
-            v[i].x = act_pair_s<OUT_F16>(r0, c[0].x, c[0].y, c[0].z, c[0].w);
-            v[i].y = act_pair_s<OUT_F16>(r1, c[1].x, c[1].y, c[1].z, c[1].w);
-            v[i].z = act_pair_s<OUT_F16>(r2, c[2].x, c[2].y, c[2].z, c[2].w);
-            v[i].w = act_pair_s<OUT_F16>(r3, c[3].x, c[3].y, c[3].z, c[3].w);
+            v[i].x = act_pair<OUT_F16>(r.x, c[0].x, c[0].y, c[0].z, c[0].w);
+            v[i].y = act_pair<OUT_F16>(r.y, c[1].x, c[1].y, c[1].z, c[1].w);
+            v[i].z = act_pair<OUT_F16>(r.z, c[2].x, c[2].y, c[2].z, c[2].w);
+            v[i].w = act_pair<OUT_F16>(r.w, c[3].x, c[3].y, c[3].z, c[3].w);
             const bool out = (i == 0) ? first_out : (i == 8) ? last_out : col_out;
             if (out) v[i] = make_uint4(0u, 0u, 0u, 0u);
           } else {
-            v[i] = make_uint4(r0, r1, r2, r3);       // out-of-image pixels were zero-filled by the TMA load: that IS the padding
+            v[i] = r;                                // out-of-image pixels were zero-filled by the TMA load: that IS the padding
           }
         }
         PF_ADD(pf_work);
@@ -495,7 +467,7 @@ conv_halo_swap_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_co
           PF_ADD(pf_ae);
           if (in_copy[s]) {
 #pragma unroll
-            for (int i = 0; i < 9; ++i) sts_u32x4(so[s] + i * 2048, v[i]);
+            for (int i = 0; i < 9; ++i) st_shared_u32x4(so[s] + i * 2048, v[i]);
           }
           if (s != 1) {
             fence_proxy_async_smem();
@@ -658,13 +630,10 @@ static int launch_conv_halo_swap_t(const fidm_conv_args& a, cudaStream_t st, uns
   p.kc1 = a.cin / 64; p.cin1 = a.cin;
   p.kc2 = a.x2 ? a.cin2 / 64 : 0;
   p.coef = reinterpret_cast<const float2*>(a.gn_coef); p.ld_coef = a.ld_gn_coef;
-  p.bias = a.bias; p.row_add = a.row_add; p.ld_row_add = a.ld_row_add;
-  p.residual = kHead ? nullptr : reinterpret_cast<const unsigned short*>(a.residual); p.ld_res = a.ld_res;
+  set_epilogue_params(p, a);                             // (the head variant is only supported without a residual)
   p.res_half = a.residual_half_res;
   p.y = reinterpret_cast<unsigned short*>(a.y); p.ld_y = a.ld_y;
-  p.colsum = a.colsum; p.cout = a.cout;
   p.colsum_slots = p.tiles_w * p.tiles_h * 4;            // == fidm_conv_colsum_slots(H, W): one slot per 64 pixels
-  p.y_nchw = a.y_nchw_f32 ? reinterpret_cast<float*>(a.y) : nullptr; p.cout_valid = a.cout_valid;
   p.prof = PROF ? prof : nullptr;
 
   CUtensorMap tmRaw, tmW, tmX2, tmW2;

@@ -31,6 +31,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "conv_epilogue.cuh"
 #include "conv_host.cuh"
 #include "sm100_primitives.cuh"
 
@@ -160,25 +161,8 @@ __device__ __forceinline__ void cluster_fold_store(const ConvTcParams& p, const 
     for (int q = 0; q < 4; ++q) {
 #pragma unroll
       for (int j = 0; j < 8; ++j) f[q][j] += add[j];
-      if (p.residual) {
-        const uint4 t = __ldg(reinterpret_cast<const uint4*>(p.residual + (pix + q) * p.ld_res + c));
-        const uint32_t u[4] = {t.x, t.y, t.z, t.w};
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          f[q][2 * k] += __uint_as_float(u[k] << 16);
-          f[q][2 * k + 1] += __uint_as_float(u[k] & 0xFFFF0000u);
-        }
-      }
-      uint4 pk;
-      __nv_bfloat162 b0 = __floats2bfloat162_rn(f[q][0], f[q][1]);
-      __nv_bfloat162 b1 = __floats2bfloat162_rn(f[q][2], f[q][3]);
-      __nv_bfloat162 b2 = __floats2bfloat162_rn(f[q][4], f[q][5]);
-      __nv_bfloat162 b3 = __floats2bfloat162_rn(f[q][6], f[q][7]);
-      pk.x = *reinterpret_cast<uint32_t*>(&b0);
-      pk.y = *reinterpret_cast<uint32_t*>(&b1);
-      pk.z = *reinterpret_cast<uint32_t*>(&b2);
-      pk.w = *reinterpret_cast<uint32_t*>(&b3);
-      *reinterpret_cast<uint4*>(p.y_out + (pix + q) * p.ld_y + c) = pk;
+      if (p.residual) epi::add_bf16x8(f[q], __ldg(reinterpret_cast<const uint4*>(p.residual + (pix + q) * p.ld_res + c)));
+      *reinterpret_cast<uint4*>(p.y_out + (pix + q) * p.ld_y + c) = epi::pack_bf16x8(f[q]);
     }
   }
 }
@@ -484,35 +468,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
           for (int j = 0; j < 32; ++j) { f[j] = __uint_as_float(v0[j]); f[32 + j] = __uint_as_float(v1[j]); }
           }
-          if (p.bias) {
-            const float4* b4 = reinterpret_cast<const float4*>(p.bias + cbase);
-#pragma unroll
-            for (int j = 0; j < 16; ++j) {
-              const float4 t = __ldg(b4 + j);
-              f[4 * j] += t.x; f[4 * j + 1] += t.y; f[4 * j + 2] += t.z; f[4 * j + 3] += t.w;
-            }
-          }
-          if (p.row_add && valid) {
-            const float4* r4 = reinterpret_cast<const float4*>(p.row_add + (long long)n * p.ld_row_add + cbase);
-#pragma unroll
-            for (int j = 0; j < 16; ++j) {
-              const float4 t = __ldg(r4 + j);
-              f[4 * j] += t.x; f[4 * j + 1] += t.y; f[4 * j + 2] += t.z; f[4 * j + 3] += t.w;
-            }
-          }
-          if (p.residual && valid) {
-            const uint4* r = reinterpret_cast<const uint4*>(p.residual + pix * p.ld_res + cbase);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              const uint4 t = __ldg(r + j);
-              const uint32_t u[4] = {t.x, t.y, t.z, t.w};
-#pragma unroll
-              for (int q = 0; q < 4; ++q) {
-                f[8 * j + 2 * q] += __uint_as_float(u[q] << 16);
-                f[8 * j + 2 * q + 1] += __uint_as_float(u[q] & 0xFFFF0000u);
-              }
-            }
-          }
+          if (p.bias) epi::add_f32_row(f, p.bias + cbase);
+          if (p.row_add && valid) epi::add_f32_row(f, p.row_add + (long long)n * p.ld_row_add + cbase);
+          if (p.residual && valid) epi::add_bf16_row(f, p.residual + pix * p.ld_res + cbase);
           if (p.y_nchw) {
             if (valid) {
               const long long hw = (long long)p.H * p.W;
@@ -525,20 +483,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             // this warpgroup's staging tile was last read by the TMA store of its previous chunk
             if (issuer) bulk_wait_group_read<0>();
             named_bar_sync(bar_a, 128);
-            uint8_t* srow = stage_out + row * 128;
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-              uint4 pk;
-              __nv_bfloat162 b0 = __floats2bfloat162_rn(f[8 * u + 0], f[8 * u + 1]);
-              __nv_bfloat162 b1 = __floats2bfloat162_rn(f[8 * u + 2], f[8 * u + 3]);
-              __nv_bfloat162 b2 = __floats2bfloat162_rn(f[8 * u + 4], f[8 * u + 5]);
-              __nv_bfloat162 b3 = __floats2bfloat162_rn(f[8 * u + 6], f[8 * u + 7]);
-              pk.x = *reinterpret_cast<uint32_t*>(&b0);
-              pk.y = *reinterpret_cast<uint32_t*>(&b1);
-              pk.z = *reinterpret_cast<uint32_t*>(&b2);
-              pk.w = *reinterpret_cast<uint32_t*>(&b3);
-              *reinterpret_cast<uint4*>(srow + ((u ^ (row & 7)) << 4)) = pk;   // 128-byte swizzle
-            }
+            epi::stage_bf16_row(stage_out + row * 128, row, f);
             fence_proxy_async_smem();
             named_bar_sync(bar_b, 128);
             if (issuer) {
@@ -547,28 +492,16 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               if (threadIdx.x == 0) TL1(10);
             }
             if (p.colsum) {
-              // Fused GroupNorm statistics: per-channel (sum, sum of squares) of the bf16 tile just staged.
-              // Thread = (column, half of the rows); a warp reads 32 consecutive channels of one row
-              // (conflict-free under the 128-byte swizzle).  Rows 0-63 / 64-127 are separate partial rows
-              // (with TN == 2 they are two different images).
+              // Fused GroupNorm statistics of the bf16 tile just staged.  Rows 0-63 / 64-127 are separate partial
+              // rows (with TN == 2 they are two different images).
               const int col = etid & 63, half = etid >> 6;
-              const uint32_t sb0 = smem_u32(stage_out) + (col & 7) * 2;
-              const int unit = col >> 3;
-              float s1 = 0.0f, s2 = 0.0f;
-#pragma unroll 8
-              for (int r = half * 64; r < half * 64 + 64; ++r) {
-                uint32_t raw;
-                asm volatile("ld.shared.u16 %0, [%1];" : "=r"(raw) : "r"(sb0 + r * 128 + ((unit ^ (r & 7)) << 4)));
-                const float v = __uint_as_float(raw << 16);
-                s1 += v;
-                s2 = fmaf(v, v, s2);
-              }
+              const float2 st = epi::staged_col_stats(smem_u32(stage_out), col, half);
               const int img = n0 + (p.TN == 2 ? half : 0);
               if (img < p.B && m_blk < m_tiles) {
                 const int slot = (p.TN == 1) ? ((m_blk % (p.tiles_w * p.tiles_h)) * 2 + half) : 0;
                 float2* dst = reinterpret_cast<float2*>(p.colsum) +
                               ((long long)img * p.colsum_slots + slot) * p.cout + cbase + col;
-                *dst = make_float2(s1, s2);
+                *dst = st;
               }
             }
           }
@@ -582,20 +515,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&tmem_empty[acc]);
-        if (valid && p.y_nchw && wg == 0) {
-          const long long hw = (long long)p.H * p.W;
-          float* o = p.y_nchw + ((long long)n * p.cout_valid) * hw + (long long)h * p.W + w;
-#pragma unroll
-          for (int j = 0; j < 16; ++j) {
-            const int c = co0 + j;
-            if (c < p.cout_valid) {
-              float val = __uint_as_float(v[j]);
-              if (p.bias) val += __ldg(p.bias + c);
-              if (p.row_add) val += __ldg(p.row_add + (long long)n * p.ld_row_add + c);
-              o[(long long)c * hw] = val;
-            }
-          }
-        }
+        if (valid && p.y_nchw && wg == 0) epi::store_head16(p, v, co0, n, h, w);
       }
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
     }
@@ -752,11 +672,7 @@ static int launch_conv_tc(const fidm_conv_args& a, cudaStream_t st, int split_k 
   p.kc2 = a.x2 ? a.cin2 / 64 : 0;
   p.ab_f16 = a.dtype == FIDM_F16;
   const int f16 = p.ab_f16;
-  p.bias = a.bias; p.row_add = a.row_add; p.ld_row_add = a.ld_row_add;
-  p.residual = reinterpret_cast<const __nv_bfloat16*>(a.residual); p.ld_res = a.ld_res;
-  p.y_nchw = a.y_nchw_f32 ? reinterpret_cast<float*>(a.y) : nullptr;
-  p.cout_valid = a.cout_valid;
-  p.colsum = a.colsum; p.cout = a.cout;
+  set_epilogue_params(p, a);
   p.colsum_slots = (p.TN == 1) ? p.tiles_w * p.tiles_h * 2 : 1;
   p.y_out = reinterpret_cast<__nv_bfloat16*>(a.y); p.ld_y = a.ld_y;
   p.tw_sh = log2_exact(p.TW); p.th_sh = log2_exact(p.TH);

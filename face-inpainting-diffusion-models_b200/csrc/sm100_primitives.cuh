@@ -92,6 +92,24 @@ __device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t threads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
 }
 
+// ----------------------------------------------------------------------------- shared-memory vector access
+__device__ __forceinline__ uint4 ld_shared_u32x4(uint32_t addr) {
+  uint4 v;
+  asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
+  return v;
+}
+__device__ __forceinline__ uint32_t ld_shared_u16(uint32_t addr) {
+  uint32_t v;
+  asm volatile("ld.shared.u16 %0, [%1];" : "=r"(v) : "r"(addr));
+  return v;
+}
+__device__ __forceinline__ void st_shared_u32x4(uint32_t addr, uint4 v) {
+  asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+}
+__device__ __forceinline__ void st_shared_u32x2(uint32_t addr, uint32_t x, uint32_t y) {
+  asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(addr), "r"(x), "r"(y) : "memory");
+}
+
 // ----------------------------------------------------------------------------- tcgen05
 __device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t cols) {  // whole warp
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(cols)
