@@ -92,6 +92,21 @@ def class_draw_order(T, inject=True, schedule="all", first=True):
     return seq
 
 
+def attention_shapes(cfg):
+    """{(tokens, heads, head_dim)} of the attention layers of the UNet built from the constructor arguments `cfg`,
+    each at the resolution the forward pass reaches it (arch.all_layers is in execution order)."""
+    from fidm_b200.arch import all_layers, unet_topology
+    res, shapes = cfg["image_size"], set()
+    for layer in all_layers(unet_topology(**cfg)):
+        if layer.kind == "attn":
+            shapes.add((res * res, layer.heads, layer.channels // layer.heads))
+        elif layer.kind == "down" or getattr(layer, "down", False):
+            res //= 2
+        elif layer.kind == "up" or getattr(layer, "up", False):
+            res *= 2
+    return shapes
+
+
 def hole_psnr(a, b, keep):
     """PSNR over the inpainted (hole) pixels only: the known region is bit-exact by construction and would flatter
     a whole-image figure."""
