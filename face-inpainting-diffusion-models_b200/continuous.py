@@ -17,6 +17,10 @@ An iteration is [admissions] -> model evaluation -> one launch of the per-slot s
 parameters, so the schedule lives on the host (SlotSchedule, pure Python) and no iteration copies control data to the
 device or synchronises.  With this package's InpaintingModelFn the evaluation is a CUDA-graph replay of the engine plan
 whose state channels and timesteps K8 writes, and an iteration without admissions is [graph replay, K8].
+
+diffusion.continuous_dpm_solver_sampler(...) has the same surface for dpm_solver_sample_loop: every request takes
+`steps` evaluations on the DPM-Solver++ grid, each slot keeps its own history m_{k-1}, and the per-slot step is K9
+(fidm_multistep_step_slots); each result equals dpm_solver_sample_loop run alone with seeds=[seed].
 """
 import collections
 import ctypes as C
@@ -26,25 +30,37 @@ from typing import NamedTuple
 import torch
 
 from . import _lib as L
-from . import seeded
+from . import dpm_solver, seeded
 
 
-def injection_draws(diffusion, schedule, cumulative, inject=True):
-    """Per timestep t, the draw of the injection noise a seeded loop uses at t (ddim_sample_loop / p_sample_loop): t for
-    cumulative noise, for fresh noise the number of injections at timesteps above t; -1 where the loop does not
-    inject (no injection, or t gated by `schedule`)."""
-    T = diffusion.num_timesteps
-    draws, fresh = [-1] * T, 0
-    for t in range(T - 1, -1, -1):
+def injection_draws(diffusion, schedule, cumulative, inject=True, grid=None):
+    """The draw of the injection noise a seeded loop uses at each timestep it visits: t for cumulative noise, for fresh
+    noise the number of injections before it; -1 where the loop does not inject (no injection, or t gated by
+    `schedule`).  Without `grid`: indexed by t, the visits of ddim_sample_loop / p_sample_loop (T-1 .. 0).  With the
+    DPM-Solver++ grid (dpm_solver.timestep_grid): indexed by grid point k, the visits of dpm_solver_sample_loop (x_T's
+    injection at grid[0] counts as the first)."""
+    ts = range(diffusion.num_timesteps - 1, -1, -1) if grid is None else [int(t) for t in grid]
+    draws, fresh = [], 0
+    for t in ts:
         if inject and not diffusion._injection_gated(t, schedule):
-            draws[t] = t if cumulative else fresh
+            draws.append(t if cumulative else fresh)
             fresh += 1
-    return draws
+        else:
+            draws.append(-1)
+    return draws[::-1] if grid is None else draws
+
+
+def dpm_slot_tables(diffusion, grid, order, schedule, cumulative, inject=True):
+    """K9's per-grid-point tables (fidm_ms_slot_args) as lists: the timestep value the model sees at t_k, the draw of
+    the injection at t_k, and the order of the update out of t_k (dpm_solver.step_orders; 1 at the last point)."""
+    return ([diffusion._t_value(int(t)) for t in grid], injection_draws(diffusion, schedule, cumulative, inject, grid),
+            dpm_solver.step_orders(len(grid), order) + [1])
 
 
 class SlotSchedule:
     """Which slot does what in each iteration.  FIFO admission into the lowest free slot; a slot evaluates its request
-    at t = T-1 in the iteration it is admitted and at t - 1 in each following one, and is free again after t = 0."""
+    at t = T-1 in the iteration it is admitted and at t - 1 in each following one, and is free again after t = 0.
+    (For DPM-Solver++ slots T is the number of evaluations and t counts them down: grid point k = T-1-t.)"""
 
     def __init__(self, slots, num_timesteps):
         self.T = num_timesteps
@@ -101,7 +117,35 @@ class ContinuousSampler:
         if denoised_fn is not None or cond_fn is not None:
             raise ValueError("continuous batching runs the fused sampler step: denoised_fn / cond_fn are not supported")
         if sampler not in ("ddim", "ddpm"):
-            raise ValueError(f"sampler must be 'ddim' or 'ddpm', got {sampler!r}")
+            hint = " (DPM-Solver++: diffusion.continuous_dpm_solver_sampler)" if sampler == "dpm_solver" else ""
+            raise ValueError(f"sampler must be 'ddim' or 'ddpm', got {sampler!r}{hint}")
+        T = diffusion.num_timesteps
+        self._setup(diffusion, model, slots, image_size, injection_schedule, channels, device, T)
+        ddim = sampler == "ddim"
+        self._t_of = self._action_of = list(range(T))     # the schedule counts timesteps
+        self._coef = diffusion._coef(self.device, eta if ddim else 0.0)
+        self._t_value = torch.tensor([diffusion._t_value(t) for t in range(T)], dtype=torch.float32, device=self.device)
+        self._inject_draw = torch.tensor(injection_draws(diffusion, injection_schedule, use_cumulative_noise,
+                                                         use_inpainting_injection), dtype=torch.int32, device=self.device)
+
+        from .gaussian_diffusion import _MEAN_CODE, _VAR_CODE
+        a = self._args = L.StepArgs()
+        a.batch, a.channels, a.hw = slots, channels, self.H * self.W
+        a.mode = L.STEP_UPDATE_INJECT
+        a.sampler = L.SAMPLER_DDIM if ddim else L.SAMPLER_DDPM
+        a.mean_type, a.var_type = _MEAN_CODE[diffusion.model_mean_type], _VAR_CODE[diffusion.model_var_type]
+        a.clip_denoised, a.cumulative = int(bool(clip_denoised)), int(bool(use_cumulative_noise))
+        a.mask_channels, a.num_timesteps = channels, T
+        a.coef, a.x, a.x_next, a.gt, a.keep_mask = (L.ptr(v) for v in (self._coef, self.x, self.x, self.gt, self.keep))
+        self._set_stem(a)
+        s = self._slot_args = L.SlotArgs()
+        s.t_value, s.inject_draw, s.out = L.ptr(self._t_value), L.ptr(self._inject_draw), L.ptr(self.out)
+        s.step_noise = int(not ddim or eta != 0.0)
+        self._entry = "fidm_sampler_step_slots"
+
+    def _setup(self, diffusion, model, slots, image_size, injection_schedule, channels, device, evaluations):
+        """What every solver's sampler shares: the argument checks (before any device work), the slot buffers, the
+        schedule of `evaluations` per request, the engine plan and the model's output channels."""
         if isinstance(slots, bool) or not isinstance(slots, int) or not 1 <= slots <= L.MAX_SLOTS:
             raise ValueError(f"slots must be an int in [1, {L.MAX_SLOTS}], got {slots!r}")
         if injection_schedule not in ("all", "high", "low"):
@@ -117,47 +161,32 @@ class ContinuousSampler:
                               "(no CPU fallback exists)")
         self.diffusion, self.model, self.device = diffusion, model, device
         self.B, self.C, (self.H, self.W) = slots, channels, image_size
-        ddim = sampler == "ddim"
-        T = diffusion.num_timesteps
-        self.schedule = SlotSchedule(slots, T)
+        self.schedule = SlotSchedule(slots, evaluations)
         self._requests = {}
         self._next_ticket = 0
 
         shape = (slots, channels) + tuple(image_size)
-        self.x = torch.zeros(shape, device=device)                 # slot states, updated in place by K8
+        self.x = torch.zeros(shape, device=device)                 # slot states, updated in place by the step kernel
         self.gt = torch.zeros(shape, device=device)
         self.keep = torch.zeros(shape, device=device)
-        self.out = torch.zeros(shape, device=device)               # K8 writes a finished sample here
-        self._coef = diffusion._coef(device, eta if ddim else 0.0)
-        self._t_value = torch.tensor([diffusion._t_value(t) for t in range(T)], dtype=torch.float32, device=device)
-        self._inject_draw = torch.tensor(injection_draws(diffusion, injection_schedule, use_cumulative_noise,
-                                                         use_inpainting_injection), dtype=torch.int32, device=device)
+        self.out = torch.zeros(shape, device=device)               # the step kernel writes a finished sample here
 
         self.plan = None
         if getattr(model, "fused_plan", None) is not None and os.environ.get("FIDM_FUSED_STEP", "1") != "0":
             slot_plan = getattr(model, "slot_plan", None)
             self.plan = slot_plan(slots, channels, *image_size) if slot_plan is not None else None
+        from .gaussian_diffusion import _VAR_CODE
+        self._out_channels = channels if _VAR_CODE[diffusion.model_var_type] == L.VAR_FIXED else 2 * channels
+        if self.plan is not None and self.plan.out.shape[1] != self._out_channels:
+            raise ValueError(f"the model has {self.plan.out.shape[1]} output channels, the diffusion's variance type "
+                             f"needs {self._out_channels}")
 
-        from .gaussian_diffusion import _MEAN_CODE, _VAR_CODE
-        a = self._args = L.StepArgs()
-        a.batch, a.channels, a.hw = slots, channels, self.H * self.W
-        a.mode = L.STEP_UPDATE_INJECT
-        a.sampler = L.SAMPLER_DDIM if ddim else L.SAMPLER_DDPM
-        a.mean_type, a.var_type = _MEAN_CODE[diffusion.model_mean_type], _VAR_CODE[diffusion.model_var_type]
-        a.clip_denoised, a.cumulative = int(bool(clip_denoised)), int(bool(use_cumulative_noise))
-        a.mask_channels, a.num_timesteps = channels, T
-        a.coef, a.x, a.x_next, a.gt, a.keep_mask = (L.ptr(v) for v in (self._coef, self.x, self.x, self.gt, self.keep))
+    def _set_stem(self, a):
+        """With the engine plan the step kernel writes the next evaluation's state channels and timesteps into it."""
         if self.plan is not None:
             a.stem_out, a.stem_dtype, a.stem_ld = (L.ptr(self.plan.x_in), L.dtype_code(self.plan.x_in.dtype),
                                                    self.plan.x_in.shape[-1])
             a.t_out = L.ptr(self.plan.t_in)
-        self._out_channels = channels if a.var_type == L.VAR_FIXED else 2 * channels
-        if self.plan is not None and self.plan.out.shape[1] != self._out_channels:
-            raise ValueError(f"the model has {self.plan.out.shape[1]} output channels, the diffusion's variance type "
-                             f"needs {self._out_channels}")
-        s = self._slot_args = L.SlotArgs()
-        s.t_value, s.inject_draw, s.out = L.ptr(self._t_value), L.ptr(self._inject_draw), L.ptr(self.out)
-        s.step_noise = int(not ddim or eta != 0.0)
 
     # ------------------------------------------------------------------ requests
     def submit(self, gt, gt_keep_mask, seed):
@@ -193,7 +222,7 @@ class ContinuousSampler:
 
     # ------------------------------------------------------------------ iterations
     def step(self):
-        """One iteration: admit queued requests into free slots, evaluate every busy slot once, take one K8 step.
+        """One iteration: admit queued requests into free slots, evaluate every busy slot once, take one K8 (K9) step.
         Returns [(ticket, image [1, C, H, W])] for the requests that finished; each image is a copy enqueued on the
         current stream, ready once the stream reaches it (the caller synchronises when it reads it)."""
         admitted = self.schedule.admit()
@@ -206,7 +235,7 @@ class ContinuousSampler:
             if all(t is None for t in ts):
                 return []
             model_out = self._evaluate(ts)
-            self._launch({b: t for b, t in enumerate(ts) if t is not None}, model_out)
+            self._launch({b: self._action_of[t] for b, t in enumerate(ts) if t is not None}, model_out)
             done = []
             for b, ticket in self.schedule.advance():
                 del self._requests[ticket]
@@ -222,7 +251,7 @@ class ContinuousSampler:
 
     def _load(self, b, req):
         """Admission of `req` into slot b: its known region and seed, and with the engine plan its conditioning
-        channels (K8's admit action writes the state channels and the timestep)."""
+        channels (the step kernel's admit action writes the state channels and the timestep)."""
         self.gt[b].copy_(req.gt[0])
         self.keep[b].copy_(req.keep[0].expand(self.C, self.H, self.W))
         self._slot_args.seeds[b] = req.seed
@@ -232,7 +261,8 @@ class ContinuousSampler:
     def _evaluate(self, ts):
         if self.plan is not None:
             return self.plan.run()                   # state channels and timesteps are already in place
-        t = torch.tensor([0 if v is None else v for v in ts], dtype=torch.long).to(self.device, non_blocking=True)
+        t = torch.tensor([0 if v is None else self._t_of[v] for v in ts], dtype=torch.long).to(self.device,
+                                                                                                non_blocking=True)
         out = self.diffusion._call_model(self.model, self.x, t, {"gt": self.gt, "gt_keep_mask": self.keep})
         out = out.detach()
         if out.dtype != torch.float32 or not out.is_contiguous():
@@ -243,9 +273,52 @@ class ContinuousSampler:
         return out
 
     def _launch(self, actions, model_out):
-        """One K8 launch: slot b takes actions[b] (SLOT_ADMIT or the timestep of its update), every other slot idles."""
+        """One launch of the step kernel: slot b takes actions[b] (SLOT_ADMIT or its grid point: the timestep of a K8
+        update, the k of a K9 one), every other slot idles."""
         s = self._slot_args
         for b in range(self.B):
             s.action[b] = actions.get(b, L.SLOT_IDLE)
         self._args.model_out = L.ptr(model_out)
-        L.check(L.lib().fidm_sampler_step_slots(C.byref(self._args), C.byref(s), L.stream()), "sampler_step_slots")
+        L.check(getattr(L.lib(), self._entry)(C.byref(self._args), C.byref(s), L.stream()), self._entry[5:])
+
+
+class ContinuousDPMSolverSampler(ContinuousSampler):
+    """ContinuousSampler for dpm_solver_sample_loop (built by GaussianDiffusion.continuous_dpm_solver_sampler): every
+    request takes `steps` evaluations on dpm_solver.timestep_grid, each slot keeps its history m_{k-1} in `self.m`,
+    and the per-slot step is K9 (fidm_multistep_step_slots) on K6's coefficient table."""
+
+    def __init__(self, diffusion, model, slots=8, image_size=(256, 256), steps=20, order=2, clip_denoised=True,
+                 use_inpainting_injection=True, injection_schedule="all", use_cumulative_noise=True, channels=3,
+                 device=None):
+        from .gaussian_diffusion import _MEAN_CODE, ModelMeanType
+        grid = dpm_solver.timestep_grid(diffusion.num_timesteps, steps)
+        tables = dpm_slot_tables(diffusion, grid, order, injection_schedule, use_cumulative_noise,
+                                 use_inpainting_injection)
+        if diffusion.model_mean_type == ModelMeanType.PREVIOUS_X:
+            raise NotImplementedError("DPM-Solver++ needs an eps or x0 prediction; PREVIOUS_X models are not supported")
+        self._setup(diffusion, model, slots, image_size, injection_schedule, channels, device, steps)
+        # the schedule's counter c runs steps-1 .. 0: grid point k = steps-1-c
+        self._t_of = [int(t) for t in grid[::-1]]
+        self._action_of = list(range(steps - 1, -1, -1))
+        dev = self.device
+        self.m = torch.zeros_like(self.x)                          # per-slot history m_{k-1}, updated in place by K9
+        self._coef = diffusion._dpm_table(dev, steps, order, use_cumulative_noise)
+        self._t_value, self._inject_draw, self._order = (torch.tensor(v, dtype=dt, device=dev) for v, dt in
+                                                         zip(tables, (torch.float32, torch.int32, torch.int32)))
+
+        a = self._args = L.MultistepArgs()
+        a.batch, a.channels, a.hw = slots, channels, self.H * self.W
+        a.mean_type, a.out_channels = _MEAN_CODE[diffusion.model_mean_type], self._out_channels
+        a.clip_denoised, a.mask_channels, a.steps = int(bool(clip_denoised)), channels, steps
+        a.coef, a.x, a.x_next, a.m_prev, a.m_out, a.gt, a.keep_mask = (
+            L.ptr(v) for v in (self._coef, self.x, self.x, self.m, self.m, self.gt, self.keep))
+        self._set_stem(a)
+        s = self._slot_args = L.MsSlotArgs()
+        s.t_value, s.inject_draw, s.order, s.out = (L.ptr(v) for v in (self._t_value, self._inject_draw, self._order,
+                                                                        self.out))
+        s.inject_tag = L.NOISE_INJECT if use_cumulative_noise else L.NOISE_INJECT_FRESH
+        # x_T's injection at t_0 = T-1 is the lockstep loop's K4 STEP_INJECT_ONLY: the K4 table's coefficients
+        cls = diffusion.coefficient_table(0.0)
+        ia, is_ = (L.C_SQRT_AB, L.C_SQRT_1MAB) if use_cumulative_noise else (L.C_SQRT_AB_F32, L.C_SQRT_1MAB_F32)
+        s.admit_inject_a, s.admit_inject_s = float(cls[int(grid[0]), ia]), float(cls[int(grid[0]), is_])
+        self._entry = "fidm_multistep_step_slots"

@@ -811,7 +811,7 @@ class GaussianDiffusion:
         return self._last_sample(self._repaint_loop(evals, model, shape, noise, clip_denoised, model_kwargs, device,
                                                     progress, injection_schedule, use_cumulative_noise, False, seeds))
 
-    # ------------------------------------------------------------------ continuous batching (K8)
+    # ------------------------------------------------------------------ continuous batching (K8, K9)
     def continuous_sampler(self, model, slots=8, image_size=(256, 256), sampler="ddim", eta=0.0, clip_denoised=True,
                            use_inpainting_injection=True, injection_schedule="all", use_cumulative_noise=True,
                            channels=3, device=None, denoised_fn=None, cond_fn=None):
@@ -824,6 +824,19 @@ class GaussianDiffusion:
                                  clip_denoised=clip_denoised, use_inpainting_injection=use_inpainting_injection,
                                  injection_schedule=injection_schedule, use_cumulative_noise=use_cumulative_noise,
                                  channels=channels, device=device, denoised_fn=denoised_fn, cond_fn=cond_fn)
+
+    def continuous_dpm_solver_sampler(self, model, slots=8, image_size=(256, 256), steps=20, order=2, clip_denoised=True,
+                                      use_inpainting_injection=True, injection_schedule="all",
+                                      use_cumulative_noise=True, channels=3, device=None):
+        """continuous_sampler for DPM-Solver++: every request takes `steps` model evaluations (multistep `order` 1 or
+        2), its result bit-identical to dpm_solver_sample_loop(model, (1, C, H, W), steps=steps, order=order, ...,
+        seeds=[seed]) run alone.  Same submit / step / pending / drain surface; arguments are checked here and at
+        submit, before any launch."""
+        from .continuous import ContinuousDPMSolverSampler
+        return ContinuousDPMSolverSampler(self, model, slots=slots, image_size=image_size, steps=steps, order=order,
+                                          clip_denoised=clip_denoised, use_inpainting_injection=use_inpainting_injection,
+                                          injection_schedule=injection_schedule,
+                                          use_cumulative_noise=use_cumulative_noise, channels=channels, device=device)
 
     def sample_with_advanced_inpainting(self, model, shape, gt=None, gt_keep_mask=None, use_ddim=True, eta=0.0,
                                         progress=True, device=None, injection_schedule="all",

@@ -250,6 +250,39 @@ typedef struct fidm_slot_args {
 int fidm_sampler_step_slots(const fidm_step_args* a, const fidm_slot_args* s, fidm_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * K9  per-slot DPM-Solver++ multistep step (continuous batching of dpm_solver_sample_loop): K6 as K8 is K4.  Each slot
+ * runs its own seeded request on the grid t_0 = T-1 > ... > t_{steps-1} = 0 of `a->coef` (K6's table); one launch takes,
+ * per slot, the action in s->action:
+ *   FIDM_SLOT_IDLE   nothing is read or written for the slot (state, history, stem, t_out, out);
+ *   FIDM_SLOT_ADMIT  x_T = draw (XT, 0) under the slot's seed, then the injection at t_0 (K4's expression with
+ *                    s->admit_inject_a / s->admit_inject_s) unless inject_draw[0] < 0, written as the state, the stem
+ *                    channels and t_out[b] = t_value[0] -- the seeded loop's prologue;
+ *   k in [0, steps)  K6's row k for the slot: m_k from x and model_out; at k = steps-1 m_k goes to out[b] and nothing
+ *                    else is written; otherwise m_k goes to m_out, x' = A*x + B0*m_k [+ B1*m_{k-1}, read from m_prev
+ *                    only where order[k] == 2], the injection at t_{k+1} with draw (inject_tag, inject_draw[k+1])
+ *                    unless that is < 0, and the state, stem and t_out[b] = t_value[k+1] are written.
+ * Every value is bit-identical to what fidm_multistep_step_seeded computes for that image alone (and, for an admission,
+ * fidm_randn_seeded followed by fidm_sampler_step_seeded's STEP_INJECT_ONLY at T-1).
+ * Fields of `a` used: the shape (batch = number of slots, at most FIDM_MAX_SLOTS), mean_type, out_channels,
+ * clip_denoised, mask_channels, steps, coef, x, model_out (read for updates), m_prev, m_out, x_next, gt, keep_mask,
+ * stem_out / stem_dtype / stem_ld and t_out; step, inject and t_out_value are ignored and inject_noise must be NULL.
+ * x_next may equal x and m_out may equal m_prev (each element is read and written by the same thread).  As for K8 the
+ * per-slot control travels by value in the launch parameters.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct fidm_ms_slot_args {
+  const float* t_value;                 /* device [steps]: what the model sees at grid point k (_scale_timesteps of t_k) */
+  const int32_t* inject_draw;           /* device [steps]: draw of the injection at t_k; -1: no injection at t_k */
+  const int32_t* order;                 /* device [steps]: 2 where the update out of t_k uses m_{k-1}, else 1 */
+  float* out;                           /* [batch][channels][hw]: m_k of a slot at its last grid point */
+  int32_t inject_tag;                   /* FIDM_NOISE_INJECT | FIDM_NOISE_INJECT_FRESH */
+  float admit_inject_a, admit_inject_s; /* injection coefficients at t_0 = T-1: the K4 table's (FIDM_C_SQRT_AB,
+                                           FIDM_C_SQRT_1MAB) for cumulative noise, the _F32 columns otherwise */
+  int32_t action[FIDM_MAX_SLOTS];       /* per slot: FIDM_SLOT_IDLE | FIDM_SLOT_ADMIT | k (the grid point evaluated) */
+  uint64_t seeds[FIDM_MAX_SLOTS];       /* per slot: the request's seed */
+} fidm_ms_slot_args;
+int fidm_multistep_step_slots(const fidm_multistep_args* a, const fidm_ms_slot_args* s, fidm_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Layout converters.  Replace torch.cat([x, masked_image, mask.repeat(1,3,1,1)], 1) of
  * unet.py:199 and the NCHW activations of the reference with one NHWC (bf16|fp32) tensor padded to
  * `c_pad` channels (zeros).  Up to 3 fp32 NCHW sources; a source with repeat>1 is broadcast.

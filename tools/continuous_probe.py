@@ -13,7 +13,12 @@ that batch), which is the host and sampler-step overhead.  Then K8 (all slots up
 against the seeded K4 at batch 8 and 64, each in a CUDA graph of 20 launches, beside a 2 GiB device-to-device copy.
 The card's name, power limit and clocks are read (not set) in the same call.
 
-    python tools/continuous_probe.py [--rounds 3] [--load 0.8]
+With --sampler dpm_solver the four arms run DPM-Solver++ 2M in --steps evaluations on the 1000-step quadratic diffusion
+(as tools/dpm_solver_probe.py; (a) and (b) through dpm_solver_sample_loop, (c) and (d) through
+continuous_dpm_solver_sampler), and the step timing is K9 (all slots updating at a second-order grid point, injection,
+bf16 stem) against the seeded K6 on the same batch; its checks add the contract on the elementwise stand-in model.
+
+    python tools/continuous_probe.py [--rounds 3] [--load 0.8] [--sampler ddim | dpm_solver] [--steps 20]
 """
 import argparse
 import ctypes
@@ -33,6 +38,31 @@ sys.path.insert(0, os.path.join(ROOT, "tools"))
 from repaint_probe import copy_gbs, event_ms, gpu_info  # noqa: E402
 
 B, S, T, N = 8, 256, 50, 64
+
+
+class Workload:
+    """The sampler the arms run: DDIM-50 on the 50-step cosine diffusion (default), or DPM-Solver++ 2M in `steps`
+    evaluations on the 1000-step quadratic one.  evals: model evaluations per request."""
+
+    def __init__(self, F, sampler, steps):
+        self.dpm, self.steps = sampler == "dpm_solver", steps
+        if self.dpm:
+            self.d = F.create_gaussian_diffusion(steps=1000, learn_sigma=True, noise_schedule="quadratic")
+        else:
+            self.d = F.create_gaussian_diffusion(steps=T, learn_sigma=True, noise_schedule="cosine")
+        self.evals = steps if self.dpm else T
+
+    def loop(self, fn, gt, keep, seeds):
+        kw = dict(model_kwargs={"gt": gt, "gt_keep_mask": keep}, device=gt.device, use_inpainting_injection=True,
+                  seeds=seeds)
+        if self.dpm:
+            return self.d.dpm_solver_sample_loop(fn, tuple(gt.shape), steps=self.steps, **kw)
+        return self.d.ddim_sample_loop(fn, tuple(gt.shape), **kw)
+
+    def continuous(self, fn):
+        if self.dpm:
+            return self.d.continuous_dpm_solver_sampler(fn, slots=B, image_size=(S, S), steps=self.steps)
+        return self.d.continuous_sampler(fn, slots=B, image_size=(S, S), sampler="ddim")
 
 
 def _pct(v, q):
@@ -58,31 +88,49 @@ class _Clock:
         return self.e0.elapsed_time(e)
 
 
-def run_alone(d, fn, gts, keeps, seeds):
+def _standin(x, t, **k):
+    """Per-sample elementwise eps model (tests/test_gpu_continuous.py), its value per image batch independent, with the
+    variance channels the learned-sigma diffusion expects."""
+    eps = torch.tanh(0.7 * x) * torch.cos(t.float().view(-1, 1, 1, 1) * 0.01) + 0.05 * k["gt"]
+    return torch.cat([eps, torch.zeros_like(eps)], 1)
+
+
+def standin_checks(w, gts, keeps, seeds, n=12):
+    """The contract on the stand-in model at 256x256: n requests through 8 continuous slots (later ones admitted as
+    earlier ones finish) against lockstep batch 8 and against each request alone."""
+    cs = w.continuous(_standin)
+    tk = [cs.submit(gts[k], keeps[k], seeds[k]) for k in range(n)]
+    res = cs.drain()
+    cont = torch.cat([res[t] for t in tk])
+    lock = w.loop(_standin, gts[:B], keeps[:B], seeds[:B])
+    alone = torch.cat([w.loop(_standin, gts[k:k + 1], keeps[k:k + 1], [seeds[k]]) for k in range(n)])
+    return {"standin_continuous_equals_lockstep_b8": bool(torch.equal(cont[:B], lock)),
+            "standin_continuous_equals_alone_b1": bool(torch.equal(cont, alone))}
+
+
+def run_alone(w, fn, gts, keeps, seeds):
     clk, done = _Clock(), []
     for k in range(N):
-        d.ddim_sample_loop(fn, (1, 3, S, S), model_kwargs={"gt": gts[k:k + 1], "gt_keep_mask": keeps[k:k + 1]},
-                           device=gts.device, use_inpainting_injection=True, seeds=[seeds[k]])
+        w.loop(fn, gts[k:k + 1], keeps[k:k + 1], [seeds[k]])
         done.append(clk.mark())
     torch.cuda.synchronize()
     lat = [clk.ms(e) for e in done]
-    return {"wall_ms": lat[-1], "latency_ms": lat, "occupancy": 1.0, "iterations": N * T}
+    return {"wall_ms": lat[-1], "latency_ms": lat, "occupancy": 1.0, "iterations": N * w.evals}
 
 
-def run_lockstep(d, fn, gts, keeps, seeds):
+def run_lockstep(w, fn, gts, keeps, seeds):
     clk, done = _Clock(), []
     for j in range(0, N, B):
-        d.ddim_sample_loop(fn, (B, 3, S, S), model_kwargs={"gt": gts[j:j + B], "gt_keep_mask": keeps[j:j + B]},
-                           device=gts.device, use_inpainting_injection=True, seeds=seeds[j:j + B])
+        w.loop(fn, gts[j:j + B], keeps[j:j + B], seeds[j:j + B])
         done += [clk.mark()] * B
     torch.cuda.synchronize()
     lat = [clk.ms(e) for e in done]
-    return {"wall_ms": lat[-1], "latency_ms": lat, "occupancy": 1.0, "iterations": N // B * T}
+    return {"wall_ms": lat[-1], "latency_ms": lat, "occupancy": 1.0, "iterations": N // B * w.evals}
 
 
-def run_continuous(d, fn, gts, keeps, seeds, arrivals_s=None):
+def run_continuous(w, fn, gts, keeps, seeds, arrivals_s=None):
     """arrivals_s: host seconds after the origin at which each request arrives (None: all queued at the origin)."""
-    cs = d.continuous_sampler(fn, slots=B, image_size=(S, S), sampler="ddim")
+    cs = w.continuous(fn)
     clk = _Clock()
     arrive_ms, done, tickets = {}, {}, {}
     k, iters, busy = 0, 0, 0
@@ -178,10 +226,95 @@ def k8_probe(d, batch, dev):
     return res
 
 
+def _graph_us(fn):
+    """us per call of `fn`, replayed in a CUDA graph of 20 calls."""
+    for _ in range(3):
+        fn()
+    stream = torch.cuda.Stream()
+    stream.wait_stream(torch.cuda.current_stream())
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.stream(stream):
+        with torch.cuda.graph(graph):
+            for _ in range(20):
+                fn()
+    torch.cuda.current_stream().wait_stream(stream)
+    graph.replay()
+    ms = min(event_ms(graph.replay, 10) for _ in range(3)) / 20
+    del graph
+    return ms * 1e3
+
+
+def k9_probe(d, steps, batch, dev):
+    """us per step, order-2 update at grid point 5 + cumulative injection + bf16 stem: seeded K6 against K9 (every slot
+    at that point, state and history in place), CUDA graph of 20."""
+    from fidm_b200 import _lib as L
+    from fidm_b200 import continuous, dpm_solver, seeded
+    from fidm_b200.gaussian_diffusion import _MEAN_CODE
+    k = 5
+    grid = dpm_solver.timestep_grid(d.num_timesteps, steps)
+    tab = d._dpm_table(dev, steps, 2, True)
+    g = torch.Generator(device=dev).manual_seed(batch)
+    x = torch.randn(batch, 3, S, S, device=dev, generator=g)
+    mo = torch.randn(batch, 6, S, S, device=dev, generator=g)
+    mp = torch.rand(batch, 3, S, S, device=dev, generator=g)
+    gt = torch.rand(batch, 3, S, S, device=dev, generator=g)
+    keep = (torch.rand(batch, 3, S, S, device=dev, generator=g) > 0.5).float()
+    x_in = torch.zeros(batch, S, S, 16, device=dev, dtype=torch.bfloat16)
+    t_in = torch.zeros(batch, device=dev)
+    seeds = seeded.check_seeds(list(range(batch)), batch).to(dev)
+    t_next = d._t_value(int(grid[k + 1]))
+
+    def k6():
+        return d._multistep(tab, k, x, mo, m_prev=mp, gt=gt, keep=keep,
+                            inject_noise=seeded.Draw(seeds, L.NOISE_INJECT, int(grid[k + 1])), stem=(x_in, t_in),
+                            t_next=t_next)
+
+    xs, ms = x.clone(), mp.clone()
+    tables = continuous.dpm_slot_tables(d, grid, 2, "all", True)
+    tv, inj, order = (torch.tensor(v, dtype=dt, device=dev) for v, dt in
+                      zip(tables, (torch.float32, torch.int32, torch.int32)))
+    out = torch.empty_like(x)
+    a = L.MultistepArgs()
+    a.batch, a.channels, a.hw, a.steps = batch, 3, S * S, steps
+    a.mean_type, a.out_channels, a.clip_denoised, a.mask_channels = _MEAN_CODE[d.model_mean_type], 6, 1, 3
+    a.coef, a.x, a.model_out, a.m_prev, a.m_out, a.x_next, a.gt, a.keep_mask = (
+        L.ptr(v) for v in (tab, xs, mo, ms, ms, xs, gt, keep))
+    a.stem_out, a.stem_dtype, a.stem_ld, a.t_out = L.ptr(x_in), L.BF16, 16, L.ptr(t_in)
+    s = L.MsSlotArgs()
+    s.t_value, s.inject_draw, s.order, s.out = L.ptr(tv), L.ptr(inj), L.ptr(order), L.ptr(out)
+    s.inject_tag = L.NOISE_INJECT
+    for b in range(batch):
+        s.action[b], s.seeds[b] = k, b
+
+    def k9():
+        L.check(L.lib().fidm_multistep_step_slots(ctypes.byref(a), ctypes.byref(s), L.stream()),
+                "multistep_step_slots")
+
+    def k9_fresh():                                  # every timed launch starts from the same state and history
+        xs.copy_(x), ms.copy_(mp)
+        k9()
+
+    # read x, eps (3 of 6 channels), m_{k-1}, gt, mask: 5 x 12 B; write m_k, x_next: 2 x 12 B; stem 3 x bf16
+    nbytes = batch * S * S * (5 * 12 + 2 * 12 + 6)
+    res = {"batch": batch, "bytes_per_step": nbytes}
+    for name, fn in (("seeded_k6", k6), ("k9", k9)):
+        us = _graph_us(fn)
+        res[name] = {"us_per_step": round(us, 2), "gbs": round(nbytes / (us * 1e-6) / 1e9, 1)}
+    m_ref, x_ref = k6()
+    ref_stem, ref_t = x_in.clone(), t_in.clone()
+    x_in.zero_(), t_in.zero_()
+    k9_fresh()
+    res["k9_equals_k6"] = bool(torch.equal(xs, x_ref) and torch.equal(ms, m_ref) and torch.equal(x_in, ref_stem)
+                               and torch.equal(t_in, ref_t))
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--rounds", type=int, default=3, help="alternating timing rounds (the median is reported)")
     ap.add_argument("--load", type=float, default=0.8, help="Poisson arrival rate of (d) as a fraction of (b)'s rate")
+    ap.add_argument("--sampler", choices=("ddim", "dpm_solver"), default="ddim", help="the sampler of every arm")
+    ap.add_argument("--steps", type=int, default=20, help="model evaluations per request of --sampler dpm_solver")
     args = ap.parse_args()
     import fidm_b200 as F
     from fidm_b200.utils.synth import synth_batch, synth_state_dict
@@ -194,28 +327,29 @@ def main():
     model.to(dev)
     model.base_model.set_precision("bf16")
     fn = F.InpaintingModelFn(model)
-    d = F.create_gaussian_diffusion(steps=T, learn_sigma=True, noise_schedule="cosine")
+    w = Workload(F, args.sampler, args.steps)
+    d = w.d
     data = synth_batch(N, S, seed=100, device=dev)
     gts, keeps = data["gt"], data["gt_keep_mask"]
     seeds = list(range(5000, 5000 + N))
     with torch.no_grad():
         # warm-up: plans and graphs of batch 1 and 8, tables; checks that (c) reproduces (a) and (b)
-        lock = d.ddim_sample_loop(fn, (B, 3, S, S), model_kwargs={"gt": gts[:B], "gt_keep_mask": keeps[:B]},
-                                  device=dev, use_inpainting_injection=True, seeds=seeds[:B])
-        alone = d.ddim_sample_loop(fn, (1, 3, S, S), model_kwargs={"gt": gts[:1], "gt_keep_mask": keeps[:1]},
-                                   device=dev, use_inpainting_injection=True, seeds=seeds[:1])
-        cs = d.continuous_sampler(fn, slots=B, image_size=(S, S), sampler="ddim")
+        lock = w.loop(fn, gts[:B], keeps[:B], seeds[:B])
+        alone = w.loop(fn, gts[:1], keeps[:1], seeds[:1])
+        cs = w.continuous(fn)
         tk = [cs.submit(gts[k], keeps[k], seeds[k]) for k in range(B)]
         res_c = cs.drain()
         cont = torch.cat([res_c[t] for t in tk])
         checks = {"continuous_equals_lockstep_b8": bool(torch.equal(cont, lock)),
                   "continuous_equals_alone_b1": bool(torch.equal(cont[:1], alone)),
                   "lockstep_b8_equals_alone_b1": bool(torch.equal(lock[:1], alone))}
+        if w.dpm:
+            checks.update(standin_checks(w, gts, keeps, seeds))
         ev = {1: eval_ms(fn, 1), B: eval_ms(fn, B)}
         rate_b = None
-        runs = {"a_alone_b1": lambda: run_alone(d, fn, gts, keeps, seeds),
-                "b_lockstep_b8": lambda: run_lockstep(d, fn, gts, keeps, seeds),
-                "c_continuous_all_queued": lambda: run_continuous(d, fn, gts, keeps, seeds),
+        runs = {"a_alone_b1": lambda: run_alone(w, fn, gts, keeps, seeds),
+                "b_lockstep_b8": lambda: run_lockstep(w, fn, gts, keeps, seeds),
+                "c_continuous_all_queued": lambda: run_continuous(w, fn, gts, keeps, seeds),
                 "d_continuous_poisson": None}
         got = {name: [] for name in runs}
         for r in range(args.rounds):
@@ -227,19 +361,24 @@ def main():
                     for _ in range(N):
                         t += rng.expovariate(rate)
                         arr.append(t)
-                    got[name].append(run_continuous(d, fn, gts, keeps, seeds, arr))
+                    got[name].append(run_continuous(w, fn, gts, keeps, seeds, arr))
                 else:
                     got[name].append(run())
                 if name == "b_lockstep_b8" and rate_b is None:
                     rate_b = N / (got[name][-1]["wall_ms"] * 1e-3)
-        steps = [k8_probe(d, b, dev) for b in (8, 64)]
+        if w.dpm:
+            steps = [k9_probe(d, args.steps, b, dev) for b in (8, 64)]
+            checks["k9_equals_k6"] = all(st.pop("k9_equals_k6") for st in steps)
+        else:
+            steps = [k8_probe(d, b, dev) for b in (8, 64)]
     cp = copy_gbs(dev)
     for st in steps:
-        for name in ("seeded_k4", "k8"):
+        for name in (("seeded_k6", "k9") if w.dpm else ("seeded_k4", "k8")):
             st[name]["fraction_of_copy"] = round(st[name]["gbs"] / cp, 3)
     out = {"probe": "continuous", "gpu": info,
-           "config": "ADM256 bf16, 256x256, DDIM-50 cosine, injection on, seeded, 8 slots, 64 requests (5-60 % holes), "
-                     "synthetic weights",
+           "config": "ADM256 bf16, 256x256, %s, injection on, seeded, 8 slots, 64 requests (5-60 %% holes), "
+                     "synthetic weights" % ("DPM-Solver++ 2M-%d quadratic 1000" % args.steps if w.dpm
+                                            else "DDIM-50 cosine"),
            "checks": checks, "eval_ms_alone": {str(k): round(v, 3) for k, v in ev.items()},
            "poisson_rate_per_s": round(args.load * rate_b, 3), "copy_gbs": cp, "step": steps, "runs": {}}
     for name, rs in got.items():
