@@ -1,6 +1,5 @@
 // Error plumbing and device probing for the C ABI (include/fidm_b200.h).
 #include <stdarg.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -12,12 +11,6 @@ void set_error(const char* fmt, ...) {
   va_start(ap, fmt);
   vsnprintf(g_err, sizeof(g_err), fmt, ap);
   va_end(ap);
-}
-bool pdl_enabled() {
-  // Off by default: measured on B200 inside the CUDA graph of a UNet evaluation, programmatic edges bought nothing
-  // (17.22 vs 17.16 ms) and with an early launch_dependents trigger they cost 1.5 % (ADM256) to 6 % (REF-FFHQ256).
-  static const bool on = getenv("FIDM_PDL") != nullptr && atoi(getenv("FIDM_PDL")) != 0;
-  return on;
 }
 }  // namespace fidm
 

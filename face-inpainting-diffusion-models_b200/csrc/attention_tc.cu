@@ -88,10 +88,6 @@ attn_tc_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant_
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  // PDL: everything above (barrier init, TMEM allocation, descriptor prefetch) overlapped the previous kernel's tail;
-  // nothing below may touch global memory before that kernel has completed.
-  pdl_wait();
-  pdl_trigger();
   const uint32_t tmem_S = tmem_base, tmem_O = tmem_base + 128;
 
   if (warp == 4) {
@@ -289,11 +285,11 @@ extern "C" int fidm_attention_qkv_nhwc_bf16(const fidm_attn_args* a, fidm_stream
   if (a->head_dim == 64) {
     static bool attr_set[kMaxDevices] = {};      // per (instantiation, device)
     FIDM_CUDA(ensure_dynamic_smem(attn_tc_kernel<64>, AttnCfg<64>::kSmem, attr_set));
-    FIDM_CUDA(launch_pdl(attn_tc_kernel<64>, grid, dim3(kAttnThreads), AttnCfg<64>::kSmem, (cudaStream_t)stream, 1, tmQKV, tmO, p));
+    FIDM_CUDA(launch_kernel(attn_tc_kernel<64>, grid, dim3(kAttnThreads), AttnCfg<64>::kSmem, (cudaStream_t)stream, 1, tmQKV, tmO, p));
   } else {
     static bool attr_set[kMaxDevices] = {};
     FIDM_CUDA(ensure_dynamic_smem(attn_tc_kernel<128>, AttnCfg<128>::kSmem, attr_set));
-    FIDM_CUDA(launch_pdl(attn_tc_kernel<128>, grid, dim3(kAttnThreads), AttnCfg<128>::kSmem, (cudaStream_t)stream, 1, tmQKV, tmO, p));
+    FIDM_CUDA(launch_kernel(attn_tc_kernel<128>, grid, dim3(kAttnThreads), AttnCfg<128>::kSmem, (cudaStream_t)stream, 1, tmQKV, tmO, p));
   }
   FIDM_CHECK_LAUNCH("attention_tc");
   return 0;

@@ -115,38 +115,16 @@ __device__ __forceinline__ int fdiv(int n, const FastDiv& f) {
   return (int)((__umulhi(f.mul, (uint32_t)n) + (uint32_t)n) >> f.sh);
 }
 
-// ---- programmatic dependent launch (PDL), opt-in with FIDM_PDL=1.  The kernels of the UNet call pdl_wait() before their
-// first access to global memory that an earlier kernel may have written (or may still read), so they MAY be launched
-// with the programmatic-stream-serialization attribute: the launch, the block scheduling and the prologue (barrier
-// init, TMEM allocation, descriptor prefetch) then overlap the predecessor.  pdl_trigger() lets the successor launch
-// early ONLY when this grid is a single wave (every block resident: at most one per SM): round 1 measured that an
-// unconditional early trigger costs 1.5-6 % at batch 8, because the successor's blocks take SM resources from the
-// later waves of a multi-wave predecessor; a multi-wave grid keeps the implicit trigger at its completion.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-constexpr unsigned kPdlSingleWaveBlocks = 148;       // B200: one block per SM
-__device__ __forceinline__ void pdl_trigger() {
-  if (gridDim.x * gridDim.y * gridDim.z <= kPdlSingleWaveBlocks) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-bool pdl_enabled();          // FIDM_PDL=0 switches the attribute off (the device-side calls are then no-ops)
-
+// ---- cudaLaunchKernelEx with a 1-D thread-block cluster of `cluster` CTAs (no attribute when cluster == 1)
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, int cluster,
-                              Args&&... args) {
+inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                 int cluster, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  int n = 0;
-  if (cluster > 1) {
-    attr[n].id = cudaLaunchAttributeClusterDimension;
-    attr[n].val.clusterDim.x = cluster; attr[n].val.clusterDim.y = 1; attr[n].val.clusterDim.z = 1;
-    ++n;
-  }
-  if (pdl_enabled()) {
-    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
-  cfg.attrs = attr; cfg.numAttrs = n;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = cluster; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr; cfg.numAttrs = cluster > 1 ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 

@@ -155,10 +155,6 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_constan
   cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  // PDL: everything above (barrier init, TMEM allocation, descriptor prefetch) overlapped the previous kernel's tail;
-  // nothing below may touch global memory before that kernel has completed.
-  pdl_wait();
-  pdl_trigger();
 
   if (warp >= 13) {
     if (warp == 13 && lane == 0) {
@@ -679,8 +675,8 @@ static int launch_conv_halo_t(const fidm_conv_args& a, cudaStream_t st) {
   const int units = (p.tiles_w * p.tiles_h * p.B / 2) * p.n_blocks;
   const int slots = num_sms() / 2;
   const int grid = (units < slots ? units : slots) * 2;
-  FIDM_CUDA(launch_pdl(conv_halo_kernel<BLOCK_N, OPK, UP, PROF>, dim3(grid), dim3(kThreads), kSmemBytes, st, 2, tmRaw, tmB, tmA2,
-                       tmB2, tmY, tmRes, p));
+  FIDM_CUDA(launch_kernel(conv_halo_kernel<BLOCK_N, OPK, UP, PROF>, dim3(grid), dim3(kThreads), kSmemBytes, st, 2, tmRaw, tmB, tmA2,
+                          tmB2, tmY, tmRes, p));
   FIDM_CHECK_LAUNCH("conv_halo");
   return 0;
 }

@@ -31,7 +31,6 @@
 // Warp roles (640 threads, 96 registers): 0-7 epilogue (two warpgroups), 8-16 transform, 17 weight-ring producer,
 // 18 MMA issuer + TMEM owner, 19 halo producer.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "conv_act.cuh"
@@ -142,8 +141,6 @@ conv_halo_swap_kernel(const __grid_constant__ CUtensorMap tmRaw, const __grid_co
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
-  pdl_trigger();
 
   if (warp >= 17) {
     if (warp == 17 && lane == 0) {
@@ -615,9 +612,7 @@ bool conv_halo_swap_supported(const fidm_conv_args& a) {
 }
 
 bool conv_halo_swap_preferred(const fidm_conv_args& a) {
-  // FIDM_HALO_SWAP=0: A/B switch back to K1h's 128-wide / 16-wide tiles
-  static const bool on = getenv("FIDM_HALO_SWAP") == nullptr || atoi(getenv("FIDM_HALO_SWAP")) != 0;
-  return on && conv_halo_swap_supported(a) && (a.y_nchw_f32 || a.cout % 256 != 0);
+  return conv_halo_swap_supported(a) && (a.y_nchw_f32 || a.cout % 256 != 0);
 }
 
 template <bool OUT_F16, bool kHead, bool PROF = false, bool ACT = true, bool UP = false>
@@ -655,8 +650,8 @@ static int launch_conv_halo_swap_t(const fidm_conv_args& a, cudaStream_t st, uns
   const int units = p.tiles_w * p.tiles_h * p.B * p.n_blocks;
   const int sms = num_sms();
   const int grid = units < sms ? units : sms;
-  FIDM_CUDA(launch_pdl(conv_halo_swap_kernel<OUT_F16, kHead, PROF, ACT, UP>, dim3(grid), dim3(kThreads), kSmemBytes, st, 1, tmRaw, tmW, tmX2,
-                       tmW2, p));
+  FIDM_CUDA(launch_kernel(conv_halo_swap_kernel<OUT_F16, kHead, PROF, ACT, UP>, dim3(grid), dim3(kThreads), kSmemBytes, st, 1, tmRaw, tmW, tmX2,
+                          tmW2, p));
   FIDM_CHECK_LAUNCH("conv_halo_swap");
   return 0;
 }

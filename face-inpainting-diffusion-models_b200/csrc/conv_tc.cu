@@ -223,10 +223,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   if (threadIdx.x == 0) TL(1);
-  // PDL: everything above (barrier init, TMEM allocation, descriptor prefetch) overlapped the previous kernel's tail;
-  // nothing below may touch global memory before that kernel has completed.
-  pdl_wait();
-  pdl_trigger();
 
   if (warp == 8) {
     // ===================================================================== TMA producer
@@ -716,8 +712,8 @@ static int launch_conv_tc(const fidm_conv_args& a, cudaStream_t st, int split_k 
   const int slots = num_sms() / CG;
   // cluster split: one unit per CTA (clusters beyond the machine's capacity queue behind the first wave)
   const int grid = p.cluster_split ? units : (units < slots ? units : slots) * CG;
-  FIDM_CUDA(launch_pdl(conv_tc_kernel<BLOCK_N, CG>, dim3(grid), dim3(kThreads), Cfg::kSmemBytes, st,
-                       p.cluster_split ? split_k : CG, tmA, tmB, tmA2, tmB2, tmY, p));
+  FIDM_CUDA(launch_kernel(conv_tc_kernel<BLOCK_N, CG>, dim3(grid), dim3(kThreads), Cfg::kSmemBytes, st,
+                          p.cluster_split ? split_k : CG, tmA, tmB, tmA2, tmB2, tmY, p));
   FIDM_CHECK_LAUNCH("conv_tc");
   return 0;
 }
@@ -738,8 +734,7 @@ extern "C" int fidm_conv_gn_fusable(int32_t batch, int32_t height, int32_t width
   a.dtype = FIDM_F16; a.batch = batch; a.height = height; a.width = width;
   a.cin = cin; a.cout = cout; a.ksize = ksize; a.stride = stride;
   a.y_nchw_f32 = cout == 16;        // the 16-wide variant is the fp32-NCHW head
-  // FIDM_HALO_MIN_FILL: percent of the CTA pairs (K1s: of the SMs) that must have a unit (default 75)
-  static const int min_fill = getenv("FIDM_HALO_MIN_FILL") ? atoi(getenv("FIDM_HALO_MIN_FILL")) : 75;
+  constexpr int min_fill = 75;      // percent of the CTA pairs (K1s: of the SMs) that must have a unit
   if (fidm::conv_halo_swap_preferred(a)) {
     // K1s: one 16 x 16 pixel box x 128 output channels per SM
     const long long units = (long long)batch * (height / 16) * (width / 16) * (cout == 16 ? 1 : cout / 128);
@@ -782,16 +777,13 @@ extern "C" int fidm_conv2d_nhwc_bf16(const fidm_conv_args* a, fidm_stream_t stre
   pick_pixel_box(Wo, Ho, &tw, &th, &tn);
   const long long m_tiles = (long long)(Wo / tw) * (Ho / th) * ((a->batch + tn - 1) / tn);
   const int want = (num_sms() * 3) / 4;
-  static const bool pair_ok = getenv("FIDM_CONV_CTA_PAIR") == nullptr || atoi(getenv("FIDM_CONV_CTA_PAIR")) != 0;
-  if (a->cout % 256 == 0 && m_tiles * (a->cout / 256) >= want)
-    return pair_ok ? launch_conv_tc<256, 2>(*a, st) : launch_conv_tc<256, 1>(*a, st);
+  if (a->cout % 256 == 0 && m_tiles * (a->cout / 256) >= want) return launch_conv_tc<256, 2>(*a, st);
   // Low-resolution layers (few pixel tiles, deep K).  Candidate (N tile, K split) pairs are scored with a small
   // cost model in SM cycles: tensor time of one CTA's share of the K loop, L2->SM operand traffic of the whole grid
   // against the ~12 KB/clk the L2 delivers (measured: 442 MB in 62 us on the 16x16 layers; these layers re-read the
   // weights once per pixel tile), and the fold of the split partials (shared by the cluster, or by the last CTA of a
   // tile on the workspace path).  tools/conv_tune.py checks the pick against every forced candidate.
   const int k_iters = a->ksize * a->ksize * (a->cin / 64) + (a->x2 ? a->cin2 / 64 : 0);
-  static const bool split_ok = getenv("FIDM_CONV_SPLIT_K") == nullptr || atoi(getenv("FIDM_CONV_SPLIT_K")) != 0;
   // FIDM_CONV_SPLIT_CLUSTER=0: fold split partials through the global workspace (the round-1 path) instead of a cluster
   static const bool cluster_ok = getenv("FIDM_CONV_SPLIT_CLUSTER") == nullptr || atoi(getenv("FIDM_CONV_SPLIT_CLUSTER")) != 0;
   // (the shared fold hands a thread 4 consecutive pixels of one box row: TW >= 4)
@@ -805,7 +797,7 @@ extern "C" int fidm_conv2d_nhwc_bf16(const fidm_conv_args* a, fidm_stream_t stre
     if (a->cout % N) continue;
     const long long tiles = m_tiles * (a->cout / N);
     for (int S = 1; S <= 8; ++S) {
-      if (S > 1 && (!split_ok || k_iters / S < 4)) break;
+      if (S > 1 && k_iters / S < 4) break;
       if (use_cluster && S != 1 && S != 2 && S != 4 && S != 8) continue;
       if (S > 1 && (!a->splitk_ws || a->splitk_ws_bytes < kSplitCounterBytes + tiles * S * N * 128 * 4 ||
                     (!use_cluster && tiles * 4 > kSplitCounterBytes)))

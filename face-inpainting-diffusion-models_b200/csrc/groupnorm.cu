@@ -10,7 +10,6 @@
 // affine coefficients in registers.  Statistics are accumulated in fp32 per thread, then reduced in
 // double precision in a fixed order (block partials, folded by the last block of each image to finish):
 // no floating-point atomics, so the result is bit-reproducible.
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -44,8 +43,6 @@ __device__ __forceinline__ float2 gn_half_coeff(const fidm_gn_args& a, int n, in
 template <typename T, int VEC>
 __global__ void gn_stats_kernel(const GnParams p, double* __restrict__ partials, int* __restrict__ counters,
                                 float2* __restrict__ coef, int ld_coef) {
-  pdl_wait();
-  pdl_trigger();
   const fidm_gn_args& a = p.a;
   extern __shared__ float red[];           // [blockDim][2]
   const int n = blockIdx.y;
@@ -150,8 +147,6 @@ __global__ void gn_stats_kernel(const GnParams p, double* __restrict__ partials,
 // and reduces it in a fixed tree -- no workspace, no cross-block step, one short launch.
 template <typename T, int VEC>
 __global__ void __launch_bounds__(256) gn_stats_direct_kernel(const GnParams p, float2* __restrict__ coef, int ld_coef) {
-  pdl_wait();
-  pdl_trigger();
   const fidm_gn_args& a = p.a;
   __shared__ double red[8][2];
   __shared__ float mr_s[2];
@@ -221,8 +216,6 @@ __device__ __forceinline__ float silu_f(float v) {
 // image of a 512-channel tensor, 8192 vectors per group, in one launch).
 template <typename TY, int NV, int CS = 1>
 __global__ void __launch_bounds__(512, 1) gn_fused_small_kernel(const fidm_gn_args a, int vpp, int stride) {
-  pdl_wait();
-  pdl_trigger();
   __shared__ double red[16][2];
   __shared__ __align__(16) double part[2];
   __shared__ float mr[2];
@@ -353,9 +346,8 @@ __global__ void __launch_bounds__(512, 1) gn_fused_small_kernel(const fidm_gn_ar
 // (image, group): the one-launch path.  Returns -1 when it does not apply.
 static bool gn_fused_small_plan(const fidm_gn_args& a, int* vpp_o, int* threads_o, int* stride_o, int* per_thread_o,
                                 int* cluster_o = nullptr) {
-  static const bool enabled = getenv("FIDM_GN_FUSED_SMALL") == nullptr || atoi(getenv("FIDM_GN_FUSED_SMALL")) != 0;
   const int cpg = a.channels / a.groups;
-  if (!enabled || a.dtype != FIDM_BF16 || (a.y_dtype != FIDM_BF16 && a.y_dtype != FIDM_F16)) return false;
+  if (a.dtype != FIDM_BF16 || (a.y_dtype != FIDM_BF16 && a.y_dtype != FIDM_F16)) return false;
   if (a.skip_norm || a.chansum || a.resample != FIDM_RESAMPLE_NONE || cpg % 8 != 0) return false;
   if (a.ld_x % 8 || a.ld_y % 8 || (uintptr_t)a.x % 16 || (uintptr_t)a.y % 16) return false;
   const int vpp = cpg / 8;
@@ -387,24 +379,22 @@ static int try_gn_fused_small(const fidm_gn_args& a, cudaStream_t st) {
   if (!gn_fused_small_plan(a, &vpp, &threads, &stride, &per_thread, &cluster)) return -1;
   dim3 grid(a.groups * cluster, a.batch);
   if (cluster == 4) {
-    if (per_thread <= 2) launch_pdl(gn_fused_small_kernel<TY, 2, 4>, grid, dim3(threads), 0, st, 4, a, vpp, stride);
-    else if (per_thread <= 4) launch_pdl(gn_fused_small_kernel<TY, 4, 4>, grid, dim3(threads), 0, st, 4, a, vpp, stride);
-    else launch_pdl(gn_fused_small_kernel<TY, 8, 4>, grid, dim3(threads), 0, st, 4, a, vpp, stride);
+    if (per_thread <= 2) launch_kernel(gn_fused_small_kernel<TY, 2, 4>, grid, dim3(threads), 0, st, 4, a, vpp, stride);
+    else if (per_thread <= 4) launch_kernel(gn_fused_small_kernel<TY, 4, 4>, grid, dim3(threads), 0, st, 4, a, vpp, stride);
+    else launch_kernel(gn_fused_small_kernel<TY, 8, 4>, grid, dim3(threads), 0, st, 4, a, vpp, stride);
   } else if (cluster == 2) {
-    if (per_thread <= 4) launch_pdl(gn_fused_small_kernel<TY, 4, 2>, grid, dim3(threads), 0, st, 2, a, vpp, stride);
-    else launch_pdl(gn_fused_small_kernel<TY, 8, 2>, grid, dim3(threads), 0, st, 2, a, vpp, stride);
+    if (per_thread <= 4) launch_kernel(gn_fused_small_kernel<TY, 4, 2>, grid, dim3(threads), 0, st, 2, a, vpp, stride);
+    else launch_kernel(gn_fused_small_kernel<TY, 8, 2>, grid, dim3(threads), 0, st, 2, a, vpp, stride);
   }
-  else if (per_thread <= 2) launch_pdl(gn_fused_small_kernel<TY, 2>, grid, dim3(threads), 0, st, 1, a, vpp, stride);
-  else if (per_thread <= 4) launch_pdl(gn_fused_small_kernel<TY, 4>, grid, dim3(threads), 0, st, 1, a, vpp, stride);
-  else launch_pdl(gn_fused_small_kernel<TY, 8>, grid, dim3(threads), 0, st, 1, a, vpp, stride);
+  else if (per_thread <= 2) launch_kernel(gn_fused_small_kernel<TY, 2>, grid, dim3(threads), 0, st, 1, a, vpp, stride);
+  else if (per_thread <= 4) launch_kernel(gn_fused_small_kernel<TY, 4>, grid, dim3(threads), 0, st, 1, a, vpp, stride);
+  else launch_kernel(gn_fused_small_kernel<TY, 8>, grid, dim3(threads), 0, st, 1, a, vpp, stride);
   FIDM_CHECK_LAUNCH("groupnorm (fused small)");
   return 0;
 }
 
 template <typename T, typename TY, int VEC, int RESAMPLE>
 __global__ void __launch_bounds__(1024, 1) gn_apply_kernel(const GnParams p) {
-  pdl_wait();
-  pdl_trigger();
   const fidm_gn_args& a = p.a;
   constexpr bool FAST = (sizeof(T) == 2);
   const int n = blockIdx.y;
@@ -552,8 +542,6 @@ __global__ void __launch_bounds__(1024, 1) gn_apply_kernel(const GnParams p) {
 // (silu(x*A + B) = h + h*tanh(h), h = x*A/2 + B/2).  Same arithmetic as the head of gn_apply_kernel, so a conv that
 // applies the activation in its operand path sees exactly the coefficients the apply pass would have used.
 __global__ void __launch_bounds__(256) gn_coeff_kernel(const fidm_gn_args a, float2* __restrict__ coef, int ld_coef) {
-  pdl_wait();
-  pdl_trigger();
   __shared__ float2 mr_s[64];
   const int n = blockIdx.x;
   const int hw = a.height * a.width;
@@ -605,7 +593,7 @@ static int launch_gn(const fidm_gn_args& a, cudaStream_t st, float2* coef = null
   };
   int chunks;
   if (!a.skip_norm && !a.chansum && (long long)hw * (a.channels / a.groups) <= 32768) {    // <= 64 KB per (image, group) block
-    launch_pdl(gn_stats_direct_kernel<T, VEC>, dim3(a.groups, a.batch), dim3(256), 0, st, 1, p, coef, ld_coef);
+    launch_kernel(gn_stats_direct_kernel<T, VEC>, dim3(a.groups, a.batch), dim3(256), 0, st, 1, p, coef, ld_coef);
     FIDM_CHECK_LAUNCH("groupnorm stats (direct)");
   } else if (!a.skip_norm && !a.chansum) {
     // workspace: [batch*groups*2] floats (mean, rstd) padded to doubles, then the per-block partials
@@ -622,13 +610,13 @@ static int launch_gn(const fidm_gn_args& a, cudaStream_t st, float2* coef = null
     }
     const long long blocks_cap = (FIDM_GN_MAX_BLOCKS > a.batch ? FIDM_GN_MAX_BLOCKS : a.batch) + a.batch;
     int* counters = reinterpret_cast<int*>(partials + blocks_cap * a.groups * 2);
-    launch_pdl(gn_stats_kernel<T, VEC>, dim3(chunks, a.batch), dim3(threads),
-               sizeof(float) * 2 * threads + 8 * 64 * 2 * sizeof(double), st, 1, p, partials, counters, coef, ld_coef);
+    launch_kernel(gn_stats_kernel<T, VEC>, dim3(chunks, a.batch), dim3(threads),
+                  sizeof(float) * 2 * threads + 8 * 64 * 2 * sizeof(double), st, 1, p, partials, counters, coef, ld_coef);
     FIDM_CHECK_LAUNCH("groupnorm stats");
   }
   if (coef) {      // statistics only: the consumer conv applies the activation in its operand path
     if (a.chansum) {         // (the statistics kernels above wrote the coefficients themselves)
-      launch_pdl(gn_coeff_kernel, dim3(a.batch), dim3(256), 0, st, 1, a, coef, ld_coef);
+      launch_kernel(gn_coeff_kernel, dim3(a.batch), dim3(256), 0, st, 1, a, coef, ld_coef);
       FIDM_CHECK_LAUNCH("groupnorm coeff");
     }
     return 0;
@@ -637,11 +625,11 @@ static int launch_gn(const fidm_gn_args& a, cudaStream_t st, float2* coef = null
   dim3 grid(chunks, a.batch);
   const size_t sm = a.chansum ? sizeof(float2) * (a.channels + a.groups) : 0;
   if (a.resample == FIDM_RESAMPLE_NONE)
-    launch_pdl(gn_apply_kernel<T, TY, VEC, FIDM_RESAMPLE_NONE>, grid, dim3(threads), sm, st, 1, p);
+    launch_kernel(gn_apply_kernel<T, TY, VEC, FIDM_RESAMPLE_NONE>, grid, dim3(threads), sm, st, 1, p);
   else if (a.resample == FIDM_RESAMPLE_DOWN)
-    launch_pdl(gn_apply_kernel<T, TY, VEC, FIDM_RESAMPLE_DOWN>, grid, dim3(threads), sm, st, 1, p);
+    launch_kernel(gn_apply_kernel<T, TY, VEC, FIDM_RESAMPLE_DOWN>, grid, dim3(threads), sm, st, 1, p);
   else
-    launch_pdl(gn_apply_kernel<T, TY, VEC, FIDM_RESAMPLE_UP>, grid, dim3(threads), sm, st, 1, p);
+    launch_kernel(gn_apply_kernel<T, TY, VEC, FIDM_RESAMPLE_UP>, grid, dim3(threads), sm, st, 1, p);
   FIDM_CHECK_LAUNCH("groupnorm apply");
   return 0;
 }
@@ -716,8 +704,6 @@ __global__ void __launch_bounds__(1024) gn_reduce_colsum_kernel(const float2* __
                                                                 float2* __restrict__ chansum, int ld, int c0,
                                                                 const fidm_gn_args a, float2* __restrict__ coef, int ld_coef) {
   constexpr int RS = 1024 / CB;
-  pdl_wait();
-  pdl_trigger();
   __shared__ double red[RS][CB][2];
   __shared__ double red8[8][CB][2];
   __shared__ double csum[CB][2];
@@ -797,9 +783,9 @@ static int reduce_colsum_cb(int channels, int batch, int cpg) {
 
 static void launch_reduce_colsum(int cb, dim3 grid, cudaStream_t st, const float2* colsum, int slots, int C, float2* chansum,
                                  int ld, int c0, const fidm_gn_args& a, float2* coef, int ld_coef) {
-  if (cb == 8) launch_pdl(gn_reduce_colsum_kernel<8>, grid, dim3(1024), 0, st, 1, colsum, slots, C, chansum, ld, c0, a, coef, ld_coef);
-  else if (cb == 16) launch_pdl(gn_reduce_colsum_kernel<16>, grid, dim3(1024), 0, st, 1, colsum, slots, C, chansum, ld, c0, a, coef, ld_coef);
-  else launch_pdl(gn_reduce_colsum_kernel<32>, grid, dim3(1024), 0, st, 1, colsum, slots, C, chansum, ld, c0, a, coef, ld_coef);
+  if (cb == 8) launch_kernel(gn_reduce_colsum_kernel<8>, grid, dim3(1024), 0, st, 1, colsum, slots, C, chansum, ld, c0, a, coef, ld_coef);
+  else if (cb == 16) launch_kernel(gn_reduce_colsum_kernel<16>, grid, dim3(1024), 0, st, 1, colsum, slots, C, chansum, ld, c0, a, coef, ld_coef);
+  else launch_kernel(gn_reduce_colsum_kernel<32>, grid, dim3(1024), 0, st, 1, colsum, slots, C, chansum, ld, c0, a, coef, ld_coef);
 }
 }  // namespace fidm
 

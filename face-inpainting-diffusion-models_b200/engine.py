@@ -197,7 +197,7 @@ class Weights:
 class Plan:
     """Flat kernel schedule + buffers for one (batch, H, W)."""
 
-    def __init__(self, weights: Weights, B, H, W, use_graph=True, out=None):
+    def __init__(self, weights: Weights, B, H, W, use_graph=True):
         self.w, self.B, self.H, self.W = weights, B, H, W
         topo = weights.topo
         dev, dt = weights.device, weights.dtype
@@ -206,7 +206,7 @@ class Plan:
         self.pool = _Pool(dev, dt)
         self.keep = []
         # fused GroupNorm statistics: per-storage [B, ld, 2] channel sums written by the producing convs
-        self.fuse_stats = os.environ.get("FIDM_FUSE_GN_STATS", "1") != "0" and weights.tc
+        self.fuse_stats = weights.tc
         # GroupNorm + SiLU applied in the consumer conv's operand path (K1h) where fidm_conv_gn_fusable() says so
         self.fuse_gn = os.environ.get("FIDM_FUSE_GN_APPLY", "1") != "0"
         self.fuse_up = os.environ.get("FIDM_FUSE_UPSAMPLE", "1") != "0"
@@ -224,9 +224,7 @@ class Plan:
         # ---- static inputs / outputs
         self.x_in = torch.zeros(B, H, W, STEM_CIN_PAD, device=dev, dtype=weights.conv["input_blocks.0.0"][0].dtype)
         self.t_in = torch.zeros(B, device=dev, dtype=torch.float32)
-        self.out = out if out is not None else torch.empty(B, topo.out_channels, H, W, device=dev,
-                                                           dtype=torch.float32)
-        assert self.out.is_contiguous() and self.out.shape[0] == B
+        self.out = torch.empty(B, topo.out_channels, H, W, device=dev, dtype=torch.float32)
         self.stats = torch.zeros(lib.fidm_groupnorm_workspace_bytes(B, 32) // 8, device=dev, dtype=torch.float64)
 
         # ---- K5: timestep path
@@ -410,8 +408,7 @@ class Plan:
         # stem: one halo load per slice through the swapped-role kernel instead of one TMA box per tap, where the layer
         # fills the machine (one 16 x 16 pixel box x 128 output channels per SM)
         if (halo_copy and w.tc and ks == 3 and stride == 1 and Ho % 16 == 0 and Wo % 16 == 0 and cout_pad % 128 == 0 and
-                self.B * (Ho // 16) * (Wo // 16) * (cout_pad // 128) * 100 >= 148 * 75 and
-                os.environ.get("FIDM_STEM_HALO", "1") != "0"):
+                self.B * (Ho // 16) * (Wo // 16) * (cout_pad // 128) * 100 >= 148 * 75):
             a.halo_copy = 1
         use_fp8 = (gn_coef is not None and name in w.conv8 and not x_half and Ho * Wo >= self.FP8_MIN_PIXELS and
                    (x2 is None or name in w.skip8))
@@ -444,7 +441,7 @@ class Plan:
         # pass is HBM-bound (large tensors) and the epilogue is off the critical path (long K loop); measured
         # on B200: 128^2 and larger, K >= 1152.  Small tensors keep the (L2-resident) statistics kernel.
         k_total = ks * ks * cin_pad + (x2.channels if x2 is not None else 0)
-        if name == "input_blocks.0.0" and os.environ.get("FIDM_STEM_STATS", "1") != "0":
+        if name == "input_blocks.0.0":
             k_total = 1152      # the stem output feeds TWO GroupNorms (first ResBlock, last skip concat): fuse its statistics
         Hy, Wy = Ho // stride, Wo // stride                      # output resolution (Ho, Wo are the INPUT's for stride 2)
         slots = self.lib.fidm_conv_colsum_slots(Hy, Wy) if (
@@ -481,8 +478,8 @@ class Plan:
         self._op(fn, C.byref(a))
 
     TC_ATTENTION = True
-    FUSE_MIN_PIXELS = int(os.environ.get("FIDM_FUSE_MIN_PIXELS", 128 * 128))
-    FP8_MIN_PIXELS = int(os.environ.get("FIDM_FP8_MIN_PIXELS", 128 * 128))
+    FUSE_MIN_PIXELS = 128 * 128
+    FP8_MIN_PIXELS = 128 * 128
 
     # ------------------------------------------------------------------ layers
     def _block(self, blk, x, dst):
@@ -602,22 +599,22 @@ class Plan:
         return y
 
     # ------------------------------------------------------------------ execution
-    def load_inputs(self, sources, timesteps, batch_offset=0):
-        """Pack the fp32 NCHW `sources` [(tensor, channels, repeat)] (rows batch_offset .. +B) into the
-        NHWC network input and copy the timesteps."""
+    def load_inputs(self, sources, timesteps):
+        """Pack the fp32 NCHW `sources` [(tensor, channels, repeat)] into the NHWC network input and copy the
+        timesteps."""
         a = L.PackArgs()
         hw = self.H * self.W
         a.batch, a.hw, a.n_src = self.B, hw, len(sources)
         total_c = 0
         for i, (t, c, r) in enumerate(sources):
-            a.src[i] = t.data_ptr() + batch_offset * c * hw * 4
+            a.src[i] = t.data_ptr()
             a.src_channels[i], a.src_repeat[i] = c, r
             total_c += c * r
         a.dst, a.dst_dtype = self.x_in.data_ptr(), L.dtype_code(self.x_in.dtype)
         # only the first 16 channels are rewritten per call; x_in was zero-filled at allocation
         a.ld_dst, a.c_pad = STEM_CIN_PAD, (16 if total_c <= 16 else STEM_CIN_PAD)
         L.check(self.lib.fidm_pack_nchw_to_nhwc(a, L.stream()), "pack")
-        self.t_in.copy_(timesteps[batch_offset:batch_offset + self.B], non_blocking=True)
+        self.t_in.copy_(timesteps[:self.B], non_blocking=True)
 
     def load_slot(self, slot, sources, c0):
         """Pack the fp32 NCHW `sources` [(tensor [1, channels, H, W], channels, repeat)] of ONE image into image `slot`
@@ -674,7 +671,7 @@ class Plan:
             g = torch.cuda.CUDAGraph()
             self._side_stream = torch.cuda.Stream()
             with torch.cuda.graph(g):
-                self.launch_all(fork_time_path=os.environ.get("FIDM_FORK_TIME_PATH", "1") != "0")
+                self.launch_all(fork_time_path=True)
             self.graph = g
         self.graph.replay()
         return self.out
@@ -691,62 +688,3 @@ class Plan:
                 n += 1
         return n
 
-
-class PlanGroup:
-    """Two (or more) half-batch plans captured as PARALLEL branches of one CUDA graph.
-
-    The UNet alternates tensor-pipe-bound kernels (K1 conv, K3 attention) with HBM-bound ones (K2
-    GroupNorm).  Samples are independent, so the batch is split into micro-batches whose kernel chains run
-    on separate streams: while one micro-batch is in a convolution the other's GroupNorm blocks co-reside
-    on the same SMs (the conv CTAs use 192 threads and no more than one CTA per SM) and use the idle HBM
-    bandwidth.  Results are identical to the single-plan execution (every kernel is per-sample)."""
-
-    def __init__(self, weights: Weights, B, H, W, parts=2, use_graph=True):
-        assert B % parts == 0
-        self.B, self.H, self.W, self.w = B, H, W, weights
-        b = B // parts
-        self.out = torch.empty(B, weights.topo.out_channels, H, W, device=weights.device, dtype=torch.float32)
-        self.parts = [Plan(weights, b, H, W, use_graph=False, out=self.out[i * b:(i + 1) * b]) for i in range(parts)]
-        self.use_graph = use_graph
-        self.graph = None
-        self.pool = self                         # bench.py reads plan.pool.nbytes()
-
-    def nbytes(self):
-        return sum(p.pool.nbytes() for p in self.parts)
-
-    def n_launches(self):
-        return sum(p.n_launches() for p in self.parts)
-
-    def load_inputs(self, sources, timesteps):
-        for i, p in enumerate(self.parts):
-            p.load_inputs(sources, timesteps, batch_offset=i * p.B)
-
-    def run(self):
-        if not self.use_graph:
-            for p in self.parts:
-                p.launch_all()
-            return self.out
-        if self.graph is None:
-            for p in self.parts:                  # eager warm-up: func attributes, driver entry points
-                p.launch_all()
-            torch.cuda.current_stream().synchronize()
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                main = torch.cuda.current_stream()
-                fork = torch.cuda.Event()
-                fork.record(main)
-                joins = []
-                for p in self.parts[1:]:
-                    side = torch.cuda.Stream()
-                    side.wait_event(fork)
-                    with torch.cuda.stream(side):
-                        p.launch_all()
-                        ev = torch.cuda.Event()
-                        ev.record(side)
-                    joins.append(ev)
-                self.parts[0].launch_all()
-                for ev in joins:
-                    main.wait_event(ev)
-            self.graph = g
-        self.graph.replay()
-        return self.out

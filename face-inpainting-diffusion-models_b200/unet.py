@@ -10,7 +10,7 @@ import torch.nn as nn
 from . import _lib as L
 from . import nn as layers
 from .arch import unet_topology
-from .engine import STEM_CIN_PAD, Plan, PlanGroup, Weights
+from .engine import STEM_CIN_PAD, Plan, Weights
 
 
 class UNetModel(nn.Module):
@@ -71,10 +71,6 @@ class UNetModel(nn.Module):
         # ---- engine state (not part of the state_dict)
         self.precision = os.environ.get("FIDM_PRECISION", "bf16")
         self.use_cuda_graph = os.environ.get("FIDM_CUDA_GRAPH", "1") != "0"
-        # optional: micro-batches as parallel graph branches (engine.PlanGroup).  Measured on B200 at batch 8:
-        # no gain (22.97 ms with 1, 23.6 ms with 2, 25.4 ms with 4 branches) -- the eval is power-capped, not
-        # latency-bound -- so the default is a single plan.
-        self.micro_batches = int(os.environ.get("FIDM_MICRO_BATCHES", "1"))
         self._weights = None
         self._plans = {}
         # checkpoints may be loaded through a wrapper (DiffusionInpaintingModel.load_state_dict)
@@ -126,11 +122,7 @@ class UNetModel(nn.Module):
                 self._weights = Weights(topo, self.state_dict(), dev, self.precision)
         key = (batch, height, width)
         if key not in self._plans:
-            mb = self.micro_batches
-            if mb > 1 and batch % mb == 0 and batch // mb >= 2 and self.use_cuda_graph:
-                self._plans[key] = PlanGroup(self._weights, batch, height, width, parts=mb, use_graph=True)
-            else:
-                self._plans[key] = Plan(self._weights, batch, height, width, use_graph=self.use_cuda_graph)
+            self._plans[key] = Plan(self._weights, batch, height, width, use_graph=self.use_cuda_graph)
         return self._plans[key]
 
     def _evaluate(self, sources, timesteps, batch, height, width, clone=True):
@@ -175,7 +167,7 @@ class DiffusionInpaintingModel(nn.Module):
         """Pack [x | masked_image | mask x3] and a uniform timestep into the plan's network input and return the plan
         (see train_inpainting.InpaintingModelFn.fused_plan).  The caller owns the plan's inputs until its loop ends."""
         n, c, h, w = x.shape
-        if c + masked_image.shape[1] + 3 > 16 or self.base_model.micro_batches > 1:
+        if c + masked_image.shape[1] + 3 > 16:
             return None
         base = self.base_model
         plan = base.plan_for(n, h, w)
@@ -187,9 +179,9 @@ class DiffusionInpaintingModel(nn.Module):
 
     def slot_plan(self, batch, channels, height, width):
         """The engine plan of `batch` slots for continuous batching (continuous.py), or None when the network input
-        [x | masked_image | mask x3] does not fit the 16-channel stem pack or the batch is split into micro-batches.
-        The plan is the one the loops of this batch size use: the caller owns its inputs while it has work."""
-        if 2 * channels + 3 > 16 or self.base_model.micro_batches > 1:
+        [x | masked_image | mask x3] does not fit the 16-channel stem pack.  The plan is the one the loops of this
+        batch size use: the caller owns its inputs while it has work."""
+        if 2 * channels + 3 > 16:
             return None
         return self.base_model.plan_for(batch, height, width)
 

@@ -65,7 +65,6 @@ if "--halo" in sys.argv:
     run_halo("3x3 128->128 @256^2 B8 (K1h, GN fused)", 8, 256, 256, 128, 128, secs)
     sys.exit(0)
 
-print("CTA_PAIR =", os.environ.get("FIDM_CONV_CTA_PAIR", "1"))
 run("3x3 256->256 @256^2 B8 (K=2304)", 8, 256, 256, 256, 256, 3)
 run("1x1 2304->256 @256^2 B8 (pure GEMM, K=2304)", 8, 256, 256, 2304, 256, 1)
 run("3x3 512->256 @256^2 B8 (K=4608)", 8, 256, 256, 512, 256, 3)

@@ -55,7 +55,7 @@ def timeline(B, H, Cin, Cout, ks=3):
                 continue
             rel = (sel - t0).double() / 1e3
             print(f"   {nm:20s} min {rel.min():6.2f}  median {rel.median():6.2f}  max {rel.max():6.2f} us   (n={sel.numel()})")
-        for i, nm in ((16, "producer: past pdl_wait"), (17, "producer: indices")):
+        for i, nm in ((16, "producer: start"), (17, "producer: indices")):
             col = pr[:, i]
             rel = (col[col > 0] - t0).double() / 1e3
             if rel.numel():

@@ -76,7 +76,6 @@ flops = 2.0 * B * H * W * Cc * Cc * 9
 nbytes = B * H * W * Cc * 2
 sustained("conv 3x3 256->256 @256^2 fp16 operands", lambda: ops.conv2d(x16, w16, bias, out=y, impl="tc"), work=flops, unit="TFLOP/s")
 sustained("conv 3x3 256->256 @256^2 bf16 operands", lambda: ops.conv2d(xb, wb, bias, out=y, impl="tc"), work=flops, unit="TFLOP/s")
-os.environ["FIDM_CONV_CTA_PAIR"] = "0"
 a = torch.randn(8192, 8192, device=dev).bfloat16()
 b = torch.randn(8192, 8192, device=dev).bfloat16()
 sustained("torch.matmul bf16 8192^3 (cuBLAS)", lambda: torch.matmul(a, b), work=2.0 * 8192 ** 3, unit="TFLOP/s")
