@@ -71,6 +71,12 @@ class MsSlotArgs(C.Structure):
                 ("action", i32 * MAX_SLOTS), ("seeds", C.c_uint64 * MAX_SLOTS)]
 
 
+class RpSlotArgs(C.Structure):
+    _fields_ = [("t_value", fp), ("eval_t", vp), ("next_t", vp), ("undo", fp), ("inject_draw", vp), ("out", fp),
+                ("n_evals", i32), ("admit_draw", i32),
+                ("action", i32 * MAX_SLOTS), ("seeds", C.c_uint64 * MAX_SLOTS)]
+
+
 class PackArgs(C.Structure):
     _fields_ = [("batch", i32), ("hw", i32), ("n_src", i32), ("src", fp * 4),
                 ("src_channels", i32 * 4), ("src_repeat", i32 * 4),
@@ -119,6 +125,7 @@ SYMBOLS = {
     "fidm_randn_seeded": (C.c_int, [fp, vp, i32, C.c_int64, i32, i32, vp]),
     "fidm_sampler_step_slots": (C.c_int, [_P(StepArgs), _P(SlotArgs), vp]),
     "fidm_multistep_step_slots": (C.c_int, [_P(MultistepArgs), _P(MsSlotArgs), vp]),
+    "fidm_repaint_step_slots": (C.c_int, [_P(StepArgs), _P(RpSlotArgs), vp]),
     "fidm_pack_nchw_to_nhwc": (C.c_int, [_P(PackArgs), vp]),
     "fidm_unpack_nhwc_to_nchw": (C.c_int, [vp, i32, i32, fp, i32, i32, i32, vp]),
     "fidm_prepare_inputs_u8": (C.c_int, [vp, vp, fp, fp, fp, fp, i32, i32, vp]),

@@ -21,6 +21,12 @@ whose state channels and timesteps K8 writes, and an iteration without admission
 diffusion.continuous_dpm_solver_sampler(...) has the same surface for dpm_solver_sample_loop: every request takes
 `steps` evaluations on the DPM-Solver++ grid, each slot keeps its own history m_{k-1}, and the per-slot step is K9
 (fidm_multistep_step_slots); each result equals dpm_solver_sample_loop run alone with seeds=[seed].
+
+diffusion.continuous_repaint_sampler(...) does the same for repaint_sample_loop: every request takes the
+len(repaint.evaluation_plan(...)) evaluations of RePaint's walk, the schedule counts them, and the per-slot step is K10
+(fidm_repaint_step_slots): K8's DDPM update, K7's re-noising where a jump follows and the injection at the level the
+walk goes on at, from per-evaluation tables built once; each result equals repaint_sample_loop run alone with
+seeds=[seed].
 """
 import collections
 import ctypes as C
@@ -30,7 +36,7 @@ from typing import NamedTuple
 import torch
 
 from . import _lib as L
-from . import dpm_solver, seeded
+from . import dpm_solver, repaint, seeded
 
 
 def injection_draws(diffusion, schedule, cumulative, inject=True, grid=None):
@@ -38,7 +44,8 @@ def injection_draws(diffusion, schedule, cumulative, inject=True, grid=None):
     noise the number of injections before it; -1 where the loop does not inject (no injection, or t gated by
     `schedule`).  Without `grid`: indexed by t, the visits of ddim_sample_loop / p_sample_loop (T-1 .. 0).  With the
     DPM-Solver++ grid (dpm_solver.timestep_grid): indexed by grid point k, the visits of dpm_solver_sample_loop (x_T's
-    injection at grid[0] counts as the first)."""
+    injection at grid[0] counts as the first).  Any other list of visited timesteps, in loop order, works the same way
+    (repaint_slot_tables)."""
     ts = range(diffusion.num_timesteps - 1, -1, -1) if grid is None else [int(t) for t in grid]
     draws, fresh = [], 0
     for t in ts:
@@ -55,6 +62,21 @@ def dpm_slot_tables(diffusion, grid, order, schedule, cumulative, inject=True):
     the injection at t_k, and the order of the update out of t_k (dpm_solver.step_orders; 1 at the last point)."""
     return ([diffusion._t_value(int(t)) for t in grid], injection_draws(diffusion, schedule, cumulative, inject, grid),
             dpm_solver.step_orders(len(grid), order) + [1])
+
+
+def repaint_slot_tables(diffusion, jump_length, jump_n_sample, schedule, cumulative):
+    """K10's per-evaluation tables (fidm_rp_slot_args) as lists, from repaint.evaluation_plan: per evaluation k the
+    timestep it updates (eval_t), the level of its injection and of the next evaluation (next_t: t_up when a jump
+    follows, else t - 1; -1 after the last), the fp32 undo pair (a_u, s_u) (0 without a jump) and the draw of the
+    injection at next_t (-1: none); then the draw of the admission's injection at T-1.  The injections are counted in
+    repaint_sample_loop's order, x_T's at T-1 first, so fresh noise numbers them as that loop does and cumulative noise
+    reuses (INJECT, t) at a revisited level."""
+    plan = repaint.evaluation_plan(diffusion.alphas_cumprod, jump_length, jump_n_sample)
+    eval_t = [e.t for e in plan]
+    next_t = [e.t - 1 if e.t_up is None else e.t_up for e in plan]
+    undo = [(e.undo_a, e.undo_s) for e in plan]
+    draws = injection_draws(diffusion, schedule, cumulative, grid=[diffusion.num_timesteps - 1] + next_t[:-1])
+    return eval_t, next_t, undo, draws[1:] + [-1], draws[0]
 
 
 class SlotSchedule:
@@ -117,7 +139,8 @@ class ContinuousSampler:
         if denoised_fn is not None or cond_fn is not None:
             raise ValueError("continuous batching runs the fused sampler step: denoised_fn / cond_fn are not supported")
         if sampler not in ("ddim", "ddpm"):
-            hint = " (DPM-Solver++: diffusion.continuous_dpm_solver_sampler)" if sampler == "dpm_solver" else ""
+            hint = {"dpm_solver": " (DPM-Solver++: diffusion.continuous_dpm_solver_sampler)",
+                    "repaint": " (RePaint: diffusion.continuous_repaint_sampler)"}.get(sampler, "")
             raise ValueError(f"sampler must be 'ddim' or 'ddpm', got {sampler!r}{hint}")
         T = diffusion.num_timesteps
         self._setup(diffusion, model, slots, image_size, injection_schedule, channels, device, T)
@@ -222,7 +245,7 @@ class ContinuousSampler:
 
     # ------------------------------------------------------------------ iterations
     def step(self):
-        """One iteration: admit queued requests into free slots, evaluate every busy slot once, take one K8 (K9) step.
+        """One iteration: admit queued requests into free slots, evaluate every busy slot once, take one K8 (K9, K10) step.
         Returns [(ticket, image [1, C, H, W])] for the requests that finished; each image is a copy enqueued on the
         current stream, ready once the stream reaches it (the caller synchronises when it reads it)."""
         admitted = self.schedule.admit()
@@ -274,7 +297,7 @@ class ContinuousSampler:
 
     def _launch(self, actions, model_out):
         """One launch of the step kernel: slot b takes actions[b] (SLOT_ADMIT or its grid point: the timestep of a K8
-        update, the k of a K9 one), every other slot idles."""
+        update, the k of a K9 or K10 one), every other slot idles."""
         s = self._slot_args
         for b in range(self.B):
             s.action[b] = actions.get(b, L.SLOT_IDLE)
@@ -322,3 +345,45 @@ class ContinuousDPMSolverSampler(ContinuousSampler):
         ia, is_ = (L.C_SQRT_AB, L.C_SQRT_1MAB) if use_cumulative_noise else (L.C_SQRT_AB_F32, L.C_SQRT_1MAB_F32)
         s.admit_inject_a, s.admit_inject_s = float(cls[int(grid[0]), ia]), float(cls[int(grid[0]), is_])
         self._entry = "fidm_multistep_step_slots"
+
+
+class ContinuousRePaintSampler(ContinuousSampler):
+    """ContinuousSampler for repaint_sample_loop (built by GaussianDiffusion.continuous_repaint_sampler): every request
+    takes the evaluations of repaint.evaluation_plan(jump_length, jump_n_sample), and the per-slot step is K10
+    (fidm_repaint_step_slots) on K4's DDPM coefficient table and the per-evaluation tables of repaint_slot_tables."""
+
+    def __init__(self, diffusion, model, slots=8, image_size=(256, 256), jump_length=10, jump_n_sample=10,
+                 clip_denoised=True, use_inpainting_injection=True, injection_schedule="all", use_cumulative_noise=True,
+                 channels=3, device=None):
+        from .gaussian_diffusion import _MEAN_CODE, _VAR_CODE
+        T = diffusion.num_timesteps
+        repaint._check(T, jump_length, jump_n_sample)
+        if not use_inpainting_injection:
+            raise ValueError("RePaint resampling needs the known-region injection (use_inpainting_injection=True)")
+        eval_t, next_t, undo, draws, admit_draw = repaint_slot_tables(diffusion, jump_length, jump_n_sample,
+                                                                      injection_schedule, use_cumulative_noise)
+        n = len(eval_t)
+        self._setup(diffusion, model, slots, image_size, injection_schedule, channels, device, n)
+        # the schedule's counter c runs n-1 .. 0: evaluation k = n-1-c
+        self._t_of = eval_t[::-1]
+        self._action_of = list(range(n - 1, -1, -1))
+        dev = self.device
+        self._coef = diffusion._coef(dev, 0.0)
+        self._t_value = torch.tensor([diffusion._t_value(t) for t in range(T)], dtype=torch.float32, device=dev)
+        self._eval_t, self._next_t, self._inject_draw = (torch.tensor(v, dtype=torch.int32, device=dev)
+                                                         for v in (eval_t, next_t, draws))
+        self._undo = torch.tensor(undo, dtype=torch.float32, device=dev)
+
+        a = self._args = L.StepArgs()
+        a.batch, a.channels, a.hw = slots, channels, self.H * self.W
+        a.mode, a.sampler = L.STEP_UPDATE_INJECT, L.SAMPLER_DDPM
+        a.mean_type, a.var_type = _MEAN_CODE[diffusion.model_mean_type], _VAR_CODE[diffusion.model_var_type]
+        a.clip_denoised, a.cumulative = int(bool(clip_denoised)), int(bool(use_cumulative_noise))
+        a.mask_channels, a.num_timesteps = channels, T
+        a.coef, a.x, a.x_next, a.gt, a.keep_mask = (L.ptr(v) for v in (self._coef, self.x, self.x, self.gt, self.keep))
+        self._set_stem(a)
+        s = self._slot_args = L.RpSlotArgs()
+        s.t_value, s.eval_t, s.next_t, s.undo, s.inject_draw, s.out = (
+            L.ptr(v) for v in (self._t_value, self._eval_t, self._next_t, self._undo, self._inject_draw, self.out))
+        s.n_evals, s.admit_draw = n, admit_draw
+        self._entry = "fidm_repaint_step_slots"

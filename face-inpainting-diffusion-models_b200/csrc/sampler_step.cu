@@ -16,6 +16,11 @@
 // K8 (fidm_sampler_step_slots, continuous batching) is the same element body with SLOTS set: the action, the timesteps,
 // the seed and the draws come per slot from the launch parameters, x_T is generated for an admitted slot, and a slot
 // updated at t = 0 writes its sample to a separate buffer.  The update and injection arithmetic is K4's own code.
+//
+// K10 (fidm_repaint_step_slots, continuous batching of RePaint) is K8 with REPAINT set: the action is the slot's
+// evaluation index k, the timesteps and the injection draw come from per-evaluation tables, the step noise is (STEP, k),
+// and where a jump follows K7's re-noising (UNDO, k) sits between the update and the injection.  A fused jump
+// evaluation therefore computes, operation for operation, the lockstep pair K4 STEP_UPDATE_ONLY -> K7.
 #include "sampler_common.cuh"
 
 namespace fidm {
@@ -33,20 +38,28 @@ struct SlotParams {
   fidm_step_args a;
   fidm_slot_args s;
 };
-// The parameters of K4 (SLOTS false) and K8 (SLOTS and SEEDED true).
-template <bool SEEDED, bool SLOTS>
+struct RpSlotParams {
+  fidm_step_args a;
+  fidm_rp_slot_args s;
+};
+// The parameters of K4 (SLOTS false), K8 (SLOTS and SEEDED true) and K10 (all three true).
+template <bool SEEDED, bool SLOTS, bool REPAINT>
 struct KernelParams {
   using type = StepParams<SEEDED>;
 };
 template <>
-struct KernelParams<true, true> {
+struct KernelParams<true, true, false> {
   using type = SlotParams;
+};
+template <>
+struct KernelParams<true, true, true> {
+  using type = RpSlotParams;
 };
 
 __device__ __forceinline__ float clamp1(float v) { return fminf(fmaxf(v, -1.0f), 1.0f); }
 
-template <int VEC, bool SEEDED, bool SLOTS>
-__global__ void __launch_bounds__(256) sampler_step_kernel(const typename KernelParams<SEEDED, SLOTS>::type p) {
+template <int VEC, bool SEEDED, bool SLOTS, bool REPAINT = false>
+__global__ void __launch_bounds__(256) sampler_step_kernel(const typename KernelParams<SEEDED, SLOTS, REPAINT>::type p) {
   const fidm_step_args& a = p.a;
   const int hw_v = a.hw / VEC;
   const long long total = (long long)a.batch * a.channels * hw_v;
@@ -63,9 +76,17 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const typename Kernel
     if constexpr (SLOTS) {
       act = p.s.action[b];
       if (act == FIDM_SLOT_IDLE) continue;
-      t_upd = act;
-      t_inj = (act == FIDM_SLOT_ADMIT) ? a.num_timesteps - 1 : act - 1;
-      if (t_inj >= 0) slot_inj_draw = p.s.inject_draw[t_inj];
+      if constexpr (REPAINT) {
+        // K10: act is the evaluation index k; the walk goes on at next_t[k] (t_up after a jump)
+        const bool admit = act == FIDM_SLOT_ADMIT;
+        t_upd = admit ? act : p.s.eval_t[act];
+        t_inj = admit ? a.num_timesteps - 1 : p.s.next_t[act];
+        slot_inj_draw = admit ? p.s.admit_draw : p.s.inject_draw[act];
+      } else {
+        t_upd = act;
+        t_inj = (act == FIDM_SLOT_ADMIT) ? a.num_timesteps - 1 : act - 1;
+        if (t_inj >= 0) slot_inj_draw = p.s.inject_draw[t_inj];
+      }
     }
     if (!SEEDED && a.t_dev) {
       t_upd = (int)a.t_dev[b];
@@ -79,7 +100,8 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const typename Kernel
     const bool inj = SLOTS ? slot_inj_draw >= 0 : a.mode != FIDM_STEP_UPDATE_ONLY;
     const bool need_var = upd && a.var_type != FIDM_VAR_FIXED && (a.sampler == FIDM_SAMPLER_DDPM || a.logvar_out != nullptr);
     bool has_z;
-    if constexpr (SLOTS) has_z = p.s.step_noise != 0;
+    if constexpr (REPAINT) has_z = true;                 // DDPM: every update draws its step noise
+    else if constexpr (SLOTS) has_z = p.s.step_noise != 0;
     else if constexpr (SEEDED) has_z = p.s.draw >= 0;
     else has_z = a.z != nullptr;
     const bool need_z = upd && has_z;
@@ -98,7 +120,9 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const typename Kernel
     if (upd) load_vec<float, VEC>(a.model_out + ooff, mo);
     if (need_var) load_vec<float, VEC>(a.model_out + ooff + (long long)a.channels * a.hw, vv);
     if (need_z) {
-      if constexpr (SLOTS)
+      if constexpr (REPAINT)
+        seeded_normals<VEC>(seed, j, FIDM_NOISE_STEP, (uint32_t)act, zz);
+      else if constexpr (SLOTS)
         seeded_normals<VEC>(seed, j, FIDM_NOISE_STEP, (uint32_t)(a.num_timesteps - 1 - t_upd), zz);
       else if constexpr (SEEDED)
         seeded_elem_normals<VEC>(p.s, e, a.hw, FIDM_NOISE_STEP, p.s.draw, zz);
@@ -114,6 +138,13 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const typename Kernel
       else
         load_vec<float, VEC>(a.inject_noise + off, n);
       load_vec<float, VEC>(a.keep_mask + e.moff, m);
+    }
+    // K10: a jump follows the evaluation where the walk does not go on at t - 1; its undo noise is (UNDO, k)
+    [[maybe_unused]] bool jump = false;
+    [[maybe_unused]] float uu[VEC];
+    if constexpr (REPAINT) {
+      jump = upd && t_inj != t_upd - 1;
+      if (jump) seeded_normals<VEC>(seed, j, FIDM_NOISE_UNDO, (uint32_t)act, uu);
     }
     float smp[VEC], x0v[VEC];
 
@@ -186,6 +217,14 @@ __global__ void __launch_bounds__(256) sampler_step_kernel(const typename Kernel
     } else {
 #pragma unroll
       for (int i = 0; i < VEC; ++i) smp[i] = xs[i];
+    }
+    if constexpr (REPAINT) {
+      if (jump) {
+        // K7's re-noising from t - 1 to t_up (sampler_resample.cu)
+        const float ua = p.s.undo[2 * act], us = p.s.undo[2 * act + 1];
+#pragma unroll
+        for (int i = 0; i < VEC; ++i) smp[i] = __fadd_rn(__fmul_rn(ua, smp[i]), __fmul_rn(us, uu[i]));
+      }
     }
 
     if (inj) {
@@ -276,10 +315,46 @@ static int sampler_step_slots(const fidm_step_args* a, const fidm_slot_args* s, 
                         SlotParams{*a, *s}, stream, who);
 }
 
+static int repaint_step_slots(const fidm_step_args* a, const fidm_rp_slot_args* s, fidm_stream_t stream) {
+  const char* who = "repaint_step_slots";
+  FIDM_REQUIRE(a != nullptr && s != nullptr, FIDM_E_BADARG, "%s: null args", who);
+  FIDM_REQUIRE(a->batch >= 1 && a->batch <= FIDM_MAX_SLOTS, FIDM_E_BADARG, "%s: %d slots outside [1, %d]", who,
+               a->batch, FIDM_MAX_SLOTS);
+  FIDM_REQUIRE(a->channels > 0 && a->hw > 0 && a->num_timesteps > 0 && s->n_evals > 0, FIDM_E_BADARG,
+               "%s: empty shape", who);
+  FIDM_REQUIRE(a->sampler == FIDM_SAMPLER_DDPM, FIDM_E_BADARG, "%s: sampler must be DDPM", who);
+  FIDM_REQUIRE(a->coef && a->x && a->x_next && a->gt && a->keep_mask && s->out && s->t_value && s->eval_t &&
+                   s->next_t && s->undo && s->inject_draw,
+               FIDM_E_BADARG,
+               "%s: coef/x/x_next/gt/keep_mask/out/t_value/eval_t/next_t/undo/inject_draw are required", who);
+  FIDM_REQUIRE(a->z == nullptr && a->inject_noise == nullptr && a->t_dev == nullptr, FIDM_E_BADARG,
+               "%s: z/inject_noise/t_dev must be NULL", who);
+  FIDM_REQUIRE(!a->sample && !a->pred_xstart && !a->mean_out && !a->logvar_out, FIDM_E_BADARG,
+               "%s: sample/pred_xstart/mean_out/logvar_out must be NULL", who);
+  if (int rc = check_mask_channels(a, who)) return rc;
+  bool any_update = false;
+  for (int b = 0; b < a->batch; ++b) {
+    const int act = s->action[b];
+    FIDM_REQUIRE(act == FIDM_SLOT_IDLE || act == FIDM_SLOT_ADMIT || (act >= 0 && act < s->n_evals), FIDM_E_BADARG,
+                 "%s: slot %d: action %d is not IDLE, ADMIT or an evaluation in [0,%d)", who, b, act, s->n_evals);
+    any_update |= act >= 0;
+  }
+  FIDM_REQUIRE(!any_update || a->model_out != nullptr, FIDM_E_BADARG, "%s: model_out required for an update", who);
+  if (int rc = check_stem(a, who)) return rc;
+  const bool vec4 = vec4_ok(a->hw, a->x, a->model_out, a->gt, a->keep_mask, a->x_next, s->out);
+  const long long elems = (long long)a->batch * a->channels * a->hw;
+  return launch_sampler(sampler_step_kernel<4, true, true, true>, sampler_step_kernel<1, true, true, true>, vec4, elems,
+                        RpSlotParams{*a, *s}, stream, who);
+}
+
 }  // namespace fidm
 
 extern "C" int fidm_sampler_step_slots(const fidm_step_args* a, const fidm_slot_args* s, fidm_stream_t stream) {
   return fidm::sampler_step_slots(a, s, stream);
+}
+
+extern "C" int fidm_repaint_step_slots(const fidm_step_args* a, const fidm_rp_slot_args* s, fidm_stream_t stream) {
+  return fidm::repaint_step_slots(a, s, stream);
 }
 
 extern "C" int fidm_sampler_step(const fidm_step_args* a, fidm_stream_t stream) {

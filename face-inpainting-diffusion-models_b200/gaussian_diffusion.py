@@ -811,7 +811,7 @@ class GaussianDiffusion:
         return self._last_sample(self._repaint_loop(evals, model, shape, noise, clip_denoised, model_kwargs, device,
                                                     progress, injection_schedule, use_cumulative_noise, False, seeds))
 
-    # ------------------------------------------------------------------ continuous batching (K8, K9)
+    # ------------------------------------------------------------------ continuous batching (K8, K9, K10)
     def continuous_sampler(self, model, slots=8, image_size=(256, 256), sampler="ddim", eta=0.0, clip_denoised=True,
                            use_inpainting_injection=True, injection_schedule="all", use_cumulative_noise=True,
                            channels=3, device=None, denoised_fn=None, cond_fn=None):
@@ -837,6 +837,21 @@ class GaussianDiffusion:
                                           clip_denoised=clip_denoised, use_inpainting_injection=use_inpainting_injection,
                                           injection_schedule=injection_schedule,
                                           use_cumulative_noise=use_cumulative_noise, channels=channels, device=device)
+
+    def continuous_repaint_sampler(self, model, slots=8, image_size=(256, 256), jump_length=10, jump_n_sample=10,
+                                   clip_denoised=True, use_inpainting_injection=True, injection_schedule="all",
+                                   use_cumulative_noise=True, channels=3, device=None):
+        """continuous_sampler for RePaint resampling: every request takes the same
+        len(repaint.evaluation_plan(self.alphas_cumprod, jump_length, jump_n_sample)) model evaluations, its result
+        bit-identical to repaint_sample_loop(model, (1, C, H, W), jump_length, jump_n_sample, ..., seeds=[seed]) run
+        alone.  Same submit / step / pending / drain surface; arguments are checked here and at submit, before any
+        launch."""
+        from .continuous import ContinuousRePaintSampler
+        return ContinuousRePaintSampler(self, model, slots=slots, image_size=image_size, jump_length=jump_length,
+                                        jump_n_sample=jump_n_sample, clip_denoised=clip_denoised,
+                                        use_inpainting_injection=use_inpainting_injection,
+                                        injection_schedule=injection_schedule,
+                                        use_cumulative_noise=use_cumulative_noise, channels=channels, device=device)
 
     def sample_with_advanced_inpainting(self, model, shape, gt=None, gt_keep_mask=None, use_ddim=True, eta=0.0,
                                         progress=True, device=None, injection_schedule="all",

@@ -200,7 +200,8 @@ int fidm_resample_undo(const fidm_resample_args* a, fidm_stream_t stream);
  * be NULL, and reads the draws from `s`.  fidm_randn_seeded fills a buffer with the same values.
  * Draws of the sampling loops: x_T (XT, 0); step noise of the k-th evaluation (STEP, k); cumulative injection noise at
  * timestep t (INJECT, t); the i-th fresh injection of a loop (INJECT_FRESH, i); RePaint undo noise after evaluation k
- * (UNDO, k).  K8 (below) takes the same draws per slot.
+ * (UNDO, k).  K8, K9 and K10 (below) take the same draws per slot; K10 takes (STEP, k) and (UNDO, k) with k the
+ * slot's own evaluation index.
  * ---------------------------------------------------------------------------------------------- */
 enum { FIDM_NOISE_XT = 0, FIDM_NOISE_STEP = 1, FIDM_NOISE_INJECT = 2, FIDM_NOISE_INJECT_FRESH = 3, FIDM_NOISE_UNDO = 4 };
 typedef struct fidm_seeded_noise {
@@ -281,6 +282,41 @@ typedef struct fidm_ms_slot_args {
   uint64_t seeds[FIDM_MAX_SLOTS];       /* per slot: the request's seed */
 } fidm_ms_slot_args;
 int fidm_multistep_step_slots(const fidm_multistep_args* a, const fidm_ms_slot_args* s, fidm_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * K10  per-slot RePaint step (continuous batching of repaint_sample_loop): K8 on RePaint's walk.  Every request takes
+ * the same n_evals model evaluations (repaint.evaluation_plan); evaluation k is at timestep eval_t[k] and the walk goes
+ * on at next_t[k], which is t_up where a jump follows and eval_t[k] - 1 otherwise.  One launch takes, per slot, the
+ * action in s->action:
+ *   FIDM_SLOT_IDLE   nothing is read or written for the slot (state, stem, t_out, out);
+ *   FIDM_SLOT_ADMIT  K8's admission: x_T = draw (XT, 0) under the slot's seed, then the injection at T-1 with draw
+ *                    s->admit_draw unless it is < 0, written as the state, the stem channels and t_out[b] = t_value[T-1];
+ *   k in [0, n_evals) K4's seeded DDPM update at eval_t[k] with step noise (STEP, k); where a jump follows (next_t[k]
+ *                    != eval_t[k] - 1) K7's re-noising x' = undo[k][0]*x + undo[k][1]*u with u = (UNDO, k); then the
+ *                    injection at next_t[k] with draw (INJECT | INJECT_FRESH as a->cumulative, inject_draw[k]) unless
+ *                    that is < 0 (K4's expression and coefficients); state, stem and t_out[b] = t_value[next_t[k]] are
+ *                    written.  At k = n_evals-1 (eval_t = 0, next_t = -1) the sample goes to out[b] instead.
+ * Every value is bit-identical to what the seeded lockstep launches compute for that image alone: for a jump
+ * evaluation fidm_sampler_step_seeded's STEP_UPDATE_ONLY followed by fidm_resample_undo_seeded, otherwise its
+ * STEP_UPDATE_INJECT / STEP_UPDATE_ONLY.  Fields of `a` used: as K8, with sampler DDPM only; as for K8 the per-slot
+ * control travels by value in the launch parameters, and x_next may equal x.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct fidm_rp_slot_args {
+  const float* t_value;                 /* device [num_timesteps]: what the model sees for t (_scale_timesteps) */
+  const int32_t* eval_t;                /* device [n_evals]: the timestep evaluation k updates */
+  const int32_t* next_t;                /* device [n_evals]: the level of the injection and of evaluation k+1; -1 last.
+                                           The kernel takes next_t[k] != eval_t[k] - 1 to mean that a jump follows
+                                           (RePaint's t_up is always >= eval_t[k]), so a table without a jump at k
+                                           must hold eval_t[k] - 1 there */
+  const float* undo;                    /* device [n_evals][2]: (a_u, s_u) in fp32; 0 where no jump follows */
+  const int32_t* inject_draw;           /* device [n_evals]: draw of the injection at next_t[k]; -1: none */
+  float* out;                           /* [batch][channels][hw]: the sample of a slot at its last evaluation */
+  int32_t n_evals;                      /* evaluations per request */
+  int32_t admit_draw;                   /* draw of the admission's injection at T-1; -1: none */
+  int32_t action[FIDM_MAX_SLOTS];       /* per slot: FIDM_SLOT_IDLE | FIDM_SLOT_ADMIT | k (the evaluation) */
+  uint64_t seeds[FIDM_MAX_SLOTS];       /* per slot: the request's seed */
+} fidm_rp_slot_args;
+int fidm_repaint_step_slots(const fidm_step_args* a, const fidm_rp_slot_args* s, fidm_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Layout converters.  Replace torch.cat([x, masked_image, mask.repeat(1,3,1,1)], 1) of

@@ -18,7 +18,14 @@ With --sampler dpm_solver the four arms run DPM-Solver++ 2M in --steps evaluatio
 continuous_dpm_solver_sampler), and the step timing is K9 (all slots updating at a second-order grid point, injection,
 bf16 stem) against the seeded K6 on the same batch; its checks add the contract on the elementwise stand-in model.
 
-    python tools/continuous_probe.py [--rounds 3] [--load 0.8] [--sampler ddim | dpm_solver] [--steps 20]
+With --sampler repaint the four arms run RePaint(--jump-length, --jump-n-sample) on the 50-step cosine diffusion
+((a) and (b) through repaint_sample_loop, (c) and (d) through continuous_repaint_sampler) with 16 requests: at the
+default (5, 3) a request takes 140 evaluations, so a round takes seconds rather than minutes.  The step timing is K10
+(every slot on a jump evaluation, injection on, bf16 stem) against the seeded K4 STEP_UPDATE_ONLY + K7 pair it
+replaces; its checks add the contract on the stand-in model.
+
+    python tools/continuous_probe.py [--rounds 3] [--load 0.8] [--sampler ddim | dpm_solver | repaint] [--steps 20]
+                                     [--jump-length 5] [--jump-n-sample 3]
 """
 import argparse
 import ctypes
@@ -41,27 +48,39 @@ B, S, T, N = 8, 256, 50, 64
 
 
 class Workload:
-    """The sampler the arms run: DDIM-50 on the 50-step cosine diffusion (default), or DPM-Solver++ 2M in `steps`
-    evaluations on the 1000-step quadratic one.  evals: model evaluations per request."""
+    """The sampler the arms run: DDIM-50 on the 50-step cosine diffusion (default), DPM-Solver++ 2M in `steps`
+    evaluations on the 1000-step quadratic one, or RePaint(jump_length, jump_n_sample) on the 50-step cosine one.
+    evals: model evaluations per request; n: requests per arm."""
 
-    def __init__(self, F, sampler, steps):
-        self.dpm, self.steps = sampler == "dpm_solver", steps
+    def __init__(self, F, sampler, steps, jump_length=5, jump_n_sample=3):
+        from fidm_b200 import repaint
+        self.dpm, self.rp, self.steps = sampler == "dpm_solver", sampler == "repaint", steps
+        self.jl, self.jn = jump_length, jump_n_sample
         if self.dpm:
             self.d = F.create_gaussian_diffusion(steps=1000, learn_sigma=True, noise_schedule="quadratic")
         else:
             self.d = F.create_gaussian_diffusion(steps=T, learn_sigma=True, noise_schedule="cosine")
-        self.evals = steps if self.dpm else T
+        if self.rp:
+            self.evals = len(repaint.evaluation_plan(self.d.alphas_cumprod, jump_length, jump_n_sample))
+        else:
+            self.evals = steps if self.dpm else T
+        self.n = 16 if self.rp else N
 
     def loop(self, fn, gt, keep, seeds):
         kw = dict(model_kwargs={"gt": gt, "gt_keep_mask": keep}, device=gt.device, use_inpainting_injection=True,
                   seeds=seeds)
         if self.dpm:
             return self.d.dpm_solver_sample_loop(fn, tuple(gt.shape), steps=self.steps, **kw)
+        if self.rp:
+            return self.d.repaint_sample_loop(fn, tuple(gt.shape), jump_length=self.jl, jump_n_sample=self.jn, **kw)
         return self.d.ddim_sample_loop(fn, tuple(gt.shape), **kw)
 
     def continuous(self, fn):
         if self.dpm:
             return self.d.continuous_dpm_solver_sampler(fn, slots=B, image_size=(S, S), steps=self.steps)
+        if self.rp:
+            return self.d.continuous_repaint_sampler(fn, slots=B, image_size=(S, S), jump_length=self.jl,
+                                                     jump_n_sample=self.jn)
         return self.d.continuous_sampler(fn, slots=B, image_size=(S, S), sampler="ddim")
 
 
@@ -110,22 +129,22 @@ def standin_checks(w, gts, keeps, seeds, n=12):
 
 def run_alone(w, fn, gts, keeps, seeds):
     clk, done = _Clock(), []
-    for k in range(N):
+    for k in range(w.n):
         w.loop(fn, gts[k:k + 1], keeps[k:k + 1], [seeds[k]])
         done.append(clk.mark())
     torch.cuda.synchronize()
     lat = [clk.ms(e) for e in done]
-    return {"wall_ms": lat[-1], "latency_ms": lat, "occupancy": 1.0, "iterations": N * w.evals}
+    return {"wall_ms": lat[-1], "latency_ms": lat, "occupancy": 1.0, "iterations": w.n * w.evals}
 
 
 def run_lockstep(w, fn, gts, keeps, seeds):
     clk, done = _Clock(), []
-    for j in range(0, N, B):
+    for j in range(0, w.n, B):
         w.loop(fn, gts[j:j + B], keeps[j:j + B], seeds[j:j + B])
         done += [clk.mark()] * B
     torch.cuda.synchronize()
     lat = [clk.ms(e) for e in done]
-    return {"wall_ms": lat[-1], "latency_ms": lat, "occupancy": 1.0, "iterations": N // B * w.evals}
+    return {"wall_ms": lat[-1], "latency_ms": lat, "occupancy": 1.0, "iterations": w.n // B * w.evals}
 
 
 def run_continuous(w, fn, gts, keeps, seeds, arrivals_s=None):
@@ -134,9 +153,9 @@ def run_continuous(w, fn, gts, keeps, seeds, arrivals_s=None):
     clk = _Clock()
     arrive_ms, done, tickets = {}, {}, {}
     k, iters, busy = 0, 0, 0
-    while k < N or cs.pending():
+    while k < w.n or cs.pending():
         now = time.perf_counter() - clk.t0
-        while k < N and (arrivals_s is None or arrivals_s[k] <= now):
+        while k < w.n and (arrivals_s is None or arrivals_s[k] <= now):
             tk = cs.submit(gts[k], keeps[k], seeds[k])
             tickets[tk] = k
             arrive_ms[tk] = 0.0 if arrivals_s is None else arrivals_s[k] * 1e3
@@ -309,12 +328,86 @@ def k9_probe(d, steps, batch, dev):
     return res
 
 
+def k10_probe(d, jl, jn, batch, dev):
+    """us per step, every slot on the same jump evaluation (DDPM update, undo, cumulative injection at t_up, bf16 stem):
+    the seeded K4 STEP_UPDATE_ONLY + K7 pair against K10, each in a CUDA graph of 20."""
+    from fidm_b200 import _lib as L
+    from fidm_b200 import continuous, seeded
+    from fidm_b200.gaussian_diffusion import _MEAN_CODE, _VAR_CODE
+    eval_t, next_t, undo, draws, admit = continuous.repaint_slot_tables(d, jl, jn, "all", True)
+    k = next(k for k in range(len(eval_t)) if next_t[k] != eval_t[k] - 1 and draws[k] >= 0)
+    t, t_up, (ua, us) = eval_t[k], next_t[k], undo[k]
+    g = torch.Generator(device=dev).manual_seed(batch)
+    x = torch.randn(batch, 3, S, S, device=dev, generator=g)
+    mo = torch.randn(batch, 6, S, S, device=dev, generator=g)
+    gt = torch.rand(batch, 3, S, S, device=dev, generator=g)
+    keep = (torch.rand(batch, 3, S, S, device=dev, generator=g) > 0.5).float()
+    smp, nxt = torch.empty_like(x), torch.empty_like(x)
+    x_in = torch.zeros(batch, S, S, 16, device=dev, dtype=torch.bfloat16)
+    t_in = torch.zeros(batch, device=dev)
+    seeds = seeded.check_seeds(list(range(batch)), batch).to(dev)
+    coef = d._coef(dev, 0.0)
+    a4 = L.StepArgs()                                # K4 STEP_UPDATE_ONLY as _repaint_loop launches it
+    a4.batch, a4.channels, a4.hw, a4.mode, a4.sampler = batch, 3, S * S, L.STEP_UPDATE_ONLY, L.SAMPLER_DDPM
+    a4.mean_type, a4.var_type = _MEAN_CODE[d.model_mean_type], _VAR_CODE[d.model_var_type]
+    a4.clip_denoised, a4.cumulative, a4.mask_channels, a4.num_timesteps = 1, 1, 1, d.num_timesteps
+    a4.t_update, a4.t_inject = t, -1
+    a4.coef, a4.x, a4.model_out, a4.sample = L.ptr(coef), L.ptr(x), L.ptr(mo), L.ptr(smp)
+    s4 = L.SeededNoise()
+    s4.seeds, s4.draw, s4.inject_tag, s4.inject_draw = L.ptr(seeds), k, L.NOISE_INJECT, 0
+
+    def pair():
+        L.check(L.lib().fidm_sampler_step_seeded(ctypes.byref(a4), ctypes.byref(s4), L.stream()), "sampler_step_seeded")
+        d._resample(smp, seeded.Draw(seeds, L.NOISE_UNDO, k), ua, us, t_inject=t_up, gt=gt, keep=keep,
+                    inject_noise=seeded.Draw(seeds, L.NOISE_INJECT, t_up), stem=(x_in, t_in),
+                    t_next=d._t_value(t_up), next_buf=nxt)
+
+    tv = torch.tensor([d._t_value(v) for v in range(d.num_timesteps)], dtype=torch.float32, device=dev)
+    et, nt, dr = (torch.tensor(v, dtype=torch.int32, device=dev) for v in (eval_t, next_t, draws))
+    ud = torch.tensor(undo, dtype=torch.float32, device=dev)
+    out = torch.empty_like(x)
+    a = L.StepArgs()
+    a.batch, a.channels, a.hw, a.sampler = batch, 3, S * S, L.SAMPLER_DDPM
+    a.mean_type, a.var_type = a4.mean_type, a4.var_type
+    a.clip_denoised, a.cumulative, a.mask_channels, a.num_timesteps = 1, 1, 3, d.num_timesteps
+    a.coef, a.x, a.model_out, a.gt, a.keep_mask, a.x_next = (L.ptr(v) for v in (coef, x, mo, gt, keep, nxt))
+    a.stem_out, a.stem_dtype, a.stem_ld, a.t_out = L.ptr(x_in), L.BF16, 16, L.ptr(t_in)
+    s = L.RpSlotArgs()
+    s.t_value, s.eval_t, s.next_t, s.undo, s.inject_draw, s.out = (L.ptr(v) for v in (tv, et, nt, ud, dr, out))
+    s.n_evals, s.admit_draw = len(eval_t), admit
+    for b in range(batch):
+        s.action[b], s.seeds[b] = k, b
+
+    def k10():
+        L.check(L.lib().fidm_repaint_step_slots(ctypes.byref(a), ctypes.byref(s), L.stream()), "repaint_step_slots")
+
+    # per pixel, K4 DDPM with learned variance: read x 12, model_out 24, write sample 12; K7: read sample, gt, keep
+    # 3 x 12, write x 12, stem 6.  K10 moves the same minus the sample's write and read (read x, model_out, gt, keep;
+    # write x, stem): 78 of 102 B
+    n_pair = batch * S * S * (12 + 24 + 12 + 3 * 12 + 12 + 6)
+    n_k10 = batch * S * S * (12 + 24 + 2 * 12 + 12 + 6)
+    res = {"batch": batch, "evaluation": k, "t": t, "t_up": t_up, "bytes_per_step_pair": n_pair,
+           "bytes_per_step_k10": n_k10}
+    for name, fn, nb in (("seeded_k4_k7", pair, n_pair), ("k10", k10, n_k10)):
+        us_ = _graph_us(fn)
+        res[name] = {"us_per_step": round(us_, 2), "gbs": round(nb / (us_ * 1e-6) / 1e9, 1)}
+    pair()
+    ref, ref_stem, ref_t = nxt.clone(), x_in.clone(), t_in.clone()
+    nxt.zero_(), x_in.zero_(), t_in.zero_()
+    k10()
+    res["k10_equals_k4_k7"] = bool(torch.equal(nxt, ref) and torch.equal(x_in, ref_stem) and torch.equal(t_in, ref_t))
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--rounds", type=int, default=3, help="alternating timing rounds (the median is reported)")
     ap.add_argument("--load", type=float, default=0.8, help="Poisson arrival rate of (d) as a fraction of (b)'s rate")
-    ap.add_argument("--sampler", choices=("ddim", "dpm_solver"), default="ddim", help="the sampler of every arm")
+    ap.add_argument("--sampler", choices=("ddim", "dpm_solver", "repaint"), default="ddim",
+                    help="the sampler of every arm")
     ap.add_argument("--steps", type=int, default=20, help="model evaluations per request of --sampler dpm_solver")
+    ap.add_argument("--jump-length", type=int, default=5, help="RePaint jump length of --sampler repaint")
+    ap.add_argument("--jump-n-sample", type=int, default=3, help="RePaint jump_n_sample of --sampler repaint")
     args = ap.parse_args()
     import fidm_b200 as F
     from fidm_b200.utils.synth import synth_batch, synth_state_dict
@@ -327,7 +420,7 @@ def main():
     model.to(dev)
     model.base_model.set_precision("bf16")
     fn = F.InpaintingModelFn(model)
-    w = Workload(F, args.sampler, args.steps)
+    w = Workload(F, args.sampler, args.steps, args.jump_length, args.jump_n_sample)
     d = w.d
     data = synth_batch(N, S, seed=100, device=dev)
     gts, keeps = data["gt"], data["gt_keep_mask"]
@@ -343,7 +436,7 @@ def main():
         checks = {"continuous_equals_lockstep_b8": bool(torch.equal(cont, lock)),
                   "continuous_equals_alone_b1": bool(torch.equal(cont[:1], alone)),
                   "lockstep_b8_equals_alone_b1": bool(torch.equal(lock[:1], alone))}
-        if w.dpm:
+        if w.dpm or w.rp:
             checks.update(standin_checks(w, gts, keeps, seeds))
         ev = {1: eval_ms(fn, 1), B: eval_ms(fn, B)}
         rate_b = None
@@ -358,27 +451,31 @@ def main():
                     rate = args.load * rate_b                       # requests per second
                     rng = random.Random(r)
                     arr, t = [], 0.0
-                    for _ in range(N):
+                    for _ in range(w.n):
                         t += rng.expovariate(rate)
                         arr.append(t)
                     got[name].append(run_continuous(w, fn, gts, keeps, seeds, arr))
                 else:
                     got[name].append(run())
                 if name == "b_lockstep_b8" and rate_b is None:
-                    rate_b = N / (got[name][-1]["wall_ms"] * 1e-3)
+                    rate_b = w.n / (got[name][-1]["wall_ms"] * 1e-3)
         if w.dpm:
             steps = [k9_probe(d, args.steps, b, dev) for b in (8, 64)]
             checks["k9_equals_k6"] = all(st.pop("k9_equals_k6") for st in steps)
+        elif w.rp:
+            steps = [k10_probe(d, w.jl, w.jn, b, dev) for b in (8, 64)]
+            checks["k10_equals_k4_k7"] = all(st.pop("k10_equals_k4_k7") for st in steps)
         else:
             steps = [k8_probe(d, b, dev) for b in (8, 64)]
     cp = copy_gbs(dev)
     for st in steps:
-        for name in (("seeded_k6", "k9") if w.dpm else ("seeded_k4", "k8")):
+        for name in (("seeded_k6", "k9") if w.dpm else ("seeded_k4_k7", "k10") if w.rp else ("seeded_k4", "k8")):
             st[name]["fraction_of_copy"] = round(st[name]["gbs"] / cp, 3)
     out = {"probe": "continuous", "gpu": info,
-           "config": "ADM256 bf16, 256x256, %s, injection on, seeded, 8 slots, 64 requests (5-60 %% holes), "
+           "config": "ADM256 bf16, 256x256, %s, injection on, seeded, 8 slots, %d requests (5-60 %% holes), "
                      "synthetic weights" % ("DPM-Solver++ 2M-%d quadratic 1000" % args.steps if w.dpm
-                                            else "DDIM-50 cosine"),
+                                            else "RePaint(%d, %d) cosine 50, %d evaluations per request"
+                                            % (w.jl, w.jn, w.evals) if w.rp else "DDIM-50 cosine", w.n),
            "checks": checks, "eval_ms_alone": {str(k): round(v, 3) for k, v in ev.items()},
            "poisson_rate_per_s": round(args.load * rate_b, 3), "copy_gbs": cp, "step": steps, "runs": {}}
     for name, rs in got.items():
@@ -386,8 +483,8 @@ def main():
         walls = [r["wall_ms"] for r in rs]
         med = rs[walls.index(statistics.median_low(walls))]
         out["runs"][name] = {
-            "images_per_s": round(N / (med["wall_ms"] * 1e-3), 3),
-            "all_images_per_s": [round(N / (w * 1e-3), 3) for w in walls],
+            "images_per_s": round(w.n / (med["wall_ms"] * 1e-3), 3),
+            "all_images_per_s": [round(w.n / (v * 1e-3), 3) for v in walls],
             "latency_p50_ms": round(_pct(med["latency_ms"], 0.5), 1),
             "latency_p95_ms": round(_pct(med["latency_ms"], 0.95), 1),
             "mean_slot_occupancy": round(med["occupancy"], 3),
